@@ -27,6 +27,11 @@ N > 1 GPUs: the headline `value` is ONE fit with its CpG rows sharded over the G
 memory), then the identical test / alpha iterations on every rank -> "scaling": "strong".  The leg first checks, on 5 outer
 iterations, that alpha is bit-identical on all ranks and equals the one-GPU fit of the same data to 1e-9 (`row_sharded.parity`).
 `fit_sharded` = the other partitioning (independent fits, one per GPU, no collective; weak scaling) as an extra key.
+
+--dump-outputs DIR: after the timed steps, the u (M x n_u), alpha (K + n_u x N) and cost of the fit behind `value` (the resident
+arm's fit on one GPU, the row-sharded fit with u gathered in row order on several; with --impl reference, the oracle's fit on its
+row sample) go to DIR/{u,alpha,cost}.npy in float64.  The inputs are drawn from fixed seeds, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -51,6 +56,7 @@ OUTER_PER_STEP = 100
 CPU_SAMPLE_ROWS = 100_000
 METRIC = "update_iters_per_sec"
 UNIT = "inner update iterations/s at 1M CpG x 256 samples (K=6, n_u=2)"
+DUMP_BYTES = 60 << 20          # --dump-outputs: the .npy files stay under 64 MB in all, headers included
 
 
 def parse():
@@ -67,7 +73,11 @@ def parse():
     ap.add_argument("--engine", default="auto", choices=["auto", "fused", "gram", "stream"], help="device engine of the timed region")
     ap.add_argument("--boot-resamples", type=int, default=1000, help="resamples of the BASELINE config-4 bootstrap leg (0 = skip the leg)")
     ap.add_argument("--boot-rows", type=int, default=500_000, help="CpG rows of the bootstrap leg (debug)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write u, alpha and cost of the timed fit as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def workload_config(M, extra=None):
@@ -78,6 +88,21 @@ def workload_config(M, extra=None):
     if extra:
         cfg.update(extra)
     return cfg
+
+
+def dump_outputs(out_dir, arrays):
+    """Write `arrays` as out_dir/<name>.npy in float64 so that two builds can be compared output for output.  An array larger than
+    its share of DUMP_BYTES is replaced by a fixed, seeded sample of its rows, with the sampled row indices in <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            n_keep = share // (a.nbytes // a.shape[0] + 8)
+            rows = np.sort(np.random.RandomState(0).choice(a.shape[0], n_keep, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def synth_host(M, seed=0):
@@ -183,6 +208,9 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     leg = cpu_reference_leg(args.steps, args.warmup)
+    if args.dump_outputs:
+        u_last, a_last, tr = leg["result"]
+        dump_outputs(args.dump_outputs, {"u": u_last, "alpha": a_last, "cost": tr["costs"][-1]})
     line = {"impl": "reference", "metric": METRIC, "value": leg["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": leg["s_per_step_sample"] * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic", "config": workload_config(M_FULL),
@@ -504,6 +532,12 @@ def run_b200(args, rank, world, local_rank):
         fit.finish(0.0)
         st_rs = be.batch.states()[0]
         assert st_rs.n_outer == n_total and np.isfinite(st_rs.cost)
+        if args.dump_outputs:
+            (u_rows, a_rs, _n, c_rs), = be.results()
+            u_parts = [None] * world
+            dist.all_gather_object(u_parts, u_rows)             # rank order = row order (row_range)
+            if rank == 0:
+                dump_outputs(args.dump_outputs, {"u": np.concatenate(u_parts), "alpha": a_rs, "cost": c_rs})
         row_sharded = {"value": 2 * N_ITER2 * OUTER_PER_STEP * args.steps / (float(rs_ms[0]) * 1e-3), "unit": UNIT, "scaling": "strong",
                        "ms_per_step": float(rs_ms[0]) / args.steps, "rows_per_gpu": hi - lo,
                        "ms_per_outer_iteration": float(rs_ms[0]) / (args.steps * OUTER_PER_STEP),
@@ -516,6 +550,9 @@ def run_b200(args, rank, world, local_rank):
         be.close()
         del be, sprob
 
+    if args.dump_outputs and row_sharded is None and rank == 0:
+        (u_last, a_last, _n, c_last), = batch.results()
+        dump_outputs(args.dump_outputs, {"u": u_last, "alpha": a_last, "cost": c_last})
     if args.profile:
         if rank == 0:
             print(json.dumps({"profile_run": True, "engine": engine, "ms": kern}))

@@ -43,15 +43,20 @@ def test_bootstrap_seed_sequence_and_restart_jobs():
         bootstrap_seeds([5], 3)                                    # `--seed 5` reaches bt_ci as a list (Q1)
 
 
-def test_bench_clock_sampler_window():
-    """bench.py's nvidia-smi sampler: only samples inside the timed region count; a region shorter than the sampling period falls
-    back to all samples (warm-up ran the same kernels) and says so."""
+def _bench_module():
     import importlib.util
     import os
-    import time
     spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_clock_sampler_window():
+    """bench.py's nvidia-smi sampler: only samples inside the timed region count; a region shorter than the sampling period falls
+    back to all samples (warm-up ran the same kernels) and says so."""
+    import time
+    bench = _bench_module()
 
     class FakeProc:
         def terminate(self):
@@ -72,3 +77,49 @@ def test_bench_clock_sampler_window():
     s2.mark_begin()
     out2 = s2.stop()
     assert out2["samples"] == 1 and out2["sm_mhz"] == 1900.0 and out2["window"].startswith("warm-up")
+
+
+def test_bench_dump_outputs_budget(tmp_path):
+    """bench.py --dump-outputs: float64 .npy files under 64 MB in all; an array over its share becomes the same seeded sample of
+    its rows on every run, with the row indices beside it."""
+    import os
+    bench = _bench_module()
+    u = np.random.RandomState(0).uniform(size=(4_000_000, 2))         # 64 MB on its own
+    alpha = np.random.RandomState(1).uniform(size=(8, 256)).astype(np.float32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"u": u, "alpha": alpha, "cost": 2.5})
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["alpha.npy", "cost.npy", "u.npy", "u_rows.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) < 64 * 2 ** 20
+    got = {n: np.load(tmp_path / "a" / n) for n in names}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["alpha.npy"], alpha) and got["cost.npy"] == 2.5
+    rows = got["u_rows.npy"].astype(np.int64)
+    assert np.all(np.diff(rows) > 0) and np.array_equal(got["u.npy"], u[rows])
+    assert rows[-1] > 3 * len(rows) and len(rows) * (u[0].nbytes + 8) > 0.99 * bench.DUMP_BYTES / 3    # spread over u, fills its share
+    assert all(np.array_equal(got[n], np.load(tmp_path / "b" / n)) for n in names)
+    u_headline = u[:1_000_000]                                         # the default workload's u (1M x 2) is written whole
+    bench.dump_outputs(str(tmp_path / "c"), {"u": u_headline, "alpha": alpha, "cost": 2.5})
+    assert not (tmp_path / "c" / "u_rows.npy").exists() and np.array_equal(np.load(tmp_path / "c" / "u.npy"), u_headline)
+
+
+def test_bench_reference_arm_dumps_its_last_step(tmp_path, monkeypatch, capsys):
+    """--impl reference --dump-outputs writes the oracle's (u, alpha, cost) of its last timed step."""
+    import argparse
+    bench = _bench_module()
+    u, a = np.arange(6.0).reshape(3, 2), np.full((8, 4), 0.125)
+    leg = {"result": (u, a, {"costs": [9.0, 7.5]}), "value": 1.0, "unit": bench.UNIT, "cores": 1, "kind": "port", "sample": "",
+           "s_per_step_sample": 1.0}
+    monkeypatch.setattr(bench, "cpu_reference_leg", lambda steps, warmup: leg)
+    bench.run_reference(argparse.Namespace(steps=1, warmup=0, gpus=1, dump_outputs=str(tmp_path)), 0, 1)
+    assert '"impl": "reference"' in capsys.readouterr().out
+    assert np.array_equal(np.load(tmp_path / "u.npy"), u) and np.array_equal(np.load(tmp_path / "alpha.npy"), a)
+    assert np.load(tmp_path / "cost.npy") == 7.5
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"]])
+def test_bench_refuses_bad_step_counts(monkeypatch, argv):
+    bench = _bench_module()
+    monkeypatch.setattr("sys.argv", ["bench.py", *argv])
+    with pytest.raises(SystemExit):
+        bench.parse()
