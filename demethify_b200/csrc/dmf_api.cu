@@ -38,53 +38,6 @@ struct dmf_handle_s {
     int max_smem_optin;
 };
 
-struct dmf_batch_s {
-    dmf_handle_s* h;
-    dmf_shape_t shape;
-    Geom g;
-    FitDev* fits_dev;       // in workspace
-    FitState* states_dev;   // in workspace, contiguous [n_fits]
-    int ktb, c_alpha, ntc_alpha;      // alpha / cost kernels
-    int kb, nub, c_u, ntc_u;          // U kernel
-    unsigned smem_alpha, smem_u, smem_cost;
-    int occ;
-    long long launches;
-    FitState* pinned;       // host staging for state polling
-    // Gram-form engine (dmf_gram.cuh)
-    int engine;             // DMF_ENGINE_*
-    int gram_ok;            // this shape has Gram-engine instantiations
-    Geom gg;                // tile geometry of the Gram-engine streaming passes (no u_prev in the stage)
-    int kb_g, nub_g, c_g, ntc_g, pb_g, c_p, ntc_p, ktb_in;
-    int n_parts_u, n_groups_u;
-    unsigned smem_rg, smem_panel;
-    int p1_ok;                      // own geometry of the one-unknown multiplicity-form panel kernel (two CTAs per SM)
-    Geom gp1;
-    unsigned smem_p1;
-    int n_active;                   // fits_dev holds the descriptors of the first n_active still-running fits (compacted at every poll)
-    // peer exchange (row-sharded runs): symmetric buffers of all ranks, see peer_allreduce_kernel
-    double** peers_dev;             // device array [world]
-    unsigned* xchg_ticket;          // device
-    int peer_rank, peer_world;
-    long long peer_slot_stride, peer_flag_off;
-    unsigned xchg_epoch;
-    // fused engine (dmf_fused.cuh)
-    int fused_ok;                   // this shape / layout has a fused-pass instantiation
-    int kb_f, nub_f, s_f;
-    FusedArgs fa;                   // launch template (geometry, stage layout); fits / iteration arguments are filled per launch
-    unsigned smem_f;
-    int fused_pending;              // a dmf_fused_outer ran since the cost of the current iterate was last evaluated
-    int multmode;                   // fits are bootstrap resamples in multiplicity form
-    int sharded;                    // CpG rows sharded over GPUs: kernels publish partial sums, finalize runs on all-reduced sums
-    std::vector<FitDev> fits_host;
-    double *stats_local, *stats_global;
-    size_t stats_doubles, stats_gbx, stats_scal;
-    // momentum table (library-owned, grows on demand): a_t and (a_t - 1) / a_{t+1}
-    std::vector<double> mom_host;   // [a_0 .. a_{n-1} | m_0 .. m_{n-1}] is rebuilt on growth
-    double* mom_dev;
-    size_t mom_cap;                 // entries per array on the device
-    long long t_hi;                 // upper bound of the inner-iteration index any fit of the batch can have reached
-};
-
 namespace {
 
 // ---------------------------------------------------------------------------------------------
@@ -107,119 +60,137 @@ fused_kern_t by_types_f(const dmf_shape_t& s, int kb, int nub, int sblk) {
     return g_fused[i](kb, nub, sblk);
 }
 
-int next_pow2(int v) { int p = 1; while (p < v) p <<= 1; return p; }
-
 // ---------------------------------------------------------------------------------------------
-// Geometry.  One stage of the ring holds tile_rows rows of every streamed matrix with the global pitch.
+// Geometry.  One stage of the ring holds tile_rows rows of every streamed matrix (X, D, Rk, U, Uprev).
+struct StageLayout { size_t off[kMaxSrc], bytes, tx[kMaxSrc]; };
+// `row`: bytes per row of each matrix in the stage, `copy`: bytes per row that a tile copies; `x_tail` bytes follow the X rows.
+// Every matrix starts 128-byte aligned.
+StageLayout stage_layout(long long rows, const size_t (&row)[kMaxSrc], const size_t (&copy)[kMaxSrc], size_t x_tail = 0) {
+    StageLayout L{};
+    size_t o = 0;
+    for (int i = 0; i < kMaxSrc; ++i) {
+        L.off[i] = o;
+        L.tx[i] = rows * copy[i];
+        o = align_up(o + rows * row[i] + (i == 0 ? x_tail : 0), 128);
+    }
+    L.bytes = o;
+    return L;
+}
+void set_stages(Geom& g, const StageLayout& L) {
+    g.offX = (unsigned)L.off[0]; g.offD = (unsigned)L.off[1]; g.offR = (unsigned)L.off[2]; g.offU = (unsigned)L.off[3]; g.offUp = (unsigned)L.off[4];
+    g.stage_bytes = (unsigned)L.bytes;
+    for (int i = 0; i < kMaxSrc; ++i) g.tile_tx[i] = (unsigned)L.tx[i];
+}
+
+// CTAs per fit: fill the GPU (SMs x occupancy) across the whole batch, never more than tiles.  Multi-fit batches: fits terminate
+// at different outer iterations, so every fit gets at least 32 CTAs (the grid is oversubscribed, terminated fits return at once)
+// and the stragglers still spread over the GPU.
+int ctas_per_fit(const dmf_handle_s* h, const dmf_shape_t& s, int occ, int n_tiles) {
+    long long per_fit = std::max<long long>(s.n_fits > 1 ? 32 : 1, (long long)h->sm_count * occ / s.n_fits);
+    if (s.max_ctas_per_fit > 0) per_fit = std::min<long long>(per_fit, s.max_ctas_per_fit);
+    return (int)std::min<long long>(per_fit, n_tiles);
+}
+int groups_of(int parts) { return (parts + kGroup - 1) / kGroup; }
+
+// Launch geometry of every engine for one shape.  Engines the shape cannot use keep their zero values.
 struct Plan {
+    // stream engine: cost / alpha / U passes (g.ntc and g.rg are set per launch)
+    Geom g;
     int ktb, c_alpha, ntc_alpha;          // alpha / cost kernels: register-row bucket, columns per thread
-    int kb, nub, c_u, rpt_max, ntc_u;     // U kernel buckets
-    int Kp, nup, rpt;
-    int tile_rows, n_tiles, n_parts, n_groups, part_stride, occ;
-    unsigned offX, offD, offR, offU, offUp, stage_bytes, smem_alpha, smem_u, smem_cost, row_bulk;
-    size_t ws_bytes, off_fits, off_states, off_tickets, off_part, off_gpart, per_fit_tickets, per_fit_part, per_fit_gpart;
-    // Gram engine
-    int gram_ok, kb_g, nub_g, c_g, rpt_g_max, rpt_g, ntc_g, occ_g, pb_g, c_p, ntc_p, ktb_in;
-    int tile_rows_g, n_tiles_g, n_parts_g, n_groups_g, wpr_g, ng_g, stages_g;
+    int kb, nub, c_u, ntc_u;              // U kernel buckets
+    unsigned smem_alpha, smem_u, smem_cost;
+    // Gram-form engine (dmf_gram.cuh): own tile geometry, no u_prev in the stage
+    int gram_ok;
+    Geom gg;
+    int kb_g, nub_g, c_g, ntc_g, pb_g, c_p, ntc_p, ktb_in;
     int n_parts_u, n_groups_u;     // u_inner_kernel: one thread per row, many more CTAs than the streaming passes
-    unsigned g_offX, g_offD, g_offR, g_offU, g_offUp, g_stage_bytes, smem_rg, smem_panel;
+    unsigned smem_rg, smem_panel;
     int mult_ok;                   // multiplicity form (bootstrap resamples) available for this shape
+    unsigned tx_mult[kMaxSrc];     // gg.tile_tx of the multiplicity form: per-source-row sums and multiplicities instead of U, Uprev
     // the 128-register panel variant of the multiplicity form (one unknown type) gets smaller tiles of its own: two CTAs per SM
-    int p1_ok, p1_tile_rows, p1_n_tiles, p1_stages;
-    unsigned p1_offX, p1_offD, p1_offR, p1_offU, p1_offUp, p1_stage_bytes, p1_smem;
+    int p1_ok;
+    Geom gp1;
+    unsigned smem_p1;
+    // fused engine (dmf_fused.cuh)
+    int fused_ok, kb_f, nub_f, s_f;
+    FusedShape fc;
+    FusedArgs fa;                  // launch template (geometry, stage layout); fits / iteration arguments are filled per launch
+    unsigned smem_f;
+    // workspace layout
+    size_t ws_bytes, off_fits, off_states, off_tickets, off_part, off_gpart, per_fit_tickets, per_fit_part, per_fit_gpart;
     size_t off_usum, per_fit_usum;
     size_t off_rowgram, off_stats, off_gstats, off_red, per_fit_rowgram, per_fit_stats, per_fit_red;
     size_t stats_gbx, stats_scal;      // offsets (in doubles) of gbx and scal inside a per-fit stats block [gram | gbx | scal(8)]
-    // fused engine
-    int fused_ok, kb_f, nub_f, s_f, n_tiles_f, n_parts_f, n_groups_f;
-    unsigned f_pitchX, f_pitchD, f_offD, f_offR, f_offU, f_offUp, f_stage_bytes, f_offStats, f_offTab, f_zero_off, smem_f;
 };
 
-constexpr int pow2ceil_h(int v) { int p = 1; while (p < v) p <<= 1; return p; }
-constexpr int ng_of_h(int nub) { return nub + nub * (nub + 1) / 2; }
-
-// U-pass instantiations (dmf_inst_body.cuh): known bucket, unknown bucket, columns/thread, rows/thread/tile
-struct UEntry { int kb, nub, c, rpt; };
-const UEntry kUTable[] = {{6, 2, 2, 4}, {8, 2, 2, 4}, {8, 8, 2, 1}, {16, 2, 2, 4}, {16, 8, 2, 1}, {16, 16, 1, 1}, {32, 2, 1, 4}, {32, 8, 1, 1}, {32, 32, 1, 1}};
-
 int make_plan(const dmf_handle_s* h, const dmf_shape_t& s, Plan& p) {
+    p = Plan{};
     if (s.M <= 0 || s.N <= 0 || s.K < 0 || s.n_u <= 0 || s.n_fits <= 0) return fail(DMF_E_SHAPE, "M, N, n_u, n_fits must be positive and K >= 0");
     if (s.mode == DMF_MODE_UNSUPERVISED && s.K != 0) return fail(DMF_E_SHAPE, "unsupervised mode requires K = 0");
     if (s.mode == DMF_MODE_PURITY && s.K == 0) return fail(DMF_E_SHAPE, "purity mode requires K >= 1");
     if (s.dtype != DMF_F64 && s.dtype != DMF_F32) return fail(DMF_E_ARG, "dtype must be DMF_F64 or DMF_F32");
     if (s.wtype != DMF_W_FLOAT && s.wtype != DMF_W_U16) return fail(DMF_E_ARG, "wtype must be DMF_W_FLOAT or DMF_W_U16");
-    p.Kp = s.K + (s.K & 1);
-    p.nup = s.n_u + (s.n_u & 1);
-    if (s.ldx < s.N || s.ldd < s.N || s.ldr < p.Kp || s.ldu < p.nup) return fail(DMF_E_SHAPE, "row pitch smaller than the (even-padded) row");
+    const int Kp = s.K + (s.K & 1), nup = s.n_u + (s.n_u & 1);
+    if (s.ldx < s.N || s.ldd < s.N || s.ldr < Kp || s.ldu < nup) return fail(DMF_E_SHAPE, "row pitch smaller than the (even-padded) row");
     if ((s.ldx | s.ldd | s.ldu | (s.K ? s.ldr : 0)) & 1) return fail(DMF_E_SHAPE, "row pitches must be even (zero padded)");
     const size_t sT = s.dtype == DMF_F64 ? 8 : 4;
     const size_t sW = s.wtype == DMF_W_U16 ? 2 : sT;
     if (s.u_slot < s.M * s.ldu || (s.u_slot * sT) % 16) return fail(DMF_E_SHAPE, "u_slot must be >= M*ldu and a multiple of 16 bytes");
     if (s.u_slots != 0 && s.u_slots != 2 && s.u_slots != 4) return fail(DMF_E_SHAPE, "u_slots must be 2 (or 0) or 4");
     const int Kt = s.K + s.n_u;
-    const int rowlen = p.Kp + p.nup;
+    const int rowlen = Kp + nup;
     if (rowlen > kMaxKt || Kt > kMaxKt) return fail(DMF_E_SHAPE, "K + n_u (even padded) > 32 is not supported by this build");
     p.ktb = rowlen <= 8 ? 8 : (rowlen <= 16 ? 16 : 32);
     p.c_alpha = p.ktb <= 16 ? 2 : 1;
-    const UEntry* ue = nullptr;
-    for (const UEntry& e : kUTable)
-        if (e.kb >= p.Kp && e.nub >= p.nup) { ue = &e; break; }
+    const KernEntry* ue = nullptr;
+    for (const KernEntry& e : kUTable)
+        if (e.kb >= Kp && e.nub >= nup) { ue = &e; break; }
     if (!ue) return fail(DMF_E_SHAPE, "no U-pass instantiation for this K / n_u");
-    p.kb = ue->kb; p.nub = ue->nub; p.c_u = ue->c; p.rpt_max = ue->rpt;
+    p.kb = ue->kb; p.nub = ue->nub; p.c_u = ue->c;
     if (s.N > kConsumers * p.c_alpha || s.N > kConsumers * p.c_u)
         return fail(DMF_E_SHAPE, "N too large for this K + n_u in this build (N <= 512 for small K + n_u, <= 256 otherwise)");
-    p.ntc_alpha = next_pow2((s.N + p.c_alpha - 1) / p.c_alpha);
-    p.ntc_u = next_pow2((s.N + p.c_u - 1) / p.c_u);
+    p.ntc_alpha = pow2ceil((s.N + p.c_alpha - 1) / p.c_alpha);
+    p.ntc_u = pow2ceil((s.N + p.c_u - 1) / p.c_u);
     const int rg_u = kConsumers / p.ntc_u;
 
     const size_t px = s.ldx * sT, pd = s.ldd * sW, pr = s.K ? s.ldr * sT : 0, pu = (size_t)s.ldu * sT;
     // smallest row multiple that keeps every tile start 16-byte aligned
     int ra = 1;
     while (ra < 16 && ((ra * px) % 16 || (ra * pd) % 16 || (ra * pr) % 16 || (ra * pu) % 16)) ra <<= 1;
-    const size_t row_bytes = px + pd + pr + 2 * pu;
     const size_t smem_cap = (size_t)h->max_smem_optin;
-    p.occ = (p.ktb <= 8 && ((p.kb + 2 * p.nub) * p.c_u <= 24)) ? 2 : 1;   // must mirror the __launch_bounds__ of the kernels
-    auto stage_of = [&](long long tr) {
-        auto a128 = [](size_t v) { return align_up(v, 128); };
-        return a128(tr * px) + a128(tr * pd) + a128(tr * pr) + 2 * a128(tr * pu);
-    };
-    p.rpt = 0;
-    for (int attempt = 0; attempt < 2 && !p.rpt; ++attempt) {
-        const size_t budget = (p.occ == 2 ? std::min<size_t>(smem_cap, 112 * 1024) : std::min<size_t>(smem_cap, 220 * 1024)) - kCtlBytes - 4096;
-        for (int rpt = p.rpt_max; rpt >= 1; rpt >>= 1) {
-            const long long tr = (long long)rpt * rg_u;
+    const size_t rows_s[kMaxSrc] = {px, pd, pr, pu, pu};
+    int occ = std::min(pass_min_blocks(p.ktb), u_pass_min_blocks(p.kb, p.nub, p.c_u));
+    int rpt = 0;
+    for (int attempt = 0; attempt < 2 && !rpt; ++attempt) {
+        const size_t budget = (occ == 2 ? std::min<size_t>(smem_cap, 112 * 1024) : std::min<size_t>(smem_cap, 220 * 1024)) - kCtlBytes - 4096;
+        for (int r = ue->rpt; r >= 1; r >>= 1) {
+            const long long tr = (long long)r * rg_u;
             if (tr % ra) continue;
-            if (stage_of(tr) * kStages + (size_t)2 * tr * s.n_u * ((p.ntc_u + 31) / 32) * 8 <= budget) { p.rpt = rpt; break; }
+            if (stage_layout(tr, rows_s, rows_s).bytes * kStages + (size_t)2 * tr * s.n_u * ((p.ntc_u + 31) / 32) * 8 <= budget) { rpt = r; break; }
         }
-        if (!p.rpt) {
-            if (p.occ == 2) p.occ = 1; else break;
+        if (!rpt) {
+            if (occ == 2) occ = 1; else break;
         }
     }
-    if (!p.rpt) return fail(DMF_E_SHAPE, "one row tile does not fit in shared memory (or pitches force an unsupported tile alignment)");
-    const long long tr = (long long)p.rpt * rg_u;
-    p.tile_rows = (int)tr;
-    p.n_tiles = (int)((s.M + tr - 1) / tr);
-    auto a128 = [](size_t v) { return (unsigned)align_up(v, 128); };
-    p.offX = 0;
-    p.offD = a128(p.offX + tr * px);
-    p.offR = a128(p.offD + tr * pd);
-    p.offU = a128(p.offR + tr * pr);
-    p.offUp = a128(p.offU + tr * pu);
-    p.stage_bytes = a128(p.offUp + tr * pu);
-    p.row_bulk = (px % 16 == 0 ? 1u : 0u) | (pd % 16 == 0 ? 2u : 0u) | ((pr % 16 == 0 && pr) ? 4u : 0u);
+    if (!rpt) return fail(DMF_E_SHAPE, "one row tile does not fit in shared memory (or pitches force an unsupported tile alignment)");
+    const long long tr = (long long)rpt * rg_u;
+    Geom& g = p.g;
+    g.M = s.M; g.N = s.N; g.K = s.K; g.nu = s.n_u; g.Kt = Kt;
+    g.ldx = s.ldx; g.ldd = s.ldd; g.ldr = s.K ? s.ldr : 0; g.ldu = s.ldu;
+    g.Kp = Kp; g.nup = nup; g.rpt = rpt;
+    g.uslot_bytes = s.u_slot * sT;
+    g.tile_rows = (int)tr;
+    g.n_tiles = (int)((s.M + tr - 1) / tr);
+    g.ntc = p.ntc_alpha; g.rg = kConsumers / p.ntc_alpha;
+    g.n_parts = ctas_per_fit(h, s, occ, g.n_tiles);
+    g.n_groups = groups_of(g.n_parts);
+    set_stages(g, stage_layout(tr, rows_s, rows_s));
+    g.row_bulk = (px % 16 == 0 ? 1u : 0u) | (pd % 16 == 0 ? 2u : 0u) | ((pr % 16 == 0 && pr) ? 4u : 0u);
+    g.mode = s.mode;
+    g.stages = kStages;
+    int part_stride = (int)align_up((size_t)std::max(Kt * s.N, 4), 2);
 
-    // CTAs per fit: fill the GPU (SMs x occupancy) across the whole batch, never more than tiles
-    long long target = (long long)h->sm_count * p.occ;
-    // multi-fit batches: fits terminate at different outer iterations, so every fit gets at least kMinParts CTAs (the grid is
-    // oversubscribed, terminated fits return at once) and the stragglers still spread over the GPU
-    const long long kMinParts = s.n_fits > 1 ? 32 : 1;
-    long long per_fit = std::max<long long>(kMinParts, target / s.n_fits);
-    if (s.max_ctas_per_fit > 0) per_fit = std::min<long long>(per_fit, s.max_ctas_per_fit);
-    p.n_parts = (int)std::min<long long>(per_fit, p.n_tiles);
-    p.n_groups = (p.n_parts + kGroup - 1) / kGroup;
-    p.part_stride = (int)align_up((size_t)std::max(Kt * s.N, 4), 2);
-
-    const size_t pipe = kCtlBytes + (size_t)kStages * p.stage_bytes;
+    const size_t pipe = kCtlBytes + (size_t)kStages * g.stage_bytes;
     const size_t epi_alpha = kCtlBytes + ((size_t)(Kt + 1) * s.N + 32) * 8;
     const int wpr_u = (p.ntc_u + 31) / 32;
     const size_t red_u = wpr_u > 1 ? (size_t)2 * tr * wpr_u * s.n_u * 8 : 0;
@@ -228,152 +199,134 @@ int make_plan(const dmf_handle_s* h, const dmf_shape_t& s, Plan& p) {
     p.smem_cost = (unsigned)std::max(pipe, (size_t)kCtlBytes + 512);
     if (std::max(p.smem_alpha, p.smem_u) > smem_cap) return fail(DMF_E_SHAPE, "shared-memory plan exceeds the device limit");
 
-    // ---- Gram-form engine (dmf_gram.cuh): n_u <= 4, own tile geometry (no u_prev in the stage, rows per thread from kGramTable)
-    p.gram_ok = 0;
-    p.n_parts_g = p.n_groups_g = p.n_parts_u = p.n_groups_u = 0;
-    p.mult_ok = 0;
-    p.p1_ok = 0;
-    p.per_fit_usum = 0;
-    p.per_fit_rowgram = p.per_fit_stats = p.per_fit_red = 0;
-    p.stats_gbx = p.stats_scal = 0;
-    if (s.n_u <= 4 || (s.n_u <= 8 && p.Kp <= 6)) {      // 5 .. 8 unknown types: 4-column kernels only (K <= 6)
-        p.kb_g = s.K == 0 ? 0 : (p.Kp <= 6 ? 6 : (p.Kp <= 16 ? 16 : 32));
-        p.nub_g = s.n_u == 1 ? 1 : (s.n_u == 2 ? 2 : (s.n_u <= 4 ? 4 : 8));
-        p.c_g = p.kb_g <= 6 ? 4 : (p.kb_g <= 16 ? 2 : 1);
-        // rows per thread and tile: the 4-column kernels walk a tile in batches of their register rows (4 / 4 / 2 / 1 for 1 / 2 / 4 / 8
-        // unknown types), so 4 rows per thread and tile for all of them
-        p.rpt_g_max = p.c_g == 4 ? 4 : (p.nub_g == 1 ? 4 : (p.nub_g == 2 ? 3 : 2));
-        p.ng_g = ng_of_h(p.nub_g);
+    // ---- Gram-form engine (dmf_gram.cuh): the first kRowgramTable entry that covers K and n_u (n_u <= 4, or n_u <= 8 when K <= 6)
+    const KernEntry* ge = nullptr;
+    for (const KernEntry& e : kRowgramTable)
+        if (e.kb >= Kp && e.nub >= s.n_u) { ge = &e; break; }
+    if (ge) {
+        p.kb_g = ge->kb; p.nub_g = ge->nub; p.c_g = ge->c;
+        // rows per thread and tile: the 4-column kernels walk a tile in batches of their register rows, 4 rows per thread and tile for all
+        const int rpt_g_max = p.c_g == 4 ? 4 : ge->rpt;
+        const int ng = ng_of(p.nub_g);
         p.pb_g = rowlen <= 8 ? 8 : 16;
         p.c_p = p.pb_g == 8 ? 4 : 1;
         p.ktb_in = Kt <= 8 ? 8 : (Kt <= 16 ? 16 : 32);
         if (s.N <= kConsumers * p.c_g && s.N <= kConsumers * p.c_p) {
-            p.ntc_g = next_pow2((s.N + p.c_g - 1) / p.c_g);
-            p.ntc_p = next_pow2((s.N + p.c_p - 1) / p.c_p);
-            p.wpr_g = (p.ntc_g + 31) / 32;
+            p.ntc_g = pow2ceil((s.N + p.c_g - 1) / p.c_g);
+            p.ntc_p = pow2ceil((s.N + p.c_p - 1) / p.c_p);
+            const int wpr_g = (p.ntc_g + 31) / 32;
             const int rg_g = kConsumers / p.ntc_g;
-            // must mirror the __launch_bounds__ of rowgram_kernel / gram_panel_kernel
-            const int occ_rg = p.c_g == 4 ? 1 : (((p.kb_g + 2 * p.nub_g) * p.c_g + 2 * pow2ceil_h(p.rpt_g_max * p.ng_g) <= 56) ? 2 : 1);
-            const int occ_pn = (2 * (p.pb_g + 1) * p.c_p <= 40) ? 2 : 1;
-            p.occ_g = std::min(occ_rg, occ_pn);
-            auto a128g = [](size_t v) { return align_up(v, 128); };
+            int occ_g = std::min(rowgram_min_blocks(p.kb_g, p.nub_g, p.c_g, rpt_g_max), panel_min_blocks(2, p.pb_g, p.c_p));
             // the U region also holds the per-source-row sums of the multiplicity form (NG doubles per row), followed by the multiplicities
-            const size_t pu_stage = std::max(pu, (size_t)p.ng_g * 8);
-            auto stage_g = [&](long long tr) { return a128g(tr * px) + a128g(tr * pd) + a128g(tr * pr) + a128g(tr * pu_stage) + a128g(tr * 4); };
+            const size_t rows_g[kMaxSrc] = {px, pd, pr, std::max(pu, (size_t)ng * 8), 4};
+            const size_t copy_g[kMaxSrc] = {px, pd, pr, pu, 0}, copy_m[kMaxSrc] = {px, pd, pr, (size_t)ng * 8, 4};
             const size_t epi_panel = kCtlBytes + (size_t)(p.pb_g + 1) * s.N * 8 + 256;
-            p.rpt_g = 0;
-            p.stages_g = kStages;
-            for (int attempt = 0; attempt < 2 && !p.rpt_g; ++attempt) {
-                const size_t budget = (p.occ_g == 2 ? std::min<size_t>(smem_cap, 112 * 1024) : std::min<size_t>(smem_cap, 220 * 1024)) - kCtlBytes - 1024;
+            int rpt_g = 0, stages_g = kStages;
+            for (int attempt = 0; attempt < 2 && !rpt_g; ++attempt) {
+                const size_t budget = (occ_g == 2 ? std::min<size_t>(smem_cap, 112 * 1024) : std::min<size_t>(smem_cap, 220 * 1024)) - kCtlBytes - 1024;
                 // full rows-per-thread first (register slots beyond rpt would be dead work), with a shallower ring if need be
-                for (int rpt = p.rpt_g_max; rpt >= 1 && !p.rpt_g; rpt = (p.c_g == 4 ? rpt >> 1 : rpt - 1)) {
-                    const long long trg = (long long)rpt * rg_g;
+                for (int r = rpt_g_max; r >= 1 && !rpt_g; r = (p.c_g == 4 ? r >> 1 : r - 1)) {
+                    const long long trg = (long long)r * rg_g;
                     if (trg % ra) continue;
                     for (int stg = kStages; stg >= 3; --stg)
-                        if (stage_g(trg) * stg <= budget && epi_panel <= budget + kCtlBytes) { p.rpt_g = rpt; p.stages_g = stg; break; }
+                        if (stage_layout(trg, rows_g, copy_g).bytes * stg <= budget && epi_panel <= budget + kCtlBytes) { rpt_g = r; stages_g = stg; break; }
                 }
-                if (!p.rpt_g) {
-                    if (p.occ_g == 2) p.occ_g = 1; else break;
+                if (!rpt_g) {
+                    if (occ_g == 2) occ_g = 1; else break;
                 }
             }
-            if (p.rpt_g) {
-                const long long trg = (long long)p.rpt_g * rg_g;
-                p.tile_rows_g = (int)trg;
-                p.n_tiles_g = (int)((s.M + trg - 1) / trg);
-                p.g_offX = 0;
-                p.g_offD = (unsigned)a128g(p.g_offX + trg * px);
-                p.g_offR = (unsigned)a128g(p.g_offD + trg * pd);
-                p.g_offU = (unsigned)a128g(p.g_offR + trg * pr);
-                p.g_offUp = (unsigned)a128g(p.g_offU + trg * pu_stage);
-                p.g_stage_bytes = (unsigned)a128g(p.g_offUp + trg * 4);
+            if (rpt_g) {
+                const long long trg = (long long)rpt_g * rg_g;
+                Geom& q = p.gg;
+                q = g;
+                q.rpt = rpt_g;
+                q.tile_rows = (int)trg; q.n_tiles = (int)((s.M + trg - 1) / trg);
+                q.ntc = p.ntc_g; q.rg = rg_g;
+                q.n_parts = ctas_per_fit(h, s, occ_g, q.n_tiles);
+                q.n_groups = groups_of(q.n_parts);
+                q.stages = stages_g;
+                set_stages(q, stage_layout(trg, rows_g, copy_g));
+                const StageLayout lm = stage_layout(trg, rows_g, copy_m);
+                for (int i = 0; i < kMaxSrc; ++i) p.tx_mult[i] = (unsigned)lm.tx[i];
                 p.mult_ok = (p.c_g == 4 && p.pb_g == 8 && p.nub_g <= 4 && trg % 4 == 0 && s.mode != DMF_MODE_UNSUPERVISED) ? 1 : 0;
-                p.per_fit_usum = p.mult_ok ? align_up((size_t)s.M * p.ng_g * 8, 256) : 0;
-                p.p1_ok = 0;
+                p.per_fit_usum = p.mult_ok ? align_up((size_t)s.M * ng * 8, 256) : 0;
                 if (p.mult_ok && s.n_u == 1) {
                     const size_t budget1 = std::min<size_t>(smem_cap, 112 * 1024) - kCtlBytes - 1024;
                     for (long long tr1 = trg / 2; tr1 >= 4 && !p.p1_ok; tr1 /= 2) {
                         if (tr1 % ra || tr1 % 4) continue;
+                        const StageLayout l1 = stage_layout(tr1, rows_g, copy_m);
                         for (int stg = kStages; stg >= 3; --stg)
-                            if (stage_g(tr1) * stg <= budget1 && epi_panel <= budget1 + kCtlBytes) {
-                                p.p1_ok = 1; p.p1_tile_rows = (int)tr1; p.p1_stages = stg;
-                                p.p1_n_tiles = (int)((s.M + tr1 - 1) / tr1);
-                                p.p1_offX = 0;
-                                p.p1_offD = (unsigned)a128g(tr1 * px);
-                                p.p1_offR = (unsigned)a128g(p.p1_offD + tr1 * pd);
-                                p.p1_offU = (unsigned)a128g(p.p1_offR + tr1 * pr);
-                                p.p1_offUp = (unsigned)a128g(p.p1_offU + tr1 * pu_stage);
-                                p.p1_stage_bytes = (unsigned)a128g(p.p1_offUp + tr1 * 4);
-                                p.p1_smem = (unsigned)std::max(kCtlBytes + (size_t)stg * p.p1_stage_bytes, epi_panel);
+                            if (l1.bytes * stg <= budget1 && epi_panel <= budget1 + kCtlBytes) {
+                                Geom& r = p.gp1;
+                                r = q;
+                                r.tile_rows = (int)tr1; r.n_tiles = (int)((s.M + tr1 - 1) / tr1); r.stages = stg;
+                                r.rpt = 1;                                  // unused by the panel kernel (it strides over the rows of a tile)
+                                r.n_parts = std::min(q.n_parts, r.n_tiles); r.n_groups = groups_of(r.n_parts);
+                                set_stages(r, l1);
+                                p.smem_p1 = (unsigned)std::max(kCtlBytes + (size_t)stg * r.stage_bytes, epi_panel);
+                                p.p1_ok = 1;
                                 break;
                             }
                     }
                 }
-                long long per_fit_g = std::max<long long>(kMinParts, (long long)h->sm_count * p.occ_g / s.n_fits);
-                if (s.max_ctas_per_fit > 0) per_fit_g = std::min<long long>(per_fit_g, s.max_ctas_per_fit);
-                p.n_parts_g = (int)std::min<long long>(per_fit_g, p.n_tiles_g);
-                p.n_groups_g = (p.n_parts_g + kGroup - 1) / kGroup;
-                p.n_parts_u = (int)std::min<long long>((s.M + kThreads - 1) / kThreads, std::max<long long>(p.n_parts_g, (long long)h->sm_count * 8 / s.n_fits));
-                p.n_groups_u = (p.n_parts_u + kGroup - 1) / kGroup;
-                const size_t pipe_g = kCtlBytes + (size_t)p.stages_g * p.g_stage_bytes;
+                p.n_parts_u = (int)std::min<long long>((s.M + kThreads - 1) / kThreads, std::max<long long>(q.n_parts, (long long)h->sm_count * 8 / s.n_fits));
+                p.n_groups_u = groups_of(p.n_parts_u);
+                const size_t pipe_g = kCtlBytes + (size_t)stages_g * q.stage_bytes;
                 p.smem_rg = (unsigned)std::max(pipe_g, (size_t)kCtlBytes + 512);
                 p.smem_panel = (unsigned)std::max(pipe_g, epi_panel);
-                p.part_stride = std::max(p.part_stride, (int)align_up((size_t)2 * (p.pb_g + 1) * s.N, 2));
-                p.per_fit_rowgram = align_up((size_t)s.M * p.wpr_g * p.ng_g * 8, 256);
+                part_stride = std::max(part_stride, (int)align_up((size_t)2 * (p.pb_g + 1) * s.N, 2));
+                p.per_fit_rowgram = align_up((size_t)s.M * wpr_g * ng * 8, 256);
                 p.stats_gbx = (size_t)Kt * Kt * s.N;
                 p.stats_scal = p.stats_gbx + (size_t)Kt * s.N;
                 p.per_fit_stats = align_up((p.stats_scal + 8) * 8, 256);
-                p.per_fit_red = align_up((size_t)p.part_stride * 8, 256);
+                p.per_fit_red = align_up((size_t)part_stride * 8, 256);
                 p.gram_ok = 1;
             }
         }
     }
     // ---- fused engine (dmf_fused.cuh): FP64, n_u <= 2, K <= 8, N <= 256, four U slots, rows that bulk copies can place one by one
-    p.fused_ok = 0;
-    p.n_parts_f = p.n_groups_f = 0;
     if (p.gram_ok && s.dtype == DMF_F64 && s.n_u <= 2 && s.K <= 8 && s.N <= 256 && s.u_slots >= 4 && (s.ldd * sW) % 16 == 0) {
         p.kb_f = s.K == 0 ? 0 : (s.K <= 4 ? 4 : (s.K <= 6 ? 6 : 8));
         p.nub_f = s.n_u;
         p.s_f = s.N <= 64 ? 1 : (s.N <= 128 ? 2 : 4);
-        const int ng = ng_of_h(p.nub_f), ncol = p.nub_f * p.kb_f + (ng - p.nub_f), nblk = (ncol + 7) / 8;
-        auto a128f = [](size_t v) { return (unsigned)align_up(v, 128); };
+        p.fc = fused_shape(p.s_f, p.nub_f);          // rows per tile, ring depth and statistics buffers of the width class
+        const int ng = ng_of(p.nub_f), ncol = p.nub_f * p.kb_f + (ng - p.nub_f);
         // a tile is ONE bulk copy per matrix: it keeps the caller's row pitch in shared memory (dmf_shape_t recommends pitches that
         // are free of bank conflicts); 16 zero bytes behind the X rows of every stage serve the panel columns that do not exist.
-        // Rows per tile, ring depth and statistics buffers depend on the width class (FusedCfg in dmf_fused.cuh).
-        const int f_rows = fused_cfg_rows(p.s_f), f_stages = fused_cfg_stages(p.s_f);
-        p.f_pitchX = (unsigned)px;
-        p.f_pitchD = (unsigned)pd;
-        p.f_zero_off = (unsigned)((size_t)f_rows * px);
-        p.f_offD = a128f((size_t)f_rows * p.f_pitchX + 16);
-        p.f_offR = a128f(p.f_offD + (size_t)f_rows * p.f_pitchD);
-        p.f_offU = a128f(p.f_offR + (size_t)f_rows * pr);
-        p.f_offUp = a128f(p.f_offU + (size_t)f_rows * pu);
-        p.f_stage_bytes = a128f(p.f_offUp + (size_t)f_rows * pu);
-        p.f_offStats = kFusedCtlBytes + f_stages * p.f_stage_bytes;
-        // row statistics (one partial per A-warp sample group and row; fused_cfg_nstat buffers), then the per-sample table of the A-warps
-        p.f_offTab = a128f(p.f_offStats + (unsigned)fused_cfg_nstat(p.s_f) * fused_cfg_sgroups(p.s_f) * f_rows * ng * 8u);
-        p.smem_f = p.f_offTab + 32u * p.s_f * 2u * p.nub_f * 8u;
-        (void)nblk;
+        const StageLayout lf = stage_layout(p.fc.rows, rows_s, rows_s, 16);
+        FusedArgs& fa = p.fa;
+        fa.pitchX = (unsigned)px;
+        fa.pitchD = (unsigned)pd;
+        fa.zero_off = (unsigned)((size_t)p.fc.rows * px);
+        fa.offD = (unsigned)lf.off[1]; fa.offR = (unsigned)lf.off[2]; fa.offU = (unsigned)lf.off[3]; fa.offUp = (unsigned)lf.off[4];
+        fa.stage_bytes = (unsigned)lf.bytes;
+        fa.offStats = kFusedCtlBytes + p.fc.stages * fa.stage_bytes;
+        // row statistics (one partial per A-warp sample group and row; nstat buffers), then the per-sample table of the A-warps
+        fa.offTab = (unsigned)align_up(fa.offStats + (unsigned)p.fc.nstat * p.fc.sgroups * p.fc.rows * ng * 8u, 128);
+        p.smem_f = fa.offTab + 32u * p.s_f * 2u * p.nub_f * 8u;
         const size_t n_rec = 2 + (size_t)(ncol + p.nub_f) * s.N;
-        if (p.smem_f <= smem_cap && kFusedCtlBytes + n_rec * 8 <= p.f_offStats) {
-            p.n_tiles_f = (int)((s.M + f_rows - 1) / f_rows);
-            long long per_fit_f = std::max<long long>(kMinParts, (long long)h->sm_count / s.n_fits);
-            if (s.max_ctas_per_fit > 0) per_fit_f = std::min<long long>(per_fit_f, s.max_ctas_per_fit);
-            p.n_parts_f = (int)std::min<long long>(per_fit_f, p.n_tiles_f);
-            p.n_groups_f = (p.n_parts_f + kGroup - 1) / kGroup;
-            p.part_stride = std::max(p.part_stride, (int)align_up(n_rec, 2));
-            p.per_fit_red = align_up((size_t)p.part_stride * 8, 256);
+        if (p.smem_f <= smem_cap && kFusedCtlBytes + n_rec * 8 <= fa.offStats) {
+            fa.n_tiles = (int)((s.M + p.fc.rows - 1) / p.fc.rows);
+            fa.g = g;
+            fa.g.n_parts = ctas_per_fit(h, s, 1, fa.n_tiles);
+            fa.g.n_groups = groups_of(fa.g.n_parts);
+            part_stride = std::max(part_stride, (int)align_up(n_rec, 2));
+            p.per_fit_red = align_up((size_t)part_stride * 8, 256);
             p.fused_ok = 1;
         }
     }
-    const int parts_max = std::max(std::max(p.n_parts, p.n_parts_g), p.n_parts_f), groups_max = std::max(std::max(std::max(p.n_groups, p.n_groups_g), p.n_groups_u), p.n_groups_f);
+    // one partial-record stride for every engine: they share the workspace
+    for (Geom* q : {&p.g, &p.gg, &p.gp1, &p.fa.g}) q->part_stride = part_stride;
+    const int parts_max = std::max({p.g.n_parts, p.gg.n_parts, p.fa.g.n_parts});
+    const int groups_max = std::max({p.g.n_groups, p.gg.n_groups, p.n_groups_u, p.fa.g.n_groups});
     // u_inner_kernel records are 8 doubles apart: n_parts_u * 8 <= parts_max * part_stride holds because part_stride >= 2 * 9 * N
 
     // workspace layout
     p.off_fits = 0;
     p.off_states = align_up(p.off_fits + sizeof(FitDev) * s.n_fits, 256);
     p.per_fit_tickets = align_up(sizeof(unsigned) * (groups_max + 1), 128);
-    p.per_fit_part = align_up((size_t)parts_max * p.part_stride * 8, 128);
-    p.per_fit_gpart = align_up((size_t)groups_max * p.part_stride * 8, 128);
+    p.per_fit_part = align_up((size_t)parts_max * part_stride * 8, 128);
+    p.per_fit_gpart = align_up((size_t)groups_max * part_stride * 8, 128);
     p.off_tickets = align_up(p.off_states + sizeof(FitState) * s.n_fits, 256);
     p.off_part = align_up(p.off_tickets + p.per_fit_tickets * s.n_fits, 256);
     p.off_gpart = align_up(p.off_part + p.per_fit_part * s.n_fits, 256);
@@ -385,6 +338,38 @@ int make_plan(const dmf_handle_s* h, const dmf_shape_t& s, Plan& p) {
     p.ws_bytes = align_up(p.off_usum + p.per_fit_usum * s.n_fits, 256);
     return DMF_OK;
 }
+
+}  // namespace
+
+struct dmf_batch_s {
+    dmf_handle_s* h;
+    dmf_shape_t shape;
+    Plan p;                 // make_plan, adjusted to the batch by dmf_batch_create (gather, multiplicity form, engines it rules out)
+    FitDev* fits_dev;       // in workspace
+    FitState* states_dev;   // in workspace, contiguous [n_fits]
+    long long launches;
+    FitState* pinned;       // host staging for state polling
+    int engine;             // DMF_ENGINE_*
+    int n_active;                   // fits_dev holds the descriptors of the first n_active still-running fits (compacted at every poll)
+    // peer exchange (row-sharded runs): symmetric buffers of all ranks, see peer_allreduce_kernel
+    double** peers_dev;             // device array [world]
+    unsigned* xchg_ticket;          // device
+    int peer_rank, peer_world;
+    long long peer_slot_stride, peer_flag_off;
+    unsigned xchg_epoch;
+    int fused_pending;              // a dmf_fused_outer ran since the cost of the current iterate was last evaluated
+    int multmode;                   // fits are bootstrap resamples in multiplicity form
+    int sharded;                    // CpG rows sharded over GPUs: kernels publish partial sums, finalize runs on all-reduced sums
+    std::vector<FitDev> fits_host;
+    double *stats_local, *stats_global;
+    // momentum table (library-owned, grows on demand): a_t and (a_t - 1) / a_{t+1}
+    std::vector<double> mom_host;   // [a_0 .. a_{n-1} | m_0 .. m_{n-1}] is rebuilt on growth
+    double* mom_dev;
+    size_t mom_cap;                 // entries per array on the device
+    long long t_hi;                 // upper bound of the inner-iteration index any fit of the batch can have reached
+};
+
+namespace {
 
 // Make sure the device momentum table covers indices [0, need].  Growth synchronises the stream (rare: the table doubles).
 int ensure_mom(dmf_batch_s* b, long long need, cudaStream_t st) {
@@ -442,7 +427,7 @@ int launch(dmf_batch_s* b, kern_t k, int ntc, unsigned smem, int flags, int k_in
     if (!k) return fail(DMF_E_SHAPE, "no kernel instantiation for this shape");
     if (b->multmode) return fail(DMF_E_STATE, "fits in multiplicity form run on the Gram-form engine only (dmf_gram_*)");
     PassArgs a;
-    a.g = b->g;
+    a.g = b->p.g;
     a.g.ntc = ntc;
     a.g.rg = kConsumers / ntc;
     a.fits = b->fits_dev;
@@ -451,23 +436,23 @@ int launch(dmf_batch_s* b, kern_t k, int ntc, unsigned smem, int flags, int k_in
     a.tol = tol;
     a.ca0 = a.cb0 = a.with_x = a.pad = 0;
     a.mom_a = b->mom_dev; a.mom_m = b->mom_dev ? b->mom_dev + b->mom_cap : nullptr;
-    dim3 grid(b->g.n_parts, b->n_active, 1);
+    dim3 grid(a.g.n_parts, b->n_active, 1);
     k<<<grid, kThreads, smem, st>>>(a);
     CUDA_TRY(cudaGetLastError());
     b->launches++;
     return DMF_OK;
 }
 
-kern_t k_cost(dmf_batch_s* b, int initial) { return by_types(b->shape, g_cost, b->ktb, initial, b->c_alpha); }
-kern_t k_alpha(dmf_batch_s* b) { return by_types(b->shape, g_alpha, b->ktb, 0, b->c_alpha); }
-kern_t k_u(dmf_batch_s* b) { return by_types(b->shape, g_u, b->kb, b->nub, b->c_u); }
-kern_t k_rowgram(dmf_batch_s* b, int initial) { return by_types(b->shape, g_rowgram, b->kb_g, b->nub_g, initial | (b->c_g == 4 ? 2 : 0)); }
-kern_t k_panel(dmf_batch_s* b) { return by_types(b->shape, g_panel, b->pb_g, b->c_p, b->multmode); }
-kern_t k_panel_u1(dmf_batch_s* b) { return by_types(b->shape, g_panel, b->pb_g, b->c_p, 2); }     // multiplicity form, n_u == 1
-kern_t k_uinner(dmf_batch_s* b) { return by_types(b->shape, g_uinner, b->nub_g, b->multmode ? 1 : 0, 0); }
-kern_t k_costcross(dmf_batch_s* b) { return by_types(b->shape, g_uinner, b->nub_g, 2, 0); }
-kern_t k_usum(dmf_batch_s* b) { return by_types(b->shape, g_uinner, b->nub_g, 3, 0); }
-kern_t k_ainner(dmf_batch_s* b) { return by_types(b->shape, g_ainner, b->ktb_in, 0, 0); }
+kern_t k_cost(dmf_batch_s* b, int initial) { return by_types(b->shape, g_cost, b->p.ktb, initial, b->p.c_alpha); }
+kern_t k_alpha(dmf_batch_s* b) { return by_types(b->shape, g_alpha, b->p.ktb, 0, b->p.c_alpha); }
+kern_t k_u(dmf_batch_s* b) { return by_types(b->shape, g_u, b->p.kb, b->p.nub, 0); }
+kern_t k_rowgram(dmf_batch_s* b, int initial) { return by_types(b->shape, g_rowgram, b->p.kb_g, b->p.nub_g, initial); }
+kern_t k_panel(dmf_batch_s* b) { return by_types(b->shape, g_panel, b->p.pb_g, b->p.c_p, b->multmode); }
+kern_t k_panel_u1(dmf_batch_s* b) { return by_types(b->shape, g_panel, b->p.pb_g, b->p.c_p, 2); }     // multiplicity form, n_u == 1
+kern_t k_uinner(dmf_batch_s* b) { return by_types(b->shape, g_uinner, b->p.nub_g, b->multmode ? 1 : 0, 0); }
+kern_t k_costcross(dmf_batch_s* b) { return by_types(b->shape, g_uinner, b->p.nub_g, 2, 0); }
+kern_t k_usum(dmf_batch_s* b) { return by_types(b->shape, g_uinner, b->p.nub_g, 3, 0); }
+kern_t k_ainner(dmf_batch_s* b) { return by_types(b->shape, g_ainner, b->p.ktb_in, 0, 0); }
 
 // Gram-engine launch: geometry gg; ntc selects the thread mapping of the kernel; grid_x CTAs per fit (0: one CTA per fit on grid.x)
 int launch_g(dmf_batch_s* b, kern_t k, int ntc, unsigned smem, int flags, int k_inner, double tol, int ca0, int cb0, int with_x,
@@ -475,7 +460,7 @@ int launch_g(dmf_batch_s* b, kern_t k, int ntc, unsigned smem, int flags, int k_
              const Geom* geom = nullptr) {
     if (!k) return fail(DMF_E_SHAPE, "no Gram-engine kernel instantiation for this shape");
     PassArgs a;
-    a.g = geom ? *geom : b->gg;
+    a.g = geom ? *geom : b->p.gg;
     a.g.ntc = ntc;
     a.g.rg = kConsumers / ntc;
     a.fits = b->fits_dev;
@@ -485,13 +470,13 @@ int launch_g(dmf_batch_s* b, kern_t k, int ntc, unsigned smem, int flags, int k_
     a.ca0 = ca0; a.cb0 = cb0; a.with_x = with_x; a.pad = 0;
     a.mom_a = b->mom_dev; a.mom_m = b->mom_dev + b->mom_cap;
     // grid_mode 1 (alpha_inner_kernel): one warp per 32 / L samples of a fit, L = ktb_in lanes per sample
-    const int spw = 32 / b->ktb_in;
+    const int spw = 32 / b->p.ktb_in;
     dim3 grid = grid_mode == 1 ? dim3(b->n_active, (b->shape.N + spw - 1) / spw, 1) : dim3(a.g.n_parts, b->n_active, 1);
     if (grid_mode == 2) {
-        a.g.n_parts = b->n_parts_u;
-        a.g.n_groups = b->n_groups_u;
-        if (b->n_parts_u != b->gg.n_parts) a.g.part_stride = 8;
-        grid = dim3(b->n_parts_u, b->n_active, 1);
+        a.g.n_parts = b->p.n_parts_u;
+        a.g.n_groups = b->p.n_groups_u;
+        if (b->p.n_parts_u != b->p.gg.n_parts) a.g.part_stride = 8;
+        grid = dim3(b->p.n_parts_u, b->n_active, 1);
     }
     if (grid_mode == 1) a.g.fit_major = 0;
     else if (a.g.fit_major) {
@@ -642,6 +627,7 @@ int dmf_batch_create(dmf_handle_t h, const dmf_shape_t* shape, const dmf_fit_des
     dmf_batch_s* b = new dmf_batch_s;
     b->h = h;
     b->shape = s;
+    b->p = p;
     b->multmode = n_mult ? 1 : 0;
     b->launches = 0;
     b->pinned = nullptr;
@@ -654,99 +640,40 @@ int dmf_batch_create(dmf_handle_t h, const dmf_shape_t* shape, const dmf_fit_des
     b->fits_host = host;
     b->stats_local = p.gram_ok ? reinterpret_cast<double*>(base + p.off_stats) : nullptr;
     b->stats_global = p.gram_ok ? reinterpret_cast<double*>(base + p.off_gstats) : nullptr;
-    b->stats_doubles = p.per_fit_stats / 8; b->stats_gbx = p.stats_gbx; b->stats_scal = p.stats_scal;
-    Geom& g = b->g;
-    g.M = s.M; g.N = s.N; g.K = s.K; g.nu = s.n_u; g.Kt = s.K + s.n_u;
-    g.ldx = s.ldx; g.ldd = s.ldd; g.ldr = s.K ? s.ldr : 0; g.ldu = s.ldu;
-    g.Kp = p.Kp; g.nup = p.nup; g.rpt = p.rpt;
-    g.uslot_bytes = s.u_slot * (s.dtype == DMF_F64 ? 8 : 4);
-    g.tile_rows = p.tile_rows; g.n_tiles = p.n_tiles;
-    g.ntc = p.ntc_alpha; g.rg = kConsumers / p.ntc_alpha;
-    g.n_parts = p.n_parts; g.n_groups = p.n_groups; g.part_stride = p.part_stride;
-    g.offX = p.offX; g.offD = p.offD; g.offR = p.offR; g.offU = p.offU; g.offUp = p.offUp; g.stage_bytes = p.stage_bytes;
-    g.row_bulk = p.row_bulk; g.mode = s.mode; g.gather = gather ? 1 : 0;
-    g.fit_major = 0; g.multmode = 0; g.stages = kStages;
-    {
-        const unsigned sT = s.dtype == DMF_F64 ? 8 : 4, sW = s.wtype == DMF_W_U16 ? 2 : sT;
-        g.tile_tx[0] = (unsigned)(p.tile_rows * s.ldx * sT);
-        g.tile_tx[1] = (unsigned)(p.tile_rows * s.ldd * sW);
-        g.tile_tx[2] = s.K ? (unsigned)(p.tile_rows * s.ldr * sT) : 0u;
-        g.tile_tx[3] = g.tile_tx[4] = (unsigned)(p.tile_rows * s.ldu * sT);
-    }
-    b->ktb = p.ktb; b->c_alpha = p.c_alpha; b->kb = p.kb; b->nub = p.nub; b->c_u = p.c_u;
-    b->ntc_alpha = p.ntc_alpha; b->ntc_u = p.ntc_u;
-    b->smem_alpha = p.smem_alpha; b->smem_u = p.smem_u; b->smem_cost = p.smem_cost; b->occ = p.occ;
     b->fits_dev = reinterpret_cast<FitDev*>(base + p.off_fits);
     b->states_dev = reinterpret_cast<FitState*>(base + p.off_states);
-    b->gram_ok = p.gram_ok;
-    b->engine = p.gram_ok ? DMF_ENGINE_GRAM : DMF_ENGINE_STREAM;      // multiplicity form implies gram (checked above)
-    b->fused_ok = (p.fused_ok && !gather && !n_mult) ? 1 : 0;
     b->fused_pending = 0;
-    if (b->fused_ok) {
-        b->kb_f = p.kb_f; b->nub_f = p.nub_f; b->s_f = p.s_f; b->smem_f = p.smem_f;
-        FusedArgs& fa = b->fa;
-        memset(&fa, 0, sizeof(fa));
-        fa.g = g;
-        fa.g.n_parts = p.n_parts_f; fa.g.n_groups = p.n_groups_f; fa.g.fit_major = 0; fa.g.multmode = 0;
-        fa.n_tiles = p.n_tiles_f;
-        fa.pitchX = p.f_pitchX; fa.pitchD = p.f_pitchD; fa.offD = p.f_offD; fa.offR = p.f_offR; fa.offU = p.f_offU; fa.offUp = p.f_offUp;
-        fa.stage_bytes = p.f_stage_bytes; fa.offStats = p.f_offStats; fa.offTab = p.f_offTab;
-        fa.zero_off = p.f_zero_off;
+    // what the plan leaves to the fits of the batch
+    Plan& bp = b->p;
+    for (Geom* q : {&bp.g, &bp.gg, &bp.gp1}) q->gather = gather ? 1 : 0;
+    bp.gg.multmode = bp.gp1.multmode = b->multmode;
+    bp.gg.fit_major = bp.gp1.fit_major = shared_inputs ? 1 : 0;
+    if (b->multmode) std::copy(bp.tx_mult, bp.tx_mult + kMaxSrc, bp.gg.tile_tx);
+    bp.p1_ok = b->multmode && p.p1_ok;
+    bp.fused_ok = p.fused_ok && !gather && !n_mult;
+    b->engine = p.gram_ok ? DMF_ENGINE_GRAM : DMF_ENGINE_STREAM;      // multiplicity form implies gram (checked above)
+    if (bp.fused_ok) {
         fused_kern_t kf = by_types_f(s, p.kb_f, p.nub_f, p.s_f);
         if (!kf || cudaFuncSetAttribute((const void*)kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_f) != cudaSuccess) {
             cudaGetLastError();
-            b->fused_ok = 0;
+            bp.fused_ok = 0;
         } else {
             b->engine = DMF_ENGINE_FUSED;
         }
     }
     if (p.gram_ok) {
-        Geom& q = b->gg;
-        q = g;
-        q.rpt = p.rpt_g;
-        q.tile_rows = p.tile_rows_g; q.n_tiles = p.n_tiles_g;
-        q.ntc = p.ntc_g; q.rg = kConsumers / p.ntc_g;
-        q.n_parts = p.n_parts_g; q.n_groups = p.n_groups_g;
-        q.offX = p.g_offX; q.offD = p.g_offD; q.offR = p.g_offR; q.offU = p.g_offU; q.offUp = p.g_offUp; q.stage_bytes = p.g_stage_bytes;
-        q.multmode = b->multmode;
-        q.stages = p.stages_g;
-        q.fit_major = shared_inputs ? 1 : 0;
-        const unsigned sT = s.dtype == DMF_F64 ? 8 : 4, sW = s.wtype == DMF_W_U16 ? 2 : sT;
-        q.tile_tx[0] = (unsigned)(p.tile_rows_g * s.ldx * sT);
-        q.tile_tx[1] = (unsigned)(p.tile_rows_g * s.ldd * sW);
-        q.tile_tx[2] = s.K ? (unsigned)(p.tile_rows_g * s.ldr * sT) : 0u;
-        q.tile_tx[3] = b->multmode ? (unsigned)(p.tile_rows_g * p.ng_g * 8) : (unsigned)(p.tile_rows_g * s.ldu * sT);
-        q.tile_tx[4] = b->multmode ? (unsigned)(p.tile_rows_g * 4) : 0u;
-        b->kb_g = p.kb_g; b->nub_g = p.nub_g; b->c_g = p.c_g; b->ntc_g = p.ntc_g; b->pb_g = p.pb_g; b->c_p = p.c_p; b->ntc_p = p.ntc_p;
-        b->ktb_in = p.ktb_in; b->smem_rg = p.smem_rg; b->smem_panel = p.smem_panel;
-        b->n_parts_u = p.n_parts_u; b->n_groups_u = p.n_groups_u;
-        b->p1_ok = (b->multmode && p.p1_ok) ? 1 : 0;
-        if (b->p1_ok) {
-            Geom& r = b->gp1;
-            r = q;
-            r.tile_rows = p.p1_tile_rows; r.n_tiles = p.p1_n_tiles; r.stages = p.p1_stages;
-            r.rpt = 1;                                  // unused by the panel kernel (it strides over the rows of a tile)
-            r.n_parts = std::min(q.n_parts, p.p1_n_tiles); r.n_groups = (r.n_parts + kGroup - 1) / kGroup;
-            r.offX = p.p1_offX; r.offD = p.p1_offD; r.offR = p.p1_offR; r.offU = p.p1_offU; r.offUp = p.p1_offUp; r.stage_bytes = p.p1_stage_bytes;
-            const unsigned sT1 = s.dtype == DMF_F64 ? 8 : 4, sW1 = s.wtype == DMF_W_U16 ? 2 : sT1;
-            r.tile_tx[0] = (unsigned)(p.p1_tile_rows * s.ldx * sT1);
-            r.tile_tx[1] = (unsigned)(p.p1_tile_rows * s.ldd * sW1);
-            r.tile_tx[2] = s.K ? (unsigned)(p.p1_tile_rows * s.ldr * sT1) : 0u;
-            r.tile_tx[3] = (unsigned)(p.p1_tile_rows * p.ng_g * 8);
-            r.tile_tx[4] = (unsigned)(p.p1_tile_rows * 4);
-            b->smem_p1 = p.p1_smem;
+        if ((long long)p.n_parts_u * 8 > (long long)std::max(p.g.n_parts, p.gg.n_parts) * p.g.part_stride ||
+            (long long)p.n_groups_u * 8 > (long long)std::max(p.g.n_groups, p.gg.n_groups) * p.g.part_stride) {
+            bp.n_parts_u = p.gg.n_parts; bp.n_groups_u = p.gg.n_groups;     // partial-sum buffers too small for the wide grid (tiny N): use the pass grid
         }
-        if ((long long)p.n_parts_u * 8 > (long long)std::max(p.n_parts, p.n_parts_g) * p.part_stride || (long long)p.n_groups_u * 8 > (long long)std::max(p.n_groups, p.n_groups_g) * p.part_stride) {
-            b->n_parts_u = p.n_parts_g; b->n_groups_u = p.n_groups_g;     // partial-sum buffers too small for the wide grid (tiny N): use the pass grid
-        }
-        if ((rc = set_smem(k_rowgram(b, 0), b->smem_rg)) || (rc = set_smem(k_rowgram(b, 1), b->smem_rg)) || (rc = set_smem(k_panel(b), b->smem_panel)) ||
-            (rc = set_smem(k_uinner(b), 0)) || (rc = set_smem(k_ainner(b), 0)) || (b->multmode && ((rc = set_smem(k_costcross(b), 0)) || (rc = set_smem(k_panel_u1(b), std::max(b->smem_panel, b->p1_ok ? b->smem_p1 : 0u)))))) {
+        if ((rc = set_smem(k_rowgram(b, 0), p.smem_rg)) || (rc = set_smem(k_rowgram(b, 1), p.smem_rg)) || (rc = set_smem(k_panel(b), p.smem_panel)) ||
+            (rc = set_smem(k_uinner(b), 0)) || (rc = set_smem(k_ainner(b), 0)) || (b->multmode && ((rc = set_smem(k_costcross(b), 0)) || (rc = set_smem(k_panel_u1(b), std::max(p.smem_panel, bp.p1_ok ? p.smem_p1 : 0u)))))) {
             delete b;
             return rc;
         }
     }
-    if ((rc = set_smem(k_cost(b, 0), b->smem_cost)) || (rc = set_smem(k_cost(b, 1), b->smem_cost)) || (rc = set_smem(k_alpha(b), b->smem_alpha)) ||
-        (rc = set_smem(k_u(b), b->smem_u))) {
+    if ((rc = set_smem(k_cost(b, 0), p.smem_cost)) || (rc = set_smem(k_cost(b, 1), p.smem_cost)) || (rc = set_smem(k_alpha(b), p.smem_alpha)) ||
+        (rc = set_smem(k_u(b), p.smem_u))) {
         delete b;
         return rc;
     }
@@ -775,15 +702,16 @@ int dmf_batch_destroy(dmf_batch_t b) {
 
 int dmf_batch_geometry(dmf_batch_t b, int32_t* ctas_per_fit, int32_t* tile_rows, int32_t* smem_bytes) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
+    const Plan& p = b->p;
     if (b->engine == DMF_ENGINE_FUSED) {
-        if (ctas_per_fit) *ctas_per_fit = b->fa.g.n_parts;
-        if (tile_rows) *tile_rows = fused_cfg_rows(b->s_f);
-        if (smem_bytes) *smem_bytes = (int32_t)b->smem_f;
+        if (ctas_per_fit) *ctas_per_fit = p.fa.g.n_parts;
+        if (tile_rows) *tile_rows = p.fc.rows;
+        if (smem_bytes) *smem_bytes = (int32_t)p.smem_f;
         return DMF_OK;
     }
-    if (ctas_per_fit) *ctas_per_fit = b->engine == DMF_ENGINE_GRAM ? b->gg.n_parts : b->g.n_parts;
-    if (tile_rows) *tile_rows = b->engine == DMF_ENGINE_GRAM ? b->gg.tile_rows : b->g.tile_rows;
-    if (smem_bytes) *smem_bytes = b->engine == DMF_ENGINE_GRAM ? (int32_t)std::max(b->smem_rg, b->smem_panel) : (int32_t)std::max(b->smem_alpha, b->smem_u);
+    if (ctas_per_fit) *ctas_per_fit = b->engine == DMF_ENGINE_GRAM ? p.gg.n_parts : p.g.n_parts;
+    if (tile_rows) *tile_rows = b->engine == DMF_ENGINE_GRAM ? p.gg.tile_rows : p.g.tile_rows;
+    if (smem_bytes) *smem_bytes = b->engine == DMF_ENGINE_GRAM ? (int32_t)std::max(p.smem_rg, p.smem_panel) : (int32_t)std::max(p.smem_alpha, p.smem_u);
     return DMF_OK;
 }
 
@@ -791,35 +719,35 @@ int dmf_pass_init(dmf_batch_t b, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
     b->t_hi = 0;
     if (b->n_active != b->shape.n_fits) { int rc0 = upload_fits(b, nullptr, (cudaStream_t)stream); if (rc0) return rc0; }
-    return launch(b, k_cost(b, 1), b->ntc_alpha, b->smem_cost, kFlagInitial, 0, 0.0, (cudaStream_t)stream);
+    return launch(b, k_cost(b, 1), b->p.ntc_alpha, b->p.smem_cost, kFlagInitial, 0, 0.0, (cudaStream_t)stream);
 }
 int dmf_pass_cost(dmf_batch_t b, double tol, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    return launch(b, k_cost(b, 0), b->ntc_alpha, b->smem_cost, 0, 0, tol, (cudaStream_t)stream);
+    return launch(b, k_cost(b, 0), b->p.ntc_alpha, b->p.smem_cost, 0, 0, tol, (cudaStream_t)stream);
 }
 int dmf_pass_u(dmf_batch_t b, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
     b->t_hi += 1;     // keeps the momentum-table bound valid if Gram-engine steps follow on the same batch
-    return launch(b, k_u(b), b->ntc_u, b->smem_u, 0, 0, 0.0, (cudaStream_t)stream);
+    return launch(b, k_u(b), b->p.ntc_u, b->p.smem_u, 0, 0, 0.0, (cudaStream_t)stream);
 }
 int dmf_pass_alpha(dmf_batch_t b, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
     if (b->shape.mode == DMF_MODE_PURITY) return fail(DMF_E_STATE, "purity batches use dmf_pass_fw");
-    return launch(b, k_alpha(b), b->ntc_alpha, b->smem_alpha, 0, 0, 0.0, (cudaStream_t)stream);
+    return launch(b, k_alpha(b), b->p.ntc_alpha, b->p.smem_alpha, 0, 0, 0.0, (cudaStream_t)stream);
 }
 int dmf_pass_fw(dmf_batch_t b, int32_t k_inner, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
     if (b->shape.mode != DMF_MODE_PURITY) return fail(DMF_E_STATE, "Frank-Wolfe steps need a purity batch");
-    return launch(b, k_alpha(b), b->ntc_alpha, b->smem_alpha, kFlagFW, k_inner, 0.0, (cudaStream_t)stream);
+    return launch(b, k_alpha(b), b->p.ntc_alpha, b->p.smem_alpha, kFlagFW, k_inner, 0.0, (cudaStream_t)stream);
 }
 
 int dmf_batch_set_engine(dmf_batch_t b, int32_t engine) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
     if (engine != DMF_ENGINE_STREAM && engine != DMF_ENGINE_GRAM && engine != DMF_ENGINE_FUSED) return fail(DMF_E_ARG, "engine must be DMF_ENGINE_STREAM, DMF_ENGINE_GRAM or DMF_ENGINE_FUSED");
-    if (engine == DMF_ENGINE_FUSED && !b->fused_ok)
+    if (engine == DMF_ENGINE_FUSED && !b->p.fused_ok)
         return fail(DMF_E_SHAPE, "the fused engine needs FP64 storage, n_u <= 2, K <= 8, N <= 256, four U slots, no row gather and a weight pitch of a multiple of 16 bytes");
     if (b->fused_pending) return fail(DMF_E_STATE, "the cost of the current iterate is pending (dmf_fused_finish) - engines can be switched after it");
-    if (engine == DMF_ENGINE_GRAM && !b->gram_ok)
+    if (engine == DMF_ENGINE_GRAM && !b->p.gram_ok)
         return fail(DMF_E_SHAPE, "the Gram-form engine supports n_u <= 4 (n_u <= 8 when K <= 6) and needs its tile to fit in shared memory");
     if (engine == DMF_ENGINE_STREAM && b->multmode) return fail(DMF_E_STATE, "fits in multiplicity form run on the Gram-form engine only");
     b->engine = engine;
@@ -833,76 +761,77 @@ int dmf_batch_get_engine(dmf_batch_t b, int32_t* engine) {
 
 int dmf_gram_rowgram(dmf_batch_t b, int32_t initial, double tol, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
     if (initial) {
         b->t_hi = 0;
         b->fused_pending = 0;
         if (b->n_active != b->shape.n_fits) { int rc0 = upload_fits(b, nullptr, (cudaStream_t)stream); if (rc0) return rc0; }
     }
-    int rc = launch_g(b, k_rowgram(b, initial ? 1 : 0), b->ntc_g, b->smem_rg, initial ? kFlagInitial : 0, 0, tol, 0, 0, 0, 0, (cudaStream_t)stream);
+    int rc = launch_g(b, k_rowgram(b, initial ? 1 : 0), b->p.ntc_g, b->p.smem_rg, initial ? kFlagInitial : 0, 0, tol, 0, 0, 0, 0, (cudaStream_t)stream);
     if (rc || !b->multmode) return rc;
     // multiplicity form: the per-position cost terms and the set-up / termination logic
-    return launch_g(b, k_costcross(b), b->ntc_g, 0, initial ? kFlagInitial : 0, 0, tol, 0, 0, 0, 2, (cudaStream_t)stream);
+    return launch_g(b, k_costcross(b), b->p.ntc_g, 0, initial ? kFlagInitial : 0, 0, tol, 0, 0, 0, 2, (cudaStream_t)stream);
 }
 int dmf_gram_u_inner(dmf_batch_t b, int32_t n_iter2, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
     if (b->fused_pending) return fail(DMF_E_STATE, "the row statistics are stale after dmf_fused_outer: dmf_fused_finish first");
     if (n_iter2 < 0) return fail(DMF_E_ARG, "negative iteration count");
     b->t_hi += n_iter2;
     int rc = ensure_mom(b, b->t_hi, (cudaStream_t)stream);
     if (rc) return rc;
-    rc = launch_g(b, k_uinner(b), b->ntc_g, 0, 0, n_iter2, 0.0, 0, 0, 0, 2, (cudaStream_t)stream);
+    rc = launch_g(b, k_uinner(b), b->p.ntc_g, 0, 0, n_iter2, 0.0, 0, 0, 0, 2, (cudaStream_t)stream);
     if (rc || !b->multmode) return rc;
-    return launch_g(b, k_usum(b), b->ntc_g, 0, 0, 0, 0.0, 0, 0, 0, 2, (cudaStream_t)stream);      // per-source-row sums for the panel pass
+    return launch_g(b, k_usum(b), b->p.ntc_g, 0, 0, 0, 0.0, 0, 0, 0, 2, (cudaStream_t)stream);      // per-source-row sums for the panel pass
 }
 int dmf_gram_panels(dmf_batch_t b, int32_t known_block, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
-    const int nR = b->gg.Kp >> 1, nU = b->gg.nup >> 1, nb = b->pb_g / 2;
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
+    const Plan& p = b->p;
+    const int nR = p.gg.Kp >> 1, nU = p.gg.nup >> 1, nb = p.pb_g / 2;
     const int ca_lo = known_block ? 0 : nR, ca_hi = known_block ? nR : nR + nU;
     const int cb_hi = known_block ? nR : nR + nU;
     int rc;
     const bool u1 = b->multmode && !known_block && b->shape.n_u == 1;
-    const bool own = u1 && b->p1_ok;                    // smaller tiles, two CTAs per SM
+    const bool own = u1 && p.p1_ok;                    // smaller tiles, two CTAs per SM
     for (int ca = ca_lo; ca < ca_hi; ++ca)
         for (int cb = 0; cb < cb_hi; cb += nb)
-            if ((rc = launch_g(b, u1 ? k_panel_u1(b) : k_panel(b), b->ntc_p, own ? b->smem_p1 : b->smem_panel, 0, b->nub_g, 0.0,
-                               ca, cb, cb == 0 ? 1 : 0, 0, (cudaStream_t)stream, own ? &b->gp1 : nullptr))) return rc;
+            if ((rc = launch_g(b, u1 ? k_panel_u1(b) : k_panel(b), p.ntc_p, own ? p.smem_p1 : p.smem_panel, 0, p.nub_g, 0.0,
+                               ca, cb, cb == 0 ? 1 : 0, 0, (cudaStream_t)stream, own ? &p.gp1 : nullptr))) return rc;
     return DMF_OK;
 }
 int dmf_gram_alpha_inner(dmf_batch_t b, int32_t n_iter2, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
     if (n_iter2 < 0) return fail(DMF_E_ARG, "negative iteration count");
     // alpha steps never run ahead of the U steps by more than one call; cover t_hi + n_iter2 to be independent of call order
     int rc = ensure_mom(b, b->t_hi + n_iter2, (cudaStream_t)stream);
     if (rc) return rc;
-    return launch_g(b, k_ainner(b), b->ntc_p, 0, b->shape.mode == DMF_MODE_PURITY ? kFlagFW : 0, n_iter2, 0.0, 0, 0, 0, 1, (cudaStream_t)stream);
+    return launch_g(b, k_ainner(b), b->p.ntc_p, 0, b->shape.mode == DMF_MODE_PURITY ? kFlagFW : 0, n_iter2, 0.0, 0, 0, 0, 1, (cudaStream_t)stream);
 }
 int dmf_batch_set_sharded(dmf_batch_t b, int32_t on, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "row sharding needs the Gram-form engine (n_u <= 4, or n_u <= 8 with K <= 6)");
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "row sharding needs the Gram-form engine (n_u <= 4, or n_u <= 8 with K <= 6)");
     if (b->multmode) return fail(DMF_E_STATE, "row sharding and the multiplicity form are not combined");
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t per = b->stats_doubles;
+    const size_t per = b->p.per_fit_stats / 8;
     for (int i = 0; i < b->shape.n_fits; ++i) {
         FitDev& f = b->fits_host[i];
         double* src = on ? b->stats_global + per * i : b->stats_local + per * i;
-        f.rgram = src; f.rgbx = src + b->stats_gbx; f.rscal = src + b->stats_scal;
+        f.rgram = src; f.rgbx = src + b->p.stats_gbx; f.rscal = src + b->p.stats_scal;
     }
     int rc = upload_fits(b, nullptr, st);
     if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(st));
     b->sharded = on ? 1 : 0;
-    b->engine = b->fused_ok ? DMF_ENGINE_FUSED : DMF_ENGINE_GRAM;
+    b->engine = b->p.fused_ok ? DMF_ENGINE_FUSED : DMF_ENGINE_GRAM;
     return DMF_OK;
 }
 int dmf_batch_stats_buffers(dmf_batch_t b, void** local_dev, void** global_dev, int64_t* doubles_per_fit, int64_t* scal_offset) {
     if (!b || !local_dev || !global_dev || !doubles_per_fit || !scal_offset) return fail(DMF_E_ARG, "NULL argument");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
     *local_dev = b->stats_local; *global_dev = b->stats_global;
-    *doubles_per_fit = (int64_t)b->stats_doubles; *scal_offset = (int64_t)b->stats_scal;
+    *doubles_per_fit = (int64_t)(b->p.per_fit_stats / 8); *scal_offset = (int64_t)b->p.stats_scal;
     return DMF_OK;
 }
 int dmf_gram_finalize_cost(dmf_batch_t b, int32_t initial, double tol, void* stream) {
@@ -910,7 +839,7 @@ int dmf_gram_finalize_cost(dmf_batch_t b, int32_t initial, double tol, void* str
     if (!b->sharded) return fail(DMF_E_STATE, "dmf_gram_finalize_cost is the second half of dmf_gram_rowgram on row-sharded batches");
     PassArgs a;
     memset(&a, 0, sizeof(a));
-    a.g = b->gg;
+    a.g = b->p.gg;
     a.fits = b->fits_dev;
     a.k_inner = b->n_active;
     a.flags = (initial ? kFlagInitial : 0) | (b->shape.dtype == DMF_F32 ? kFlagF32 : 0);
@@ -923,8 +852,8 @@ int dmf_gram_finalize_cost(dmf_batch_t b, int32_t initial, double tol, void* str
 
 int dmf_batch_peer_bytes(dmf_batch_t b, int32_t world, size_t* bytes) {
     if (!b || !bytes || world < 1) return fail(DMF_E_ARG, "bad argument");
-    if (!b->gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
-    const size_t slot = b->stats_doubles * b->shape.n_fits;
+    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
+    const size_t slot = b->p.per_fit_stats / 8 * b->shape.n_fits;
     *bytes = align_up(2 * (size_t)world * slot * 8, 256) + align_up(2 * (size_t)world * 4, 256);
     return DMF_OK;
 }
@@ -944,7 +873,7 @@ int dmf_batch_set_peers(dmf_batch_t b, int32_t rank, int32_t world, const void* 
     CUDA_TRY(cudaMemsetAsync(b->xchg_ticket, 0, 256, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     b->peer_rank = rank; b->peer_world = world;
-    b->peer_slot_stride = (long long)(b->stats_doubles * b->shape.n_fits);
+    b->peer_slot_stride = (long long)(b->p.per_fit_stats / 8 * b->shape.n_fits);
     b->peer_flag_off = (long long)align_up(2 * (size_t)world * b->peer_slot_stride * 8, 256);
     b->xchg_epoch = 0;      // the caller zeroes the symmetric buffers (flags) before the first exchange
     return DMF_OK;
@@ -957,8 +886,8 @@ int dmf_gram_exchange(dmf_batch_t b, int32_t which, void* stream) {
     a.peers = b->peers_dev;
     a.local = b->stats_local; a.global = b->stats_global;
     a.ticket = b->xchg_ticket;
-    a.per_fit = (long long)b->stats_doubles; a.slot_stride = b->peer_slot_stride; a.flag_off = b->peer_flag_off;
-    a.scal_off = (long long)b->stats_scal;
+    a.per_fit = (long long)(b->p.per_fit_stats / 8); a.slot_stride = b->peer_slot_stride; a.flag_off = b->peer_flag_off;
+    a.scal_off = (long long)b->p.stats_scal;
     a.n_fits = b->shape.n_fits; a.rank = b->peer_rank; a.world = b->peer_world; a.which = which;
     a.epoch_dev = b->xchg_ticket + 16;            // the exchange count lives on the device: CUDA-graph replays advance it
     ++b->xchg_epoch;
@@ -993,20 +922,21 @@ int dmf_gram_outer(dmf_batch_t b, int32_t n_iter2, double tol, void* stream) {
 
 int dmf_fused_pass(dmf_batch_t b, int32_t n_iter2, double tol, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->fused_ok) return fail(DMF_E_SHAPE, "no fused-engine instantiation for this shape / layout");
+    if (!b->p.fused_ok) return fail(DMF_E_SHAPE, "no fused-engine instantiation for this shape / layout");
     if (b->multmode) return fail(DMF_E_STATE, "the fused engine does not run multiplicity-form batches");
     if (n_iter2 < 1 || n_iter2 > kFusedMaxInner) return fail(DMF_E_ARG, "the fused pass runs 1 .. 64 update_u iterations per visit");
     b->t_hi += n_iter2;
     int rc = ensure_mom(b, b->t_hi + n_iter2, (cudaStream_t)stream);
     if (rc) return rc;
-    fused_kern_t k = by_types_f(b->shape, b->kb_f, b->nub_f, b->s_f);
-    FusedArgs a = b->fa;
+    const Plan& p = b->p;
+    fused_kern_t k = by_types_f(b->shape, p.kb_f, p.nub_f, p.s_f);
+    FusedArgs a = p.fa;
     a.fits = b->fits_dev;
     a.n_iter2 = n_iter2;
     a.flags = b->sharded ? kFlagPartial : 0;      // row-sharded: publish this GPU's sums, dmf_fused_alpha_commit decides on the reduced ones
     a.tol = tol;
     a.mom_a = b->mom_dev; a.mom_m = b->mom_dev + b->mom_cap;
-    k<<<dim3(a.g.n_parts, b->n_active, 1), fused_cfg_threads(b->s_f, b->nub_f), b->smem_f, (cudaStream_t)stream>>>(a);
+    k<<<dim3(a.g.n_parts, b->n_active, 1), p.fc.threads, p.smem_f, (cudaStream_t)stream>>>(a);
     CUDA_TRY(cudaGetLastError());
     b->launches++;
     b->fused_pending = 1;
@@ -1020,11 +950,11 @@ int dmf_fused_outer(dmf_batch_t b, int32_t n_iter2, double tol, void* stream) {
 }
 int dmf_fused_alpha_commit(dmf_batch_t b, int32_t n_iter2, double tol, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->sharded || !b->fused_ok) return fail(DMF_E_STATE, "dmf_fused_alpha_commit follows dmf_fused_pass on a row-sharded batch");
+    if (!b->sharded || !b->p.fused_ok) return fail(DMF_E_STATE, "dmf_fused_alpha_commit follows dmf_fused_pass on a row-sharded batch");
     if (n_iter2 < 0) return fail(DMF_E_ARG, "negative iteration count");
     int rc = ensure_mom(b, b->t_hi + n_iter2, (cudaStream_t)stream);
     if (rc) return rc;
-    return launch_g(b, k_ainner(b), b->ntc_p, 0, (b->shape.mode == DMF_MODE_PURITY ? kFlagFW : 0) | kFlagFusedCommit, n_iter2, tol, 0, 0, 0, 1,
+    return launch_g(b, k_ainner(b), b->p.ntc_p, 0, (b->shape.mode == DMF_MODE_PURITY ? kFlagFW : 0) | kFlagFusedCommit, n_iter2, tol, 0, 0, 0, 1,
                     (cudaStream_t)stream);
 }
 int dmf_fused_finish(dmf_batch_t b, double tol, void* stream) {
@@ -1155,7 +1085,8 @@ namespace {
 
 struct WlsPlan {
     int slab, ntc, rg, tile_rows, n_tiles, n_parts, n_groups, part_stride, Kz, nblk;
-    unsigned offX, offD, offR, offU, stage_bytes, smem;
+    StageLayout stage;    // X, D, R1, R2
+    unsigned smem;
     size_t off_fit, off_tickets, off_part, off_gpart, off_mom, off_status, ws_bytes;
 };
 
@@ -1168,32 +1099,28 @@ int make_wls_plan(const dmf_handle_s* h, const dmf_wls_desc_t& d, WlsPlan& p) {
     if ((d.ldx | d.ldd | (d.K ? d.ldr : 0) | (d.K2 ? d.ldr2 : 0)) & 1) return fail(DMF_E_SHAPE, "wls: row pitches must be even (zero padded)");
     const size_t sT = d.dtype == DMF_F64 ? 8 : 4, sW = d.wtype == DMF_W_U16 ? 2 : sT;
     p.slab = std::min<int>(d.N, kConsumers);            // sample columns per launch (one column per thread)
-    p.ntc = next_pow2(p.slab);
+    p.ntc = pow2ceil(p.slab);
     p.rg = kConsumers / p.ntc;
     const size_t px = d.ldx * sT, pd = d.ldd * sW, pr = d.K ? d.ldr * sT : 0, pu = d.K2 ? d.ldr2 * sT : 0;
     int ra = 1;
     while (ra < 16 && ((ra * px) % 16 || (ra * pd) % 16 || (ra * pr) % 16 || (ra * pu) % 16)) ra <<= 1;
     const size_t budget = std::min<size_t>((size_t)h->max_smem_optin, 200 * 1024) - kCtlBytes - 2048;
-    auto a128 = [](size_t v) { return align_up(v, 128); };
+    const size_t rows_w[kMaxSrc] = {px, pd, pr, pu, 0};
     long long tr = 0;
     for (long long cand = (long long)p.rg * 8; cand >= 1; cand >>= 1) {
         if (cand % ra) continue;
-        if ((a128(cand * px) + a128(cand * pd) + a128(cand * pr) + a128(cand * pu)) * kStages <= budget) { tr = cand; break; }
+        if (stage_layout(cand, rows_w, rows_w).bytes * kStages <= budget) { tr = cand; break; }
     }
     if (!tr) return fail(DMF_E_SHAPE, "wls: one row tile does not fit in shared memory");
     p.tile_rows = (int)tr;
     p.n_tiles = (int)((d.M + tr - 1) / tr);
-    p.offX = 0;
-    p.offD = (unsigned)a128(tr * px);
-    p.offR = p.offD + (unsigned)a128(tr * pd);
-    p.offU = p.offR + (unsigned)a128(tr * pr);
-    p.stage_bytes = p.offU + (unsigned)a128(tr * pu);
+    p.stage = stage_layout(tr, rows_w, rows_w);
     p.n_parts = std::min(p.n_tiles, h->sm_count);
     p.n_groups = (p.n_parts + kGroup - 1) / kGroup;
     p.part_stride = kWlsBlock * kWlsBlock * p.slab;
     p.Kz = d.K + d.K2 + 2;
     p.nblk = (p.Kz + kWlsBlock - 1) / kWlsBlock;
-    p.smem = (unsigned)std::max<size_t>(kCtlBytes + (size_t)kStages * p.stage_bytes, kCtlBytes + (size_t)p.part_stride * 8 + 256);
+    p.smem = (unsigned)std::max<size_t>(kCtlBytes + (size_t)kStages * p.stage.bytes, kCtlBytes + (size_t)p.part_stride * 8 + 256);
     if (p.smem > (unsigned)h->max_smem_optin) return fail(DMF_E_SHAPE, "wls: shared-memory plan exceeds the device limit");
     p.off_fit = 0;
     p.off_tickets = 256;
@@ -1254,15 +1181,11 @@ int dmf_wls_fit(dmf_handle_t h, const dmf_wls_desc_t* dd, void* ws, size_t ws_by
         Geom& g = a.g;
         g.M = d.M; g.N = ns; g.K = d.K; g.nu = d.K2; g.Kt = d.K + d.K2;
         g.ldx = d.ldx; g.ldd = d.ldd; g.ldr = d.K ? d.ldr : 0; g.ldu = d.K2 ? d.ldr2 : 0;
-        g.tile_rows = p.tile_rows; g.n_tiles = p.n_tiles; g.ntc = next_pow2(ns); g.rg = kConsumers / g.ntc;
+        g.tile_rows = p.tile_rows; g.n_tiles = p.n_tiles; g.ntc = pow2ceil(ns); g.rg = kConsumers / g.ntc;
         // rows of a tile are walked with stride rg: a narrower last slab only changes the thread mapping
         g.n_parts = p.n_parts; g.n_groups = p.n_groups; g.part_stride = p.part_stride;
-        g.offX = p.offX; g.offD = p.offD; g.offR = p.offR; g.offU = p.offU; g.offUp = p.offU; g.stage_bytes = p.stage_bytes;
-        g.tile_tx[0] = (unsigned)(p.tile_rows * d.ldx * sT);
-        g.tile_tx[1] = (unsigned)(p.tile_rows * d.ldd * sW);
-        g.tile_tx[2] = d.K ? (unsigned)(p.tile_rows * d.ldr * sT) : 0u;
-        g.tile_tx[3] = d.K2 ? (unsigned)(p.tile_rows * d.ldr2 * sT) : 0u;
-        g.tile_tx[4] = 0;
+        set_stages(g, p.stage);
+        g.offUp = g.offU;
         a.fits = reinterpret_cast<const FitDev*>(base + p.off_fit);
         a.mom = reinterpret_cast<double*>(base + p.off_mom);
         a.Kfull = d.K + d.K2;

@@ -91,19 +91,21 @@ struct FusedCfg {
     // FU = 7 at S = 4).  Fills are in tile order, so a stride of at most NS tiles guarantees it.
     static_assert((FU + UP - 1) / UP <= NS, "U-warp tile stride must not exceed the ring depth (parity waits)");
 };
-// host-side views of the same table (nub = unknown types of the instantiation)
-constexpr int fused_cfg_rows(int s) { return s == 4 ? 16 : 32; }
-constexpr int fused_cfg_stages(int s) { return s == 4 ? DMF_STAGES : (s == 2 ? 4 : 8); }
-constexpr int fused_cfg_threads(int s, int nub) { return 32 * (kFA + kFC + kFP + (s == 4 ? DMF_FU : (nub == 2 ? DMF_FU_NARROW2 : DMF_FU_NARROW))); }
-constexpr int fused_cfg_sgroups(int s) { return 8 / (fused_cfg_rows(s) / 8); }
-constexpr int fused_cfg_nstat(int s) { return s == 4 ? 2 : fused_cfg_stages(s); }
-// the host-side views must describe the kernel's own table
-#define DMF_CFG_CHECK(S_, N_)                                                                                                      \
-    static_assert(fused_cfg_rows(S_) == FusedCfg<S_, N_>::TR && fused_cfg_stages(S_) == FusedCfg<S_, N_>::NS &&                   \
-                  fused_cfg_threads(S_, N_) == FusedCfg<S_, N_>::THREADS && fused_cfg_sgroups(S_) == FusedCfg<S_, N_>::SG &&       \
-                  fused_cfg_nstat(S_) == FusedCfg<S_, N_>::NSTAT, "fused_cfg_* out of step with FusedCfg");
-DMF_CFG_CHECK(1, 1) DMF_CFG_CHECK(1, 2) DMF_CFG_CHECK(2, 1) DMF_CFG_CHECK(2, 2) DMF_CFG_CHECK(4, 1) DMF_CFG_CHECK(4, 2)
-#undef DMF_CFG_CHECK
+// The host's view of FusedCfg for the instantiated classes (S = 1, 2, 4; one or two unknown types)
+struct FusedShape { int rows, stages, threads, sgroups, nstat; };
+template <int S, int NUB>
+constexpr FusedShape fused_shape_of() { using C = FusedCfg<S, NUB>; return {C::TR, C::NS, C::THREADS, C::SG, C::NSTAT}; }
+inline FusedShape fused_shape(int s, int nub) {
+    switch (s * 10 + nub) {
+        case 11: return fused_shape_of<1, 1>();
+        case 12: return fused_shape_of<1, 2>();
+        case 21: return fused_shape_of<2, 1>();
+        case 22: return fused_shape_of<2, 2>();
+        case 41: return fused_shape_of<4, 1>();
+        case 42: return fused_shape_of<4, 2>();
+    }
+    return FusedShape{};
+}
 constexpr int kFusedMaxInner = 64;       // beyond this the U-warps would bound the pass: Gram engine instead
 constexpr unsigned kFusedCtlBytes = 2048;
 

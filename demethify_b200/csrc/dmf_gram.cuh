@@ -35,6 +35,12 @@ __device__ __forceinline__ float clip01(float v) { return fminf(fmaxf(v, 0.0f), 
 __host__ __device__ constexpr int ng_of(int nub) { return nub + nub * (nub + 1) / 2; }
 __host__ __device__ constexpr int pow2ceil(int v) { int p = 1; while (p < v) p <<= 1; return p; }
 __host__ __device__ constexpr int tri_index(int q, int q2, int nub) { return q * nub - q * (q - 1) / 2 + (q2 - q); }   // q <= q2
+// Minimum CTAs per SM of the rowgram and panel passes (__launch_bounds__); make_plan sizes their ring for the same occupancy.
+// C == 4 is rowgram4_kernel (one CTA per SM).
+__host__ __device__ constexpr int rowgram_min_blocks(int kb, int nub, int c, int rpt) {
+    return c != 4 && (kb + 2 * nub) * c + 2 * pow2ceil(rpt * ng_of(nub)) <= 56 ? 2 : 1;
+}
+__host__ __device__ constexpr int panel_min_blocks(int pa, int pb, int c) { return pa * (pb + 1) * c <= 40 ? 2 : 1; }
 
 // ------------------------------------------------------------------------------------------------
 // shared by cost_kernel-style epilogues: CTA partial [cost, ssq_rk, ssq_u, dmax] -> fit state
@@ -91,7 +97,7 @@ __device__ __forceinline__ void cost_state_update(const Geom& g, const FitDev& f
 // values [b (NUB) | H upper triangle] are summed over the column threads of a warp with the transposed butterfly and
 // written per warp:  rowgram[row][warp-in-row][NG]  (u_inner_kernel adds the <= 8 per-warp partials in fixed order).
 template <typename T, typename WT, int KB, int NUB, int C, int RPT, bool INITIAL>
-__global__ void __launch_bounds__(kThreads, ((KB + 2 * NUB) * C + 2 * pow2ceil(RPT * ng_of(NUB)) <= 56) ? 2 : 1) rowgram_kernel(const PassArgs a) {
+__global__ void __launch_bounds__(kThreads, rowgram_min_blocks(KB, NUB, C, RPT)) rowgram_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NG = ng_of(NUB);
     constexpr int NVP = pow2ceil(RPT * NG);
@@ -319,7 +325,7 @@ struct ColLoader {
 //  * the cost is assembled from  sum d c^2  (one FMA per element, per-thread accumulator) and the row statistics:
 //    sum_j d (c - u a_u)^2 = sum_j d c^2 - 2 u^T b + u^T H u  (writer lanes add the last two terms per row).
 template <typename T, typename WT, int KB, int NUB, int RPT, bool INITIAL>
-__global__ void __launch_bounds__(kThreads, 1) rowgram4_kernel(const PassArgs a) {
+__global__ void __launch_bounds__(kThreads, rowgram_min_blocks(KB, NUB, 4, RPT)) rowgram4_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int C = 4;
     constexpr int NG = ng_of(NUB);
@@ -869,7 +875,7 @@ __global__ void __launch_bounds__(kThreads) cost_cross_kernel(const PassArgs a) 
 // zb = PB entries starting at chunk a.cb0.  The last CTA scatters the totals (and their mirror images) into
 // gram[Kt][Kt][N] and, when a.with_x, gbx[Kt][N].
 template <typename T, typename WT, int PA, int PB, int C, bool MULT>
-__global__ void __launch_bounds__(kThreads, (PA * (PB + 1) * C <= 40) ? 2 : 1) gram_panel_kernel(const PassArgs a) {
+__global__ void __launch_bounds__(kThreads, panel_min_blocks(PA, PB, C)) gram_panel_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NA = PA / 2, NB = PB / 2;      // PA == 1 (NA == 0) exists for the MULT u block with a single unknown type only
     static_assert(PA >= 2 || MULT, "PA = 1 is a multiplicity-form instantiation");
@@ -1328,6 +1334,7 @@ __global__ void __launch_bounds__(32) alpha_inner_kernel(const PassArgs a) {
     }
 }
 
+#ifndef DMF_INST_BODY     // launched by dmf_api.cu only: the instantiation units leave these kernels out
 // ------------------------------------------------------------------------------------------------
 // CpG rows sharded over GPUs: the set-up / termination logic of the rowgram pass on the all-reduced sums
 // FitDev::rscal = [cost, ||R_trunc||^2, ||u||^2, max d_x] (deconvolution.py:192-204, :218-221).  One thread per fit.
@@ -1425,5 +1432,6 @@ static __global__ void __launch_bounds__(kThreads) peer_allreduce_kernel(const X
         *a.epoch_dev = epoch;
     }
 }
+#endif  // DMF_INST_BODY
 
 }  // namespace dmf

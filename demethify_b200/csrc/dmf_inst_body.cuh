@@ -1,4 +1,7 @@
 // dmf_inst_body.cuh — included by dmf_inst_<tag>.cu with DMF_T, DMF_WT and DMF_TAG defined.
+#include <iterator>
+#include <utility>
+#define DMF_INST_BODY
 #include "dmf_inst.h"
 #include "dmf_kernels.cuh"
 #include "dmf_wls.cuh"
@@ -22,45 +25,42 @@ kern_t DMF_CAT(pick_alpha_, DMF_TAG)(int ktb, int, int c) {
     if (ktb == 32 && c == 1) return alpha_pass_kernel<DMF_T, DMF_WT, 32, 1>;
     return nullptr;
 }
-// U pass: (known bucket, unknown bucket) -> fixed (columns per thread, rows per thread per tile); see kUTable in dmf_api.cu
-kern_t DMF_CAT(pick_u_, DMF_TAG)(int kb, int nub, int) {
-#define DMF_U(KB_, NUB_, C_, RPT_) \
-    if (kb == KB_ && nub == NUB_) return u_pass_kernel<DMF_T, DMF_WT, KB_, NUB_, C_, RPT_>;
-    DMF_U(6, 2, 2, 4) DMF_U(8, 2, 2, 4) DMF_U(8, 8, 2, 1) DMF_U(16, 2, 2, 4) DMF_U(16, 8, 2, 1) DMF_U(16, 16, 1, 1)
-    DMF_U(32, 2, 1, 4) DMF_U(32, 8, 1, 1) DMF_U(32, 32, 1, 1)
-#undef DMF_U
-    return nullptr;
+// U pass and rowgram pass: the entries of kUTable / kRowgramTable (dmf_inst.h)
+template <typename T, typename WT, size_t... I>
+kern_t pick_u_in(int kb, int nub, std::index_sequence<I...>) {
+    kern_t k = nullptr;
+    ((kb == kUTable[I].kb && nub == kUTable[I].nub ? (void)(k = u_pass_kernel<T, WT, kUTable[I].kb, kUTable[I].nub, kUTable[I].c, kUTable[I].rpt>)
+                                                   : (void)0), ...);
+    return k;
 }
-// Gram engine (dmf_gram.cuh).  rowgram: (known bucket, unknown bucket) -> fixed (columns per thread, rows per thread per tile);
-// see kGramTable in dmf_api.cu
-kern_t DMF_CAT(pick_rowgram_, DMF_TAG)(int kb, int nub, int flags) {
-    const int initial = flags & 1, c4 = flags & 2;
-#define DMF_G4(KB_, NUB_, RPT_)                                                                              \
-    if (c4 && kb == KB_ && nub == NUB_)                                                                      \
-        return initial ? (kern_t)rowgram4_kernel<DMF_T, DMF_WT, KB_, NUB_, RPT_, true> : (kern_t)rowgram4_kernel<DMF_T, DMF_WT, KB_, NUB_, RPT_, false>;
-    DMF_G4(0, 1, 4) DMF_G4(0, 2, 4) DMF_G4(0, 4, 2) DMF_G4(0, 8, 1) DMF_G4(6, 1, 4) DMF_G4(6, 2, 4) DMF_G4(6, 4, 2) DMF_G4(6, 8, 1)
-#undef DMF_G4
-    if (c4) return nullptr;
-#define DMF_G(KB_, NUB_, C_, RPT_)                                                                           \
-    if (kb == KB_ && nub == NUB_)                                                                            \
-        return initial ? (kern_t)rowgram_kernel<DMF_T, DMF_WT, KB_, NUB_, C_, RPT_, true> : (kern_t)rowgram_kernel<DMF_T, DMF_WT, KB_, NUB_, C_, RPT_, false>;
-    DMF_G(0, 1, 2, 4) DMF_G(0, 2, 2, 3) DMF_G(0, 4, 2, 2)
-    DMF_G(6, 1, 2, 4) DMF_G(6, 2, 2, 3) DMF_G(6, 4, 2, 2)
-    DMF_G(16, 1, 2, 4) DMF_G(16, 2, 2, 3) DMF_G(16, 4, 2, 2)
-    DMF_G(32, 1, 1, 4) DMF_G(32, 2, 1, 3) DMF_G(32, 4, 1, 2)
-#undef DMF_G
-    return nullptr;
+kern_t DMF_CAT(pick_u_, DMF_TAG)(int kb, int nub, int) {
+    return pick_u_in<DMF_T, DMF_WT>(kb, nub, std::make_index_sequence<std::size(kUTable)>());
+}
+template <typename T, typename WT, bool INITIAL, int I>
+kern_t rowgram_at() {
+    constexpr KernEntry e = kRowgramTable[I];
+    if constexpr (e.c == 4) return rowgram4_kernel<T, WT, e.kb, e.nub, e.rpt, INITIAL>;
+    else return rowgram_kernel<T, WT, e.kb, e.nub, e.c, e.rpt, INITIAL>;
+}
+template <typename T, typename WT, bool INITIAL, size_t... I>
+kern_t pick_rowgram_in(int kb, int nub, std::index_sequence<I...>) {
+    kern_t k = nullptr;
+    ((kb == kRowgramTable[I].kb && nub == kRowgramTable[I].nub ? (void)(k = rowgram_at<T, WT, INITIAL, I>()) : (void)0), ...);
+    return k;
+}
+kern_t DMF_CAT(pick_rowgram_, DMF_TAG)(int kb, int nub, int initial) {
+    constexpr auto all = std::make_index_sequence<std::size(kRowgramTable)>();
+    return initial ? pick_rowgram_in<DMF_T, DMF_WT, true>(kb, nub, all) : pick_rowgram_in<DMF_T, DMF_WT, false>(kb, nub, all);
 }
 // mult: 0 plain, 1 multiplicity form, 2 multiplicity form, u block of a single unknown type (PA = 1)
 kern_t DMF_CAT(pick_panel_, DMF_TAG)(int pb, int c, int mult) {
     if (mult == 2) return (pb == 8 && c == 4) ? (kern_t)gram_panel_kernel<DMF_T, DMF_WT, 1, 8, 4, true> : nullptr;
     if (mult) return (pb == 8 && c == 4) ? (kern_t)gram_panel_kernel<DMF_T, DMF_WT, 2, 8, 4, true> : nullptr;
     if (pb == 8 && c == 4) return gram_panel_kernel<DMF_T, DMF_WT, 2, 8, 4, false>;
-    if (pb == 8) return gram_panel_kernel<DMF_T, DMF_WT, 2, 8, 2, false>;
-    if (pb == 16) return gram_panel_kernel<DMF_T, DMF_WT, 2, 16, 1, false>;
+    if (pb == 16 && c == 1) return gram_panel_kernel<DMF_T, DMF_WT, 2, 16, 1, false>;
     return nullptr;
 }
-// which: 0 u_inner_kernel, 1 u_inner_mult_kernel, 2 cost_cross_kernel, 3 usum_kernel
+// which: 0 u_inner_kernel, 1 u_inner_mult_kernel, 2 cost_cross_kernel, 3 usum_kernel (the multiplicity form: nub <= 4)
 kern_t DMF_CAT(pick_uinner_, DMF_TAG)(int nub, int which, int) {
 #define DMF_UI(NUB_)                                                           \
     if (nub == NUB_) {                                                         \
@@ -69,9 +69,9 @@ kern_t DMF_CAT(pick_uinner_, DMF_TAG)(int nub, int which, int) {
         if (which == 3) return usum_kernel<DMF_T, NUB_>;                       \
         return cost_cross_kernel<DMF_T, NUB_>;                                 \
     }
-    DMF_UI(1) DMF_UI(2) DMF_UI(4) DMF_UI(8)
+    DMF_UI(1) DMF_UI(2) DMF_UI(4)
 #undef DMF_UI
-    return nullptr;
+    return nub == 8 && which == 0 ? (kern_t)u_inner_kernel<DMF_T, 8> : nullptr;
 }
 kern_t DMF_CAT(pick_ainner_, DMF_TAG)(int ktb, int, int) {
     if (ktb == 8) return alpha_inner_kernel<DMF_T, 8>;

@@ -206,9 +206,13 @@ __device__ __forceinline__ int alpha_row_of(const Geom& g, int i) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// Minimum CTAs per SM of the streaming passes (__launch_bounds__); make_plan sizes their ring for the same occupancy.
+__host__ __device__ constexpr int pass_min_blocks(int ktb) { return ktb <= 8 ? 2 : 1; }      // cost_kernel, alpha_pass_kernel
+__host__ __device__ constexpr int u_pass_min_blocks(int kb, int nub, int c) { return (kb + 2 * nub) * c <= 24 ? 2 : 1; }
+
 // cost / set-up pass
 template <typename T, typename WT, int KTB, int C, bool INITIAL>
-__global__ void __launch_bounds__(kThreads, (KTB <= 8) ? 2 : 1) cost_kernel(const PassArgs a) {
+__global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) cost_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NCH = KTB / 2;
     const Geom& g = a.g;
@@ -395,7 +399,7 @@ __device__ __forceinline__ void seg_reduce(double (&v)[NV], int L, int lane, int
 // U pass: u <- clip(u_t + ((d o (x - Rk a_k - u_g a_u)) a_u^T) / l_w, 0, 1),  u_t = u + beta (u - u_prev)
 // (u_g = u_t in update_u:88, u_g = u in unsupervised_deconv:163)
 template <typename T, typename WT, int KB, int NUB, int C, int RPT>
-__global__ void __launch_bounds__(kThreads, ((KB + 2 * NUB) * C <= 24) ? 2 : 1) u_pass_kernel(const PassArgs a) {
+__global__ void __launch_bounds__(kThreads, u_pass_min_blocks(KB, NUB, C)) u_pass_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NV = RPT * NUB;
     const Geom& g = a.g;
@@ -619,7 +623,7 @@ __device__ __forceinline__ bool project_simplex(double* v, int p) {
 
 // alpha pass: G = R^T (d o (x - R a_eval)); last CTA applies the projected-gradient or Frank-Wolfe step
 template <typename T, typename WT, int KTB, int C>
-__global__ void __launch_bounds__(kThreads, (KTB <= 8) ? 2 : 1) alpha_pass_kernel(const PassArgs a) {
+__global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) alpha_pass_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NCH = KTB / 2;
     const Geom& g = a.g;

@@ -123,6 +123,7 @@ __global__ void __launch_bounds__(kThreads, 1) wls_moments_kernel(const WlsArgs 
     }
 }
 
+#ifndef DMF_INST_BODY     // launched by dmf_api.cu only: the instantiation units leave this kernel out
 // Lawson-Hanson active-set NNLS on the centred normal equations, one thread per sample.
 // Third-party algorithm on the reference path: scipy.optimize.nnls (reached through sklearn, init_func.py:9).
 static __global__ void wls_nnls_kernel(const double* __restrict__ mom, int K, int N, long long M, double* __restrict__ out /* [K][ldo] */,
@@ -214,5 +215,6 @@ static __global__ void wls_nnls_kernel(const double* __restrict__ mom, int K, in
     if (!(sum == sum)) atomicOr(status, 1);           // NaN proportions (e.g. a sample whose weights are all zero)
     if (singular) atomicOr(status, 2);
 }
+#endif  // DMF_INST_BODY
 
 }  // namespace dmf
