@@ -58,6 +58,8 @@ EXPORTS = {
     "dmf_pass_alpha": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dmf_pass_fw": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "dmf_pass_cost": (C.c_int, [C.c_void_p, C.c_double, C.c_void_p]),
+    "dmf_batch_set_step_state": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double),
+                                           C.c_void_p]),
     "dmf_batch_set_engine": (C.c_int, [C.c_void_p, C.c_int32]),
     "dmf_batch_get_engine": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
     "dmf_gram_rowgram": (C.c_int, [C.c_void_p, C.c_int32, C.c_double, C.c_void_p]),

@@ -1,6 +1,7 @@
 // dmf_api.cu — extern "C" surface of libdemethify_sm100.so (see include/demethify_b200.h).
 // Host logic only: shape validation, launch geometry, kernel dispatch, the outer-loop driver.
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -520,6 +521,23 @@ __global__ void gather_rows_kernel(const char* src, const int32_t* rows, long lo
     }
 }
 
+// dmf_batch_set_step_state: the scalars of up to kStepChunk fits travel in the kernel parameters, so the call needs no device
+// staging buffer and returns without waiting for the stream
+constexpr int kStepChunk = 128;
+struct StepStateArgs {
+    FitState* st;
+    int which, n;
+    double a[kStepChunk], l[kStepChunk], l_old[kStepChunk];
+};
+
+__global__ void set_step_state_kernel(const StepStateArgs s) {
+    const int i = threadIdx.x;
+    if (i >= s.n) return;
+    FitState& f = s.st[i];
+    if (s.which == 0) { f.a1 = s.a[i]; f.l_w = s.l[i]; f.l_w_old = s.l_old[i]; }
+    else { f.a2 = s.a[i]; f.l_h = s.l[i]; f.l_h_old = s.l_old[i]; }
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -739,6 +757,27 @@ int dmf_pass_fw(dmf_batch_t b, int32_t k_inner, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
     if (b->shape.mode != DMF_MODE_PURITY) return fail(DMF_E_STATE, "Frank-Wolfe steps need a purity batch");
     return launch(b, k_alpha(b), b->p.ntc_alpha, b->p.smem_alpha, kFlagFW, k_inner, 0.0, (cudaStream_t)stream);
+}
+int dmf_batch_set_step_state(dmf_batch_t b, int32_t which, const double* a, const double* l, const double* l_old, void* stream) {
+    if (!b || !a || !l || !l_old) return fail(DMF_E_ARG, "NULL argument");
+    if (which != 0 && which != 1) return fail(DMF_E_ARG, "which must be 0 (a1, l_w, l_w_old) or 1 (a2, l_h, l_h_old)");
+    const int n = b->shape.n_fits;
+    for (int i = 0; i < n; ++i) {        // every fit is checked before any state is written
+        if (!std::isfinite(a[i]) || !std::isfinite(l[i]) || !std::isfinite(l_old[i]))
+            return fail(DMF_E_ARG, "step state of fit " + std::to_string(i) + " is not finite");
+        if (!(l[i] > 0.0)) return fail(DMF_E_ARG, "step constant l of fit " + std::to_string(i) + " must be positive");
+    }
+    for (int i0 = 0; i0 < n; i0 += kStepChunk) {
+        StepStateArgs s;
+        s.st = b->states_dev + i0;
+        s.which = which;
+        s.n = std::min(kStepChunk, n - i0);
+        for (int i = 0; i < s.n; ++i) { s.a[i] = a[i0 + i]; s.l[i] = l[i0 + i]; s.l_old[i] = l_old[i0 + i]; }
+        set_step_state_kernel<<<1, kStepChunk, 0, (cudaStream_t)stream>>>(s);
+        CUDA_TRY(cudaGetLastError());
+        b->launches++;
+    }
+    return DMF_OK;
 }
 
 int dmf_batch_set_engine(dmf_batch_t b, int32_t engine) {

@@ -7,13 +7,14 @@ so that u0 / alpha0 are bit-identical for a given seed.
 """
 import numpy as np
 import numpy.random as rd
+import torch
 
 from . import _lib
-from .engine import DeviceProblem, FitBatch
+from .engine import DeviceProblem, FitBatch, to_device
 from .init_func import wls_intercept, wls_all_samples, constrained_nndsvd, nndsvd_initialize
 
-__all__ = ["set_seed", "cost_f_w", "projection_simplex_sort_2d", "init_BSSMF_md", "init_BSSMF_md_p",
-           "mdwbssmf_deconv", "mdwbssmf_deconv_p", "unsupervised_deconv", "last_fit_info", "best_of_restarts"]
+__all__ = ["set_seed", "cost_f_w", "projection_simplex_sort_2d", "init_BSSMF_md", "init_BSSMF_md_p", "update_u", "update_alpha",
+           "frank_wolfe_nmf", "mdwbssmf_deconv", "mdwbssmf_deconv_p", "unsupervised_deconv", "last_fit_info", "best_of_restarts"]
 
 _last = {}
 
@@ -30,17 +31,24 @@ def set_seed(seed=None):
         rd.seed(seed)
 
 
+def _split_r(R):
+    """A full R (M x Kt) as the kernels take it, [R_trunc | u] -> (R_trunc or None, u, n_u, mode).  The library pads both blocks to
+    even widths and needs their sum <= 32: the last TWO columns are "u" when Kt is even, the last one when it is odd (works up to
+    Kt = 32).  For the cost and the alpha step, which see R only as a whole, any split is equivalent."""
+    Kt = R.shape[1]
+    nu = 2 if (Kt % 2 == 0 and Kt >= 2) else 1
+    if Kt > nu:
+        return R[:, :Kt - nu], R[:, Kt - nu:], nu, _lib.DMF_MODE_PARTIAL
+    return None, R, nu, _lib.DMF_MODE_UNSUPERVISED
+
+
 def cost_f_w(y, R, alpha, d_x):
     """deconvolution.py:15-17 — sum d_x * (y - R @ alpha)^2, one streaming pass on the GPU."""
     R = np.asarray(R)
     alpha = np.asarray(alpha)
-    Kt = R.shape[1]
-    # the kernels take [R_trunc | u]; any split is equivalent for the cost.  The library pads both blocks to even widths and needs
-    # their sum <= 32: the last TWO columns are "u" when Kt is even, the last one when it is odd (works up to Kt = 32)
-    nu = 2 if (Kt % 2 == 0 and Kt >= 2) else 1
-    prob = DeviceProblem(y, d_x, R[:, :Kt - nu] if Kt > nu else None)
-    batch = FitBatch(prob, nu, [R[:, Kt - nu:]], [alpha], mode=_lib.DMF_MODE_PARTIAL if Kt > nu else _lib.DMF_MODE_UNSUPERVISED,
-                     engine="stream")
+    Rk, u, nu, mode = _split_r(R)
+    prob = DeviceProblem(y, d_x, Rk)
+    batch = FitBatch(prob, nu, [u], [alpha], mode=mode, engine="stream")
     batch.pass_init()
     cost = batch.states()[0].cost
     batch.close()
@@ -103,6 +111,71 @@ def init_BSSMF_md(init_option, meth_frequency, d_x, R_trunc, n_u, seed=None, rb_
     return u, R, alpha
 
 
+def _problem(meth_frequency, d_x, R_trunc):
+    # `meth_frequency` may be a DeviceProblem that is already resident in HBM (the n_u sweep of ic.py fits the same data many times,
+    # a user's own outer loop calls the solver steps on the same data every iteration); it brings its own d_x and R_trunc
+    return meth_frequency if isinstance(meth_frequency, DeviceProblem) else DeviceProblem(meth_frequency, d_x, R_trunc)
+
+
+def _check_shape(name, a, shape):
+    if tuple(np.shape(a)) != shape:
+        raise ValueError(f"{name} must be {shape[0]} x {shape[1]}, got shape {tuple(np.shape(a))}")
+
+
+def _host(t):
+    return t.to(torch.float64).contiguous().cpu().numpy()
+
+
+def update_u(u, alpha, n_iter2, a1, l_w_, l_w, u_, meth_frequency, R_trunc, n_u, d_x):
+    """deconvolution.py:81-90 — n_iter2 accelerated projected-gradient steps on u, one streaming pass each, from the caller's
+    iterates (u, u_) and momentum state (a1, and l_w_ = the l_w of the previous step).  -> (u, u_, a1, l_w_).  A resident DeviceProblem
+    in place of meth_frequency supplies X, d_x and R_trunc."""
+    prob = _problem(meth_frequency, d_x, R_trunc)
+    n_u = int(n_u)
+    _check_shape("u", u, (prob.M, n_u))
+    _check_shape("u_", u_, (prob.M, n_u))
+    _check_shape("alpha", alpha, (prob.K + n_u, prob.N))
+    steps = max(int(n_iter2), 0)
+    batch = FitBatch(prob, n_u, [u], [alpha], engine="stream")
+    batch.u_view(0, 1).copy_(to_device(u_, prob.dtype, prob.device))      # u_prev: the U pass reads slot u_cur ^ 1 (FitBatch put u there)
+    batch.set_step_state(0, [a1], [l_w], [l_w_])
+    for _ in range(steps):
+        batch.pass_u()
+    st, = batch.states()
+    out = _host(batch.u_view(0, st.u_slot)), _host(batch.u_view(0, st.u_slot ^ 1)), st.a1, float(l_w if steps else l_w_)
+    batch.close()
+    return out
+
+
+def update_alpha(n_iter2, alpha, a2, l_h_, l_h, alpha_, R, d_x, meth_frequency):
+    """deconvolution.py:93-102 — n_iter2 accelerated projected-gradient steps on alpha incl. the simplex projection, one streaming
+    pass each, from the caller's iterates (alpha, alpha_) and momentum state (a2, and l_h_ = the l_h of the previous step).
+    -> (alpha, alpha_, a2, l_h_).  A resident DeviceProblem in place of meth_frequency supplies X and d_x; R = [R_trunc | u] changes
+    every outer iteration and is uploaded on every call."""
+    R = np.asarray(R)
+    if R.ndim != 2 or R.shape[1] < 1:
+        raise ValueError("R must be M x Kt")
+    Rk, u, nu, mode = _split_r(R)
+    prob = meth_frequency.with_reference(Rk) if isinstance(meth_frequency, DeviceProblem) else DeviceProblem(meth_frequency, d_x, Rk)
+    Kt = R.shape[1]
+    _check_shape("R", R, (prob.M, Kt))
+    _check_shape("alpha", alpha, (Kt, prob.N))
+    _check_shape("alpha_", alpha_, (Kt, prob.N))
+    steps = max(int(n_iter2), 0)
+    batch = FitBatch(prob, nu, [u], [alpha], mode=mode, engine="stream")
+    batch.A[0, 1].copy_(to_device(alpha_, prob.dtype, prob.device))       # alpha_prev: slot a_cur ^ 1
+    batch.set_step_state(1, [a2], [l_h], [l_h_])
+    for _ in range(steps):
+        batch.pass_alpha()
+    st, = batch.states()
+    if st.done == 3:
+        batch.close()
+        raise _lib.DmfError("non-finite values reached the simplex projection")
+    out = _host(batch.A[0, st.a_slot]), _host(batch.A[0, st.a_slot ^ 1]), st.a2, float(l_h if steps else l_h_)
+    batch.close()
+    return out
+
+
 def init_BSSMF_md_p(init_option, meth_frequency, d_x, R_trunc, n_u, purity, rb_alg=wls_intercept, seed=None):
     """deconvolution.py:228-267."""
     set_seed(seed)
@@ -119,9 +192,29 @@ def init_BSSMF_md_p(init_option, meth_frequency, d_x, R_trunc, n_u, purity, rb_a
     return u, R, alpha
 
 
+def frank_wolfe_nmf(W1, W2, meth_frequency, H1, H2, purity, n_iter2, d_x):
+    """deconvolution.py:280-302 — n_iter2 Frank-Wolfe steps k = 0 .. n_iter2-1 on (H1, H2) with W1 = R_trunc and W2 = u fixed, one
+    streaming pass each.  -> (H1, H2).  A resident DeviceProblem in place of meth_frequency supplies X, d_x and W1 (its R_trunc)."""
+    prob = _problem(meth_frequency, d_x, W1)
+    if np.ndim(W2) != 2:
+        raise ValueError("W2 must be M x n_u")
+    n_u = np.shape(W2)[1]
+    if W1 is not None:
+        _check_shape("W1", W1, (prob.M, prob.K))
+    _check_shape("W2", W2, (prob.M, n_u))
+    _check_shape("H1", H1, (prob.K, prob.N))
+    _check_shape("H2", H2, (n_u, prob.N))
+    batch = FitBatch(prob, n_u, [W2], [np.vstack((H1, H2))], mode=_lib.DMF_MODE_PURITY, purity=purity, engine="stream")
+    for k in range(int(n_iter2)):
+        batch.pass_fw(k)
+    st, = batch.states()
+    H = _host(batch.A[0, st.a_slot])
+    batch.close()
+    return H[:prob.K], H[prob.K:]
+
+
 def _solve(mode, u, alpha, meth_frequency, d_x, R_trunc, n_u, n_iter1, n_iter2, tol, purity=None):
-    # `meth_frequency` may be a DeviceProblem that is already resident in HBM (the n_u sweep of ic.py fits the same data many times)
-    prob = meth_frequency if isinstance(meth_frequency, DeviceProblem) else DeviceProblem(meth_frequency, d_x, R_trunc)
+    prob = _problem(meth_frequency, d_x, R_trunc)
     batch = FitBatch(prob, n_u, [np.asarray(u).reshape(-1, n_u)], [np.asarray(alpha)], mode=mode, purity=purity)
     states = batch.fit(n_iter1, n_iter2, tol)
     (u_out, a_out, n_outer, cost), = batch.results(states)
@@ -175,7 +268,7 @@ def best_of_restarts(meth_frequency, d_x, R_trunc, n_u, init_option, seed, n_res
     else:
         base = seed[0] if isinstance(seed, (list, tuple)) else seed
         seeds = [base + r for r in range(n_restarts)]
-    prob = meth_frequency if isinstance(meth_frequency, DeviceProblem) else DeviceProblem(meth_frequency, d_x, R_trunc)
+    prob = _problem(meth_frequency, d_x, R_trunc)
     src = prob if init_option in ("uniform_", "uniform", "beta") else meth_frequency
     inits = []
     for s in seeds:

@@ -99,6 +99,10 @@ class DeviceProblem:
         self.wide = self.N * es >= 512              # short rows: bank conflicts do not matter, padding would (tile geometry, bytes)
         self.ldx = ((self.N * es + 127) // 128 * 128 + 16) // es if self.wide else (self.N + 7) // 8 * 8
         self.X = _pad_cols(X, self.ldx)
+        self._set_reference(Rk)
+        self.set_weights(D, narrow_weights)
+
+    def _set_reference(self, Rk):
         self.K = 0
         self.Rk = None
         if Rk is not None:
@@ -107,7 +111,6 @@ class DeviceProblem:
                 raise ValueError("R_trunc must be M x K")
             self.K = Rk.shape[1]
             self.Rk = _pad_cols(Rk, _even(self.K))
-        self.set_weights(D, narrow_weights)
 
     @property
     def shape(self):
@@ -209,6 +212,13 @@ class DeviceProblem:
         other = object.__new__(DeviceProblem)
         other.__dict__.update(self.__dict__)
         other.D, other.wtype = D_tensor, wtype
+        return other
+
+    def with_reference(self, Rk):
+        """Shallow copy sharing X / d_x with another R_trunc (M x K, or None): update_alpha gets a new R every outer iteration."""
+        other = object.__new__(DeviceProblem)
+        other.__dict__.update(self.__dict__)
+        other._set_reference(Rk)
         return other
 
 
@@ -325,6 +335,14 @@ class FitBatch:
 
     def pass_cost(self, tol):
         _lib.check(_lib.lib().dmf_pass_cost(self.b, float(tol), _stream_ptr()))
+
+    def set_step_state(self, which, a, l, l_old):
+        """Momentum state (one value per fit each) the next pass_u (which = 0: a1, l_w, l_w_old) or pass_alpha (which = 1: a2, l_h,
+        l_h_old) steps start from."""
+        if any(len(v) != self.n_fits for v in (a, l, l_old)):
+            raise ValueError("one step-state value per fit expected")
+        vals = [(C.c_double * self.n_fits)(*(float(x) for x in v)) for v in (a, l, l_old)]
+        _lib.check(_lib.lib().dmf_batch_set_step_state(self.b, int(which), *vals, _stream_ptr()))
 
     # -- Gram-form engine steps
     def gram_init(self):

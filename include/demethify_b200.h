@@ -146,6 +146,9 @@ int dmf_pass_alpha(dmf_batch_t b, void* stream);
 int dmf_pass_fw(dmf_batch_t b, int32_t k_inner, void* stream);
 /* cost_f_w + termination test |cf - cf_0| < tol (deconvolution.py:218-221) */
 int dmf_pass_cost(dmf_batch_t b, double tol, void* stream);
+/* Set the extrapolation state of every fit before dmf_pass_u (which = 0: a1, l_w, l_w_old) or dmf_pass_alpha
+ * (which = 1: a2, l_h, l_h_old).  Host arrays of n_fits values each.  Nothing else in the state changes. */
+int dmf_batch_set_step_state(dmf_batch_t b, int32_t which, const double* a, const double* l, const double* l_old, void* stream);
 
 /* Gram-form engine: the same outer iteration (deconvolution.py:206-221 / :320-335) on sufficient statistics ------- */
 int dmf_batch_set_engine(dmf_batch_t b, int32_t engine);
