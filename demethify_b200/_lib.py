@@ -42,6 +42,11 @@ class WlsDesc(C.Structure):
                 ("R2", C.c_void_p), ("out", C.c_void_p)]
 
 
+class ResidDesc(C.Structure):
+    _fields_ = [("M", C.c_int64), ("N", C.c_int32), ("K", C.c_int32), ("ldx", C.c_int64), ("ldr", C.c_int64), ("X", C.c_void_p),
+                ("R", C.c_void_p), ("H1", C.c_void_p)]
+
+
 EXPORTS = {
     "dmf_abi_version": (C.c_int, []),
     "dmf_last_error": (C.c_char_p, []),
@@ -85,6 +90,14 @@ EXPORTS = {
     "dmf_batch_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "dmf_wls_workspace_bytes": (C.c_int, [C.c_void_p, C.POINTER(WlsDesc), C.POINTER(C.c_size_t)]),
     "dmf_wls_fit": (C.c_int, [C.c_void_p, C.POINTER(WlsDesc), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dmf_wls_moments": (C.c_int, [C.c_void_p, C.POINTER(WlsDesc), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dmf_wls_solve": (C.c_int, [C.c_void_p, C.POINTER(WlsDesc), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dmf_resid_workspace_bytes": (C.c_int, [C.c_void_p, C.POINTER(ResidDesc), C.POINTER(C.c_size_t)]),
+    "dmf_resid_gram": (C.c_int, [C.c_void_p, C.POINTER(ResidDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dmf_resid_project": (C.c_int, [C.c_void_p, C.POINTER(ResidDesc), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_size_t, C.c_void_p]),
+    "dmf_nndsvd_apply": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                   C.c_void_p]),
     "dmf_pack_weights_u16": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dmf_nndsvd_split": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
                                    C.c_void_p, C.c_void_p]),

@@ -1171,6 +1171,77 @@ int make_wls_plan(const dmf_handle_s* h, const dmf_wls_desc_t& d, WlsPlan& p) {
     return DMF_OK;
 }
 
+wls_kern_t wls_kernel_of(const dmf_wls_desc_t& d) {
+    return d.dtype == DMF_F64 ? (d.wtype == DMF_W_U16 ? pick_wls_f64_u16() : pick_wls_f64_f64())
+                              : (d.wtype == DMF_W_U16 ? pick_wls_f32_u16() : pick_wls_f32_f32());
+}
+
+// workspace checks and kernel attribute of one dmf_wls_fit / dmf_wls_moments call
+int wls_prepare(const dmf_handle_s* h, const dmf_wls_desc_t* dd, void* ws, size_t ws_bytes, void* stream, WlsPlan& p) {
+    if (!h || !dd || !ws) return fail(DMF_E_ARG, "NULL argument");
+    const dmf_wls_desc_t& d = *dd;
+    if (!d.X || !d.D || !d.out || (d.K && !d.R1) || (d.K2 && !d.R2)) return fail(DMF_E_ARG, "wls: NULL matrix");
+    int rc = make_wls_plan(h, d, p);
+    if (rc) return rc;
+    if (ws_bytes < p.ws_bytes) return fail(DMF_E_ARG, "wls: workspace too small");
+    if (reinterpret_cast<uintptr_t>(ws) & 255) return fail(DMF_E_ARG, "workspace must be 256-byte aligned");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    char* base = static_cast<char*>(ws);
+    CUDA_TRY(cudaFuncSetAttribute((const void*)wls_kernel_of(d), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+    CUDA_TRY(cudaMemsetAsync(base + p.off_tickets, 0, p.off_part - p.off_tickets, st));
+    CUDA_TRY(cudaMemsetAsync(base + p.off_status, 0, 256, st));
+    return DMF_OK;
+}
+
+// the moment launches of sample columns j0 .. j0 + ns into the workspace's [Kz Kz][ns] matrix
+int wls_moments_slab(const dmf_wls_desc_t& d, const WlsPlan& p, char* base, int j0, int ns, cudaStream_t st) {
+    const size_t sT = d.dtype == DMF_F64 ? 8 : 4, sW = d.wtype == DMF_W_U16 ? 2 : sT;
+    FitDev f;
+    memset(&f, 0, sizeof(f));
+    f.X = static_cast<const char*>(d.X) + (size_t)j0 * sT;
+    f.D = static_cast<const char*>(d.D) + (size_t)j0 * sW;
+    f.Rk = static_cast<const char*>(d.R1);
+    f.U = const_cast<char*>(static_cast<const char*>(d.R2));
+    f.part = reinterpret_cast<double*>(base + p.off_part);
+    f.gpart = reinterpret_cast<double*>(base + p.off_gpart);
+    f.tickets = reinterpret_cast<unsigned*>(base + p.off_tickets);
+    CUDA_TRY(cudaMemcpyAsync(base + p.off_fit, &f, sizeof(f), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));   // `f` is a stack temporary
+    WlsArgs a;
+    memset(&a, 0, sizeof(a));
+    Geom& g = a.g;
+    g.M = d.M; g.N = ns; g.K = d.K; g.nu = d.K2; g.Kt = d.K + d.K2;
+    g.ldx = d.ldx; g.ldd = d.ldd; g.ldr = d.K ? d.ldr : 0; g.ldu = d.K2 ? d.ldr2 : 0;
+    g.tile_rows = p.tile_rows; g.n_tiles = p.n_tiles; g.ntc = pow2ceil(ns); g.rg = kConsumers / g.ntc;
+    // rows of a tile are walked with stride rg: a narrower last slab only changes the thread mapping
+    g.n_parts = p.n_parts; g.n_groups = p.n_groups; g.part_stride = p.part_stride;
+    set_stages(g, p.stage);
+    g.offUp = g.offU;
+    a.fits = reinterpret_cast<const FitDev*>(base + p.off_fit);
+    a.mom = reinterpret_cast<double*>(base + p.off_mom);
+    a.Kfull = d.K + d.K2;
+    a.y_is_dx = d.y_is_dx;
+    const wls_kern_t kern = wls_kernel_of(d);
+    for (int bi = 0; bi < p.nblk; ++bi)
+        for (int bj = bi; bj < p.nblk; ++bj) {
+            a.bi = bi; a.bj = bj;
+            kern<<<dim3(p.n_parts, 1, 1), kThreads, p.smem, st>>>(a);
+            CUDA_TRY(cudaGetLastError());
+        }
+    return DMF_OK;
+}
+
+// reads the NNLS status word (synchronises the stream)
+int wls_status(const void* status_dev, cudaStream_t st) {
+    int status = 0;
+    CUDA_TRY(cudaMemcpyAsync(&status, status_dev, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (status & 1) return fail(DMF_E_STATE, "wls: a sample produced non-finite proportions (all of its weights zero, or non-finite inputs)");
+    if (status & 2) return fail(DMF_E_STATE, "wls: the regressors of a sample are collinear (non-positive pivot in the normal equations)");
+    return DMF_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1185,65 +1256,62 @@ int dmf_wls_workspace_bytes(dmf_handle_t h, const dmf_wls_desc_t* d, size_t* byt
 }
 
 int dmf_wls_fit(dmf_handle_t h, const dmf_wls_desc_t* dd, void* ws, size_t ws_bytes, void* stream) {
-    if (!h || !dd || !ws) return fail(DMF_E_ARG, "NULL argument");
-    const dmf_wls_desc_t& d = *dd;
-    if (!d.X || !d.D || !d.out || (d.K && !d.R1) || (d.K2 && !d.R2)) return fail(DMF_E_ARG, "wls: NULL matrix");
     WlsPlan p;
-    int rc = make_wls_plan(h, d, p);
+    int rc = wls_prepare(h, dd, ws, ws_bytes, stream, p);
     if (rc) return rc;
-    if (ws_bytes < p.ws_bytes) return fail(DMF_E_ARG, "wls: workspace too small");
-    if (reinterpret_cast<uintptr_t>(ws) & 255) return fail(DMF_E_ARG, "workspace must be 256-byte aligned");
-    CUDA_TRY(cudaSetDevice(h->device));
+    const dmf_wls_desc_t& d = *dd;
     cudaStream_t st = (cudaStream_t)stream;
     char* base = static_cast<char*>(ws);
-    const size_t sT = d.dtype == DMF_F64 ? 8 : 4, sW = d.wtype == DMF_W_U16 ? 2 : sT;
-    wls_kern_t kern = d.dtype == DMF_F64 ? (d.wtype == DMF_W_U16 ? pick_wls_f64_u16() : pick_wls_f64_f64())
-                                         : (d.wtype == DMF_W_U16 ? pick_wls_f32_u16() : pick_wls_f32_f32());
-    CUDA_TRY(cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-    CUDA_TRY(cudaMemsetAsync(base + p.off_tickets, 0, p.off_part - p.off_tickets, st));
-    CUDA_TRY(cudaMemsetAsync(base + p.off_status, 0, 256, st));
     for (int j0 = 0; j0 < d.N; j0 += p.slab) {
         const int ns = std::min(p.slab, d.N - j0);
-        FitDev f;
-        memset(&f, 0, sizeof(f));
-        f.X = static_cast<const char*>(d.X) + (size_t)j0 * sT;
-        f.D = static_cast<const char*>(d.D) + (size_t)j0 * sW;
-        f.Rk = static_cast<const char*>(d.R1);
-        f.U = const_cast<char*>(static_cast<const char*>(d.R2));
-        f.part = reinterpret_cast<double*>(base + p.off_part);
-        f.gpart = reinterpret_cast<double*>(base + p.off_gpart);
-        f.tickets = reinterpret_cast<unsigned*>(base + p.off_tickets);
-        CUDA_TRY(cudaMemcpyAsync(base + p.off_fit, &f, sizeof(f), cudaMemcpyHostToDevice, st));
-        CUDA_TRY(cudaStreamSynchronize(st));   // `f` is a stack temporary
-        WlsArgs a;
-        memset(&a, 0, sizeof(a));
-        Geom& g = a.g;
-        g.M = d.M; g.N = ns; g.K = d.K; g.nu = d.K2; g.Kt = d.K + d.K2;
-        g.ldx = d.ldx; g.ldd = d.ldd; g.ldr = d.K ? d.ldr : 0; g.ldu = d.K2 ? d.ldr2 : 0;
-        g.tile_rows = p.tile_rows; g.n_tiles = p.n_tiles; g.ntc = pow2ceil(ns); g.rg = kConsumers / g.ntc;
-        // rows of a tile are walked with stride rg: a narrower last slab only changes the thread mapping
-        g.n_parts = p.n_parts; g.n_groups = p.n_groups; g.part_stride = p.part_stride;
-        set_stages(g, p.stage);
-        g.offUp = g.offU;
-        a.fits = reinterpret_cast<const FitDev*>(base + p.off_fit);
-        a.mom = reinterpret_cast<double*>(base + p.off_mom);
-        a.Kfull = d.K + d.K2;
-        a.y_is_dx = d.y_is_dx;
-        for (int bi = 0; bi < p.nblk; ++bi)
-            for (int bj = bi; bj < p.nblk; ++bj) {
-                a.bi = bi; a.bj = bj;
-                kern<<<dim3(p.n_parts, 1, 1), kThreads, p.smem, st>>>(a);
-                CUDA_TRY(cudaGetLastError());
-            }
-        wls_nnls_kernel<<<(ns + 63) / 64, 64, 0, st>>>(a.mom, a.Kfull, ns, d.M, d.out + j0, (long long)d.N, reinterpret_cast<int*>(base + p.off_status));
+        rc = wls_moments_slab(d, p, base, j0, ns, st);
+        if (rc) return rc;
+        wls_nnls_kernel<<<(ns + 63) / 64, 64, 0, st>>>(reinterpret_cast<double*>(base + p.off_mom), d.K + d.K2, ns, d.M, d.out + j0,
+                                                      (long long)d.N, reinterpret_cast<int*>(base + p.off_status));
         CUDA_TRY(cudaGetLastError());
     }
-    int status = 0;
-    CUDA_TRY(cudaMemcpyAsync(&status, base + p.off_status, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    if (status & 1) return fail(DMF_E_STATE, "wls: a sample produced non-finite proportions (all of its weights zero, or non-finite inputs)");
-    if (status & 2) return fail(DMF_E_STATE, "wls: the regressors of a sample are collinear (non-positive pivot in the normal equations)");
+    return wls_status(base + p.off_status, st);
+}
+
+int dmf_wls_moments(dmf_handle_t h, const dmf_wls_desc_t* dd, double* mom, void* ws, size_t ws_bytes, void* stream) {
+    if (!h || !dd || !mom) return fail(DMF_E_ARG, "NULL argument");
+    const dmf_wls_desc_t& d = *dd;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t Kz = (size_t)(d.K + d.K2 + 2);
+    if (d.M == 0 && d.N > 0 && d.K >= 0 && d.K2 >= 0) {      // a GPU that holds no rows contributes zero moments
+        CUDA_TRY(cudaSetDevice(h->device));
+        CUDA_TRY(cudaMemsetAsync(mom, 0, Kz * Kz * d.N * sizeof(double), st));
+        return DMF_OK;
+    }
+    WlsPlan p;
+    int rc = wls_prepare(h, dd, ws, ws_bytes, stream, p);
+    if (rc) return rc;
+    char* base = static_cast<char*>(ws);
+    for (int j0 = 0; j0 < d.N; j0 += p.slab) {
+        const int ns = std::min(p.slab, d.N - j0);
+        rc = wls_moments_slab(d, p, base, j0, ns, st);
+        if (rc) return rc;
+        // the slab's [Kz Kz][ns] block into columns j0 .. j0 + ns of the caller's [Kz Kz][N] matrix
+        CUDA_TRY(cudaMemcpy2DAsync(mom + j0, d.N * sizeof(double), base + p.off_mom, ns * sizeof(double), ns * sizeof(double), Kz * Kz,
+                                   cudaMemcpyDeviceToDevice, st));
+    }
     return DMF_OK;
+}
+
+int dmf_wls_solve(dmf_handle_t h, const dmf_wls_desc_t* dd, const double* mom, void* ws, size_t ws_bytes, void* stream) {
+    if (!h || !dd || !mom || !ws) return fail(DMF_E_ARG, "NULL argument");
+    const dmf_wls_desc_t& d = *dd;
+    if (!d.out) return fail(DMF_E_ARG, "wls: NULL matrix");
+    if (d.M <= 0 || d.N <= 0 || d.K < 0 || d.K2 < 0 || d.K + d.K2 <= 0) return fail(DMF_E_SHAPE, "wls: M, N positive and K + K2 >= 1 required");
+    if (d.K + d.K2 > kMaxKt) return fail(DMF_E_SHAPE, "wls: more than 32 regressors are not supported by this build");
+    if (ws_bytes < 256) return fail(DMF_E_ARG, "wls: workspace too small");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(ws, 0, 256, st));
+    // one thread per sample reads column j of the [Kz Kz][N] matrix: the same moments, K and M as dmf_wls_fit's per-slab launches
+    wls_nnls_kernel<<<(d.N + 63) / 64, 64, 0, st>>>(mom, d.K + d.K2, d.N, d.M, d.out, (long long)d.N, static_cast<int*>(ws));
+    CUDA_TRY(cudaGetLastError());
+    return wls_status(ws, st);
 }
 
 }  // extern "C"
@@ -1296,6 +1364,175 @@ int dmf_consensus(const double* alpha_runs, int32_t n_runs, int32_t Kt, int32_t 
     CUDA_TRY(cudaGetLastError());
     const long long nn = (long long)N * N;
     consensus_kernel<<<(int)((nn + 127) / 128), 128, 0, (cudaStream_t)stream>>>(labels_ws, n_runs, N, consensus);
+    CUDA_TRY(cudaGetLastError());
+    return DMF_OK;
+}
+
+}  // extern "C"
+
+// =================================================================================================
+// NNDSVD of the floored residual over row-sharded rows (dmf_resid.cuh)
+#include "dmf_resid.cuh"
+
+namespace {
+
+struct ResidPlan {
+    int nt, n_tri, tile_rows, n_tiles, n_parts, n_groups, stages;   // resid_gram_kernel
+    int p_parts, p_groups;                                          // resid_project_kernel
+    StageLayout stage;
+    unsigned smem;
+    size_t off_fits, off_tickets, off_part, off_gpart, off_pfit, off_ptickets, off_ppart, off_pgpart, ws_bytes;
+};
+
+int make_resid_plan(const dmf_handle_s* h, const dmf_resid_desc_t& d, ResidPlan& p) {
+    if (d.M < 0 || d.N <= 0 || d.K < 0) return fail(DMF_E_SHAPE, "resid: M >= 0, N > 0 and K >= 0 required");
+    if (d.N > kMaxResidN) return fail(DMF_E_SHAPE, "resid: more than 512 samples are not supported by this build");
+    if (d.K > kMaxKt) return fail(DMF_E_SHAPE, "resid: more than 32 reference columns are not supported by this build");
+    if (d.ldx < d.N || (d.K && d.ldr < d.K) || ((d.ldx | (d.K ? d.ldr : 0)) & 1))
+        return fail(DMF_E_SHAPE, "resid: row pitches must be even and at least the row");
+    p.nt = (d.N + kGramTile - 1) / kGramTile;
+    p.n_tri = p.nt * (p.nt + 1) / 2;
+    const size_t rows_w[kMaxSrc] = {(size_t)d.ldx * 8, 0, d.K ? (size_t)d.ldr * 8 : 0, 0, 0};
+    const size_t budget = (size_t)h->max_smem_optin - kCtlBytes;
+    p.tile_rows = 0;
+    for (int tr = kResMaxRows; tr >= 4 && !p.tile_rows; tr >>= 1)
+        for (int stg = kStages; stg >= 3; --stg) {
+            const size_t ring = std::max<size_t>(stage_layout(tr, rows_w, rows_w).bytes * stg, (size_t)kGramTile * kGramTile * 8);
+            if (ring + (size_t)tr * kResPitch * 8 <= budget) { p.tile_rows = tr; p.stages = stg; break; }
+        }
+    if (!p.tile_rows) return fail(DMF_E_SHAPE, "resid: one row tile does not fit in shared memory");
+    p.stage = stage_layout(p.tile_rows, rows_w, rows_w);
+    p.smem = (unsigned)(kCtlBytes + std::max<size_t>((size_t)p.stage.bytes * p.stages, (size_t)kGramTile * kGramTile * 8) +
+                        (size_t)p.tile_rows * kResPitch * 8);
+    p.n_tiles = (int)std::max<long long>(1, (d.M + p.tile_rows - 1) / p.tile_rows);
+    // two CTAs per SM over all G tiles, never more row splits than row tiles
+    p.n_parts = std::max(1, std::min(p.n_tiles, 2 * h->sm_count / p.n_tri));
+    p.n_groups = groups_of(p.n_parts);
+    p.p_parts = (int)std::max<long long>(1, std::min<long long>((d.M + 7) / 8, 4LL * h->sm_count));
+    p.p_groups = groups_of(p.p_parts);
+    const size_t TT = (size_t)kGramTile * kGramTile;
+    p.off_fits = 0;
+    p.off_tickets = align_up(sizeof(FitDev) * p.n_tri, 256);
+    p.off_part = align_up(p.off_tickets + sizeof(unsigned) * p.n_tri * (p.n_groups + 1), 256);
+    p.off_gpart = align_up(p.off_part + (size_t)p.n_tri * p.n_parts * TT * 8, 256);
+    p.off_pfit = align_up(p.off_gpart + (size_t)p.n_tri * p.n_groups * TT * 8, 256);
+    p.off_ptickets = align_up(p.off_pfit + sizeof(FitDev), 256);
+    p.off_ppart = align_up(p.off_ptickets + sizeof(unsigned) * (p.p_groups + 1), 256);
+    p.off_pgpart = align_up(p.off_ppart + (size_t)p.p_parts * 2 * kMaxKt * 8, 256);
+    p.ws_bytes = align_up(p.off_pgpart + (size_t)p.p_groups * 2 * kMaxKt * 8, 256);
+    return DMF_OK;
+}
+
+int resid_check(const dmf_handle_s* h, const dmf_resid_desc_t* d, void* ws, size_t ws_bytes, ResidPlan& p) {
+    if (!h || !d || !ws) return fail(DMF_E_ARG, "NULL argument");
+    if ((d->M && !d->X) || (d->M && d->K && (!d->R || !d->H1))) return fail(DMF_E_ARG, "resid: NULL matrix");
+    int rc = make_resid_plan(h, *d, p);
+    if (rc) return rc;
+    if (ws_bytes < p.ws_bytes) return fail(DMF_E_ARG, "resid: workspace too small");
+    if (reinterpret_cast<uintptr_t>(ws) & 255) return fail(DMF_E_ARG, "workspace must be 256-byte aligned");
+    return DMF_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dmf_resid_workspace_bytes(dmf_handle_t h, const dmf_resid_desc_t* d, size_t* bytes) {
+    if (!h || !d || !bytes) return fail(DMF_E_ARG, "NULL argument");
+    ResidPlan p;
+    int rc = make_resid_plan(h, *d, p);
+    if (rc) return rc;
+    *bytes = p.ws_bytes;
+    return DMF_OK;
+}
+
+int dmf_resid_gram(dmf_handle_t h, const dmf_resid_desc_t* d, double* G, int32_t* has_negative, void* ws, size_t ws_bytes, void* stream) {
+    ResidPlan p;
+    int rc = resid_check(h, d, ws, ws_bytes, p);
+    if (rc) return rc;
+    if (!G || !has_negative) return fail(DMF_E_ARG, "NULL argument");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    char* base = static_cast<char*>(ws);
+    CUDA_TRY(cudaMemsetAsync(has_negative, 0, sizeof(int32_t), st));
+    if (d->M == 0) {                                     // a GPU that holds no rows contributes zero
+        CUDA_TRY(cudaMemsetAsync(G, 0, (size_t)d->N * d->N * sizeof(double), st));
+        return DMF_OK;
+    }
+    const size_t TT = (size_t)kGramTile * kGramTile;
+    std::vector<FitDev> fits(p.n_tri);
+    for (int t = 0; t < p.n_tri; ++t) {
+        FitDev& f = fits[t];
+        memset(&f, 0, sizeof(f));
+        f.X = reinterpret_cast<const char*>(d->X);
+        f.Rk = d->K ? reinterpret_cast<const char*>(d->R) : nullptr;
+        f.part = reinterpret_cast<double*>(base + p.off_part) + (size_t)t * p.n_parts * TT;
+        f.gpart = reinterpret_cast<double*>(base + p.off_gpart) + (size_t)t * p.n_groups * TT;
+        f.tickets = reinterpret_cast<unsigned*>(base + p.off_tickets) + (size_t)t * (p.n_groups + 1);
+    }
+    CUDA_TRY(cudaMemcpyAsync(base + p.off_fits, fits.data(), sizeof(FitDev) * p.n_tri, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(base + p.off_tickets, 0, p.off_part - p.off_tickets, st));
+    ResidArgs a;
+    memset(&a, 0, sizeof(a));
+    Geom& g = a.g;
+    g.M = d->M; g.N = d->N; g.K = d->K;
+    g.ldx = d->ldx; g.ldr = d->K ? d->ldr : 0;
+    g.tile_rows = p.tile_rows; g.n_tiles = p.n_tiles;
+    g.n_parts = p.n_parts; g.n_groups = p.n_groups; g.part_stride = (int)TT;
+    g.stages = p.stages;
+    set_stages(g, p.stage);
+    a.fits = reinterpret_cast<const FitDev*>(base + p.off_fits);
+    a.H1 = d->H1;
+    a.G = G;
+    a.neg = has_negative;
+    a.nt = p.nt;
+    CUDA_TRY(cudaFuncSetAttribute((const void*)resid_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+    resid_gram_kernel<<<dim3(p.n_parts, p.n_tri, 1), kThreads, p.smem, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaStreamSynchronize(st));                 // `fits` is a host temporary
+    return DMF_OK;
+}
+
+int dmf_resid_project(dmf_handle_t h, const dmf_resid_desc_t* d, const double* Vh, const double* inv_sigma, int32_t rank, double* U,
+                      double* sums, void* ws, size_t ws_bytes, void* stream) {
+    ResidPlan p;
+    int rc = resid_check(h, d, ws, ws_bytes, p);
+    if (rc) return rc;
+    if (rank <= 0 || rank > kMaxKt || rank > d->N) return fail(DMF_E_SHAPE, "resid: 1 <= rank <= min(N, 32) required");
+    if (!Vh || !inv_sigma || !sums || (d->M && !U)) return fail(DMF_E_ARG, "NULL argument");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    char* base = static_cast<char*>(ws);
+    if (d->M == 0) {
+        CUDA_TRY(cudaMemsetAsync(sums, 0, 2 * (size_t)rank * sizeof(double), st));
+        return DMF_OK;
+    }
+    FitDev f;
+    memset(&f, 0, sizeof(f));
+    f.part = reinterpret_cast<double*>(base + p.off_ppart);
+    f.gpart = reinterpret_cast<double*>(base + p.off_pgpart);
+    f.tickets = reinterpret_cast<unsigned*>(base + p.off_ptickets);
+    CUDA_TRY(cudaMemcpyAsync(base + p.off_pfit, &f, sizeof(f), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(base + p.off_ptickets, 0, p.off_ppart - p.off_ptickets, st));
+    ProjArgs a;
+    memset(&a, 0, sizeof(a));
+    Geom& g = a.g;
+    g.M = d->M; g.N = d->N; g.K = d->K;
+    g.ldx = d->ldx; g.ldr = d->K ? d->ldr : 0;
+    g.n_parts = p.p_parts; g.n_groups = p.p_groups; g.part_stride = 2 * kMaxKt;
+    a.fit = reinterpret_cast<const FitDev*>(base + p.off_pfit);
+    a.X = d->X; a.R = d->R; a.H1 = d->H1; a.Vh = Vh; a.inv_s = inv_sigma; a.U = U; a.sums = sums; a.rank = rank;
+    resid_project_kernel<<<p.p_parts, kThreads, 0, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaStreamSynchronize(st));                 // `f` is a stack temporary
+    return DMF_OK;
+}
+
+int dmf_nndsvd_apply(const double* U, int64_t M, const double* Vh, const double* S, const double* sums, int32_t N, int32_t rank,
+                     double* W, double* H, void* stream) {
+    if (!Vh || !S || !sums || !H || M < 0 || N <= 0 || rank <= 0 || (M && (!U || !W))) return fail(DMF_E_ARG, "nndsvd: bad argument");
+    const int blocks = (int)std::max<long long>(1, std::min<long long>((M + 255) / 256, 1024));
+    nndsvd_apply_kernel<<<dim3(rank, blocks, 1), 256, 0, (cudaStream_t)stream>>>(U, M, Vh, S, sums, N, rank, W, H);
     CUDA_TRY(cudaGetLastError());
     return DMF_OK;
 }

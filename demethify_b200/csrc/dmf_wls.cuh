@@ -116,7 +116,9 @@ __global__ void __launch_bounds__(kThreads, 1) wls_moments_kernel(const WlsArgs 
     for (int e = threadIdx.x; e < BN; e += blockDim.x) {
         const int pq = e / g.N, jj = e - pq * g.N;
         const int p = a.bi * kWlsBlock + pq / kWlsBlock, q = a.bj * kWlsBlock + pq % kWlsBlock;
-        if (p < Kz && q < Kz) {
+        // a diagonal block accumulates both (p, q) and (q, p), which round differently ((d z_p) z_q vs (d z_q) z_p): only the
+        // upper entry is stored, mirrored, so that each moment has one writer and the matrix is exactly symmetric
+        if (p < Kz && q < Kz && p <= q) {
             a.mom[((size_t)p * Kz + q) * g.N + jj] = scratch[e];
             a.mom[((size_t)q * Kz + p) * g.N + jj] = scratch[e];
         }

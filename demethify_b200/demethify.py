@@ -56,8 +56,9 @@ def build_parser():
                    help="(B200 path) --restart R draws restart r from seed + r and keeps the lowest cost (the reference re-seeds every "
                         "restart identically, so its R restarts are one fit); with --confidence every resample is fitted R times")
     p.add_argument("--shard", choices=["fits", "rows"], default="fits",
-                   help="(B200 path, under torchrun) how --ic / --confidence use several GPUs: independent fits per GPU, or the CpG rows "
-                        "of every fit sharded over the GPUs")
+                   help="(B200 path, under torchrun) how several GPUs are used: 'fits' runs independent fits per GPU (--ic, --confidence; "
+                        "the main fit runs on every GPU), 'rows' shards the CpG rows of every fit over the GPUs (the main fit and --ic AIC / "
+                        "BIC; --confidence and --ic CCC / BCV stay fit-sharded)")
     return p
 
 
@@ -158,6 +159,29 @@ def _init_distributed():
     return dist.get_rank(), dist.get_world_size()
 
 
+def _row_sharded_main_fit(meth_f, counts, ref, n_u, purity, init_option, seed, it1, it2, tol, rank, world):
+    """The main fit with the CpG rows sharded over the ranks: rank r keeps row_range(M, r, world) of what it read; the initial
+    iterate and the fit all-reduce their row sums.  -> (u over all rows in row order on rank 0, None elsewhere; alpha)."""
+    import torch.distributed as dist
+    from .sharded import (init_BSSMF_md_p_sharded, init_BSSMF_md_sharded, mdwbssmf_deconv_sharded, row_range, unsupervised_init_sharded,
+                          wls_all_samples_sharded)
+    lo, hi = row_range(meth_f.shape[0], rank, world)
+    X, D = meth_f[lo:hi], counts[lo:hi]
+    R = None if ref is None else np.asarray(ref)[lo:hi]
+    if R is not None and n_u == 0:
+        return None, wls_all_samples_sharded(X, D, R, y_is_dx=True)                      # demethify.py:209-213
+    if R is None:
+        u0, a0 = unsupervised_init_sharded(init_option, X, D, n_u, seed=seed)
+    elif purity is not None:
+        u0, a0 = init_BSSMF_md_p_sharded(init_option, X, D, R, n_u, purity, seed=seed)
+    else:
+        u0, a0 = init_BSSMF_md_sharded(init_option, X, D, R, n_u, seed=seed)
+    u, alpha, _n, _cost = mdwbssmf_deconv_sharded(u0, a0, X, D, R, n_u, n_iter1=it1, n_iter2=it2, tol=tol, purity=purity)
+    parts = [None] * world if rank == 0 else None
+    dist.gather_object(u, parts, dst=0)
+    return (np.concatenate(parts, axis=0) if rank == 0 else None), alpha
+
+
 def main(argv=None):
     args = build_parser().parse_args(argv)
     if args.plot:
@@ -201,6 +225,10 @@ def main(argv=None):
     if args.nbunknown is None:
         args.nbunknown = [0]
     n_u = args.nbunknown[0]
+    rows_mode = args.shard == "rows" and world > 1
+    if rows_mode and args.distinct_restarts and args.restart > 1:
+        sys.stderr.write("Error: --restart R --distinct-restarts runs independent fits: use --shard fits.\n")
+        sys.exit(1)
     meth_f, counts, ref, header = read_inputs(args)
     args.methfreq = [name.split("/")[-1] for name in args.methfreq]
     it1, it2, tol = args.iterations[0], args.iterations[1], args.termination
@@ -217,6 +245,11 @@ def main(argv=None):
                                                                       iter2=it2, tol=tol, n_restarts=nb_r, shard=args.shard)
         unknown_header = ["unknown_cell_" + str(i + 1) for i in range(ic_n_u)]
         header = header + unknown_header
+    elif rows_mode and (not args.ref or (n_u >= 0 and meth_f.shape[1] >= 1)):
+        ref_estimate, proportions = _row_sharded_main_fit(meth_f, counts, ref, n_u, purity if args.purity else None, args.init, args.seed,
+                                                          it1, it2, tol, rank, world)
+        unknown_header = ["unknown_cell_" + str(i + 1) for i in range(n_u)]
+        header = header + unknown_header if args.ref else unknown_header
     elif not args.ref:
         # demethify.py:167-174: every restart re-seeds with the same seed, so all restarts are the same fit (SURVEY Q2)
         ref_estimate, proportions = unsupervised_deconv(meth_f, n_u, counts, args.init, n_iter1=it1, n_iter2=it2, tol=tol, seed=args.seed)
@@ -240,7 +273,7 @@ def main(argv=None):
     else:
         sys.exit(f'Invalid number of unknown value! : "{args.nbunknown}" ')
     time_tot = time() - t0
-    if rank != 0:                      # under torchrun every rank computed the same result; rank 0 writes the files
+    if rank != 0:                      # under torchrun every rank computed the same result (or its rows of it); rank 0 writes the files
         return
     if ref_estimate is not None:
         pd.DataFrame(ref_estimate).to_csv(outdir + "/methylation_profile_estimate.csv", index=False, header=unknown_header)

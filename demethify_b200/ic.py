@@ -147,14 +147,19 @@ def sweep_member_supported(K, n_u):
 
 def _row_sharded_member(prob_local, lo, hi, M, K, N, n_u, init_option, seed, iter1, iter2, tol, group):
     """One sweep member with the CpG rows sharded over the ranks of `group` (BASELINE config 5): every rank draws the same
-    initial iterate from the same seed, keeps its rows of u and runs the row-sharded solver -> (u_local, alpha, cost)."""
+    initial iterate from the same seed, keeps its rows of u and runs the row-sharded solver -> (u_local, alpha, cost).  The
+    `uniform` and `SVD` inits all-reduce their row sums (sharded.ShardedInit)."""
     from .bootstrap import _shape_only_init
-    from .sharded import mdwbssmf_deconv_sharded
-    if init_option not in ("uniform_", "beta"):
-        raise NotImplementedError("row-sharded sweeps draw the initial iterate from shapes only: --init uniform_ or beta")
-    # RandomState(seed) == the reference's set_seed(seed) + global stream (int -> init_genrand, list -> init_by_array, Q1)
-    u0, a0 = _shape_only_init(seed, init_option if n_u <= N else "uniform_", M, K, N, n_u, with_zero_guard=True)
-    u_loc, alpha, _n, cost = mdwbssmf_deconv_sharded(u0[lo:hi], a0, prob_local, None, None, n_u, n_iter1=iter1, n_iter2=iter2, tol=tol,
+    from .sharded import init_BSSMF_md_sharded, mdwbssmf_deconv_sharded
+    if init_option in ("uniform_", "beta"):
+        # RandomState(seed) == the reference's set_seed(seed) + global stream (int -> init_genrand, list -> init_by_array, Q1)
+        u0, a0 = _shape_only_init(seed, init_option if n_u <= N else "uniform_", M, K, N, n_u, with_zero_guard=True)
+        u0 = u0[lo:hi]
+    elif init_option in ("uniform", "SVD"):
+        u0, a0 = init_BSSMF_md_sharded(init_option, prob_local, None, None, n_u, seed=seed, group=group)
+    else:
+        raise NotImplementedError("row-sharded sweeps: --init uniform_, beta, uniform or SVD")
+    u_loc, alpha, _n, cost = mdwbssmf_deconv_sharded(u0, a0, prob_local, None, None, n_u, n_iter1=iter1, n_iter2=iter2, tol=tol,
                                                      group=group)
     return u_loc, alpha, cost
 
@@ -170,7 +175,8 @@ def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, t
 
     Under torch.distributed: shard="fits" (default) gives position p of the sweep to rank p mod world (every member re-seeds and
     is independent); shard="rows" runs EVERY member with the CpG rows sharded over the ranks (one all-reduce per outer
-    iteration, sharded.py) - the partitioning for matrices that are large per member (AIC / BIC, shape-only inits)."""
+    iteration, sharded.py) - the partitioning for matrices that are large per member (AIC / BIC; every init but ICA, and the
+    reference-based member n_u = 0)."""
     n_u_values = range(1, 25 + 1) if n_u_values is None else n_u_values
     meth_f = np.asarray(meth_f)
     n_cpg, n_samples = meth_f.shape
@@ -211,10 +217,18 @@ def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, t
         if n_u == 0:
             from .init_func import wls_all_samples
             if rows_mode:
-                raise NotImplementedError("n_u = 0 in a row-sharded sweep")
-            alpha = wls_all_samples(prob, None, None, y_is_dx=True)          # demethify.py:209-213
-            u = np.zeros((n_cpg, 0))
-            cost = cost_f_w(meth_f, np.asarray(ref), alpha, counts)
+                from .sharded import wls_all_samples_sharded
+                alpha = wls_all_samples_sharded(prob, None, None, y_is_dx=True, group=group)
+                u = np.zeros((hi - lo, 0))
+                import torch
+                cost_t = torch.tensor([cost_f_w(meth_f[lo:hi], np.asarray(ref)[lo:hi], alpha, np.asarray(counts)[lo:hi])],
+                                      dtype=torch.float64, device=prob.device)
+                dist.all_reduce(cost_t, group=group)                          # the cost over all rows
+                cost = float(cost_t.item())
+            else:
+                alpha = wls_all_samples(prob, None, None, y_is_dx=True)          # demethify.py:209-213
+                u = np.zeros((n_cpg, 0))
+                cost = cost_f_w(meth_f, np.asarray(ref), alpha, counts)
             ic_result = compute_bic(cost, 0, n_cpg, n_ct, n_samples) if ic == "BIC" else compute_aic(cost, 0, n_cpg, n_ct, n_samples)
         elif ic == "CCC":
             if ref is not None:

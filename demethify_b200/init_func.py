@@ -23,6 +23,19 @@ def wls_all_samples(X, d_x, R_full, extra=None, y_is_dx=False, precision=None):
     y = X, or d_x * X when y_is_dx (demethify.py:212).  `extra` is an optional second block of regressor columns
     (the unknown profiles u of deconvolution.py:51)."""
     prob = X if isinstance(X, DeviceProblem) else DeviceProblem(X, d_x, R_full, precision=precision)
+    desc, out, _keep = wls_desc(prob, extra, y_is_dx)
+    lib = _lib.lib()
+    h = _handle(prob.device.index if prob.device.index is not None else torch.cuda.current_device())
+    nbytes = C.c_size_t()
+    _lib.check(lib.dmf_wls_workspace_bytes(h, C.byref(desc), C.byref(nbytes)))
+    _ws, ws_ptr = aligned_workspace(nbytes.value, prob.device)
+    _lib.check(lib.dmf_wls_fit(h, C.byref(desc), ws_ptr, nbytes.value, _stream_ptr()))
+    return out.cpu().numpy()
+
+
+def wls_desc(prob, extra=None, y_is_dx=False):
+    """dmf_wls_desc_t of a resident problem with the optional second regressor block `extra` -> (desc, device output (K + K2) x N,
+    the tensors the descriptor points to that must outlive the call)."""
     dev, dt = prob.device, prob.dtype
     K2, R2 = 0, None
     if extra is not None:
@@ -35,14 +48,13 @@ def wls_all_samples(X, d_x, R_full, extra=None, y_is_dx=False, precision=None):
                         ldr2=_even(K2), X=prob.X.data_ptr(), D=prob.D.data_ptr(),
                         R1=prob.Rk.data_ptr() if prob.Rk is not None else None, R2=R2.data_ptr() if R2 is not None else None,
                         out=out.data_ptr())
-    lib = _lib.lib()
-    h = _handle(dev.index if dev.index is not None else torch.cuda.current_device())
-    nbytes = C.c_size_t()
-    _lib.check(lib.dmf_wls_workspace_bytes(h, C.byref(desc), C.byref(nbytes)))
-    ws = torch.empty(nbytes.value + 256, dtype=torch.uint8, device=dev)
-    ws_ptr = (ws.data_ptr() + 255) // 256 * 256
-    _lib.check(lib.dmf_wls_fit(h, C.byref(desc), C.c_void_p(ws_ptr), nbytes.value, _stream_ptr()))
-    return out.cpu().numpy()
+    return desc, out, R2
+
+
+def aligned_workspace(nbytes, device):
+    """A device workspace of `nbytes` at a 256-byte aligned address -> (tensor that owns it, address)."""
+    ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
+    return ws, C.c_void_p((ws.data_ptr() + 255) // 256 * 256)
 
 
 def wls_intercept(x, d_x, R_full):

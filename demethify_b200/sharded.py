@@ -8,20 +8,26 @@ and u plus a replica of alpha and of the fit state.  Per outer iteration (deconv
               then every rank runs the identical n_iter2 inner iterations on the reduced copy (dmf_gram_alpha_inner)
   cost        ONE sum all-reduce of 8 doubles per fit, then the identical termination test on every rank
 
-plus one max all-reduce (max d_x) at set-up.  Every rank therefore holds the same alpha and makes the same termination
+plus one max all-reduce (max d_x) at set-up.  The initial iterate is computed on the same row shards (`ShardedInit`): the
+`uniform` init and the reference-based fit all-reduce the WLS moment matrix, the SVD inits the N x N Gram matrix of the residual
+and the NNDSVD column norms.  Every rank therefore holds the same alpha and makes the same termination
 decision; u stays distributed.  `RowShardedFit` is the orchestration; the arithmetic sits behind a small backend
 interface whose product implementation (`GpuShardBackend`) drives libdemethify_sm100 through `FitBatch`.
 """
 import ctypes as C
 
 import numpy as np
+import numpy.random as rd
 import torch
 import torch.distributed as dist
 
 from . import _lib
-from .engine import DeviceProblem, FitBatch, _stream_ptr
+from .deconvolution import projection_simplex_sort_2d, set_seed
+from .engine import DeviceProblem, FitBatch, _handle, _stream_ptr, to_device
+from .init_func import aligned_workspace, wls_desc
 
-__all__ = ["row_range", "GpuShardBackend", "RowShardedFit", "mdwbssmf_deconv_sharded", "last_info"]
+__all__ = ["row_range", "GpuShardBackend", "RowShardedFit", "mdwbssmf_deconv_sharded", "last_info", "GpuInitBackend", "ShardedInit",
+           "wls_all_samples_sharded", "init_BSSMF_md_sharded", "init_BSSMF_md_p_sharded", "unsupervised_init_sharded"]
 
 _peer_cache = {}    # (group, world, device) -> (symmetric buffer, rendezvous handle, bytes): see enable_peer_exchange
 last_info = {}      # of the most recent mdwbssmf_deconv_sharded call: {"peer_exchange": bool, "peer_error": str | None, "collectives": int}
@@ -288,3 +294,243 @@ def mdwbssmf_deconv_sharded(u_local, alpha, X_local, d_local, R_local, n_u, n_it
         torch.cuda.synchronize()
         be.close()
     return u, a, n_outer, cost
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# The initial iterate on row-sharded data
+
+class GpuInitBackend:
+    """This rank's rows on its GPU for the initial iterate: the WLS moments (dmf_wls_moments / dmf_wls_solve) and the residual
+    reductions of the SVD inits (dmf_resid_gram / dmf_resid_project / dmf_nndsvd_apply)."""
+
+    def __init__(self, X_local, D_local, R_local, precision=None):
+        self.prob = X_local if isinstance(X_local, DeviceProblem) else DeviceProblem(X_local, D_local, R_local, precision=precision)
+        self.device = self.prob.device
+        self.M, self.N, self.K = self.prob.M, self.prob.N, self.prob.K
+        self.h = _handle(self.device.index if self.device.index is not None else torch.cuda.current_device())
+
+    def _wls_ws(self, desc):
+        nbytes = C.c_size_t()
+        _lib.check(_lib.lib().dmf_wls_workspace_bytes(self.h, C.byref(desc), C.byref(nbytes)))
+        return nbytes.value
+
+    def wls_moments(self, extra, y_is_dx):
+        """[(Kz Kz), N] moment matrix of this rank's rows (device tensor)."""
+        desc, out, keep = wls_desc(self.prob, extra, y_is_dx)
+        kz = self.K + (0 if extra is None else np.shape(extra)[1]) + 2
+        mom = torch.empty((kz * kz, self.N), dtype=torch.float64, device=self.device)
+        nbytes = self._wls_ws(desc) if self.M > 0 else 0
+        ws, ws_ptr = aligned_workspace(nbytes, self.device)
+        _lib.check(_lib.lib().dmf_wls_moments(self.h, C.byref(desc), C.c_void_p(mom.data_ptr()), ws_ptr, nbytes, _stream_ptr()))
+        return mom
+
+    def wls_solve(self, mom, M, K2):
+        """Per-sample NNLS on the all-reduced moments; M is the global row count -> (K + K2) x N ndarray."""
+        out = torch.zeros((self.K + K2, self.N), dtype=torch.float64, device=self.device)
+        desc = _lib.WlsDesc(M=int(M), N=self.N, K=self.K, K2=int(K2), out=out.data_ptr())
+        ws, ws_ptr = aligned_workspace(256, self.device)
+        _lib.check(_lib.lib().dmf_wls_solve(self.h, C.byref(desc), C.c_void_p(mom.data_ptr()), ws_ptr, 256, _stream_ptr()))
+        return out.cpu().numpy()
+
+    def _resid(self, H1):
+        """dmf_resid_desc_t over fp64 rows: r = max(x - R H1, 1e-8), or r = x when H1 is None (the reference-free init)."""
+        p = self.prob
+        X = p.X if p.dtype == torch.float64 else p.X.to(torch.float64)
+        keep = [X]
+        d = _lib.ResidDesc(M=p.M, N=p.N, K=0, ldx=X.shape[1], ldr=0, X=X.data_ptr())
+        if H1 is not None:
+            R = p.Rk if p.dtype == torch.float64 else p.Rk.to(torch.float64)
+            H = to_device(np.ascontiguousarray(H1, dtype=np.float64), torch.float64, self.device)
+            keep += [R, H]
+            d.K, d.ldr, d.R, d.H1 = p.K, R.shape[1], R.data_ptr(), H.data_ptr()
+        nbytes = C.c_size_t()
+        _lib.check(_lib.lib().dmf_resid_workspace_bytes(self.h, C.byref(d), C.byref(nbytes)))
+        ws, ws_ptr = aligned_workspace(nbytes.value, self.device)
+        keep.append(ws)
+        return d, ws_ptr, nbytes.value, keep
+
+    def resid_gram(self, H1):
+        """(sum over this rank's rows of r_m r_m^T (N x N), 1 where X has a negative entry (reference-free) else 0), device tensors."""
+        d, ws_ptr, nbytes, keep = self._resid(H1)
+        G = torch.empty((self.N, self.N), dtype=torch.float64, device=self.device)
+        neg = torch.zeros(1, dtype=torch.int32, device=self.device)
+        _lib.check(_lib.lib().dmf_resid_gram(self.h, C.byref(d), C.c_void_p(G.data_ptr()), C.c_void_p(neg.data_ptr()), ws_ptr, nbytes,
+                                             _stream_ptr()))
+        return G, neg
+
+    def resid_project(self, H1, Vh, inv_sigma):
+        """(U = r Vh^T diag(inv_sigma) of this rank's rows, [|u+|^2 per component, |u-|^2 per component] of those rows)."""
+        d, ws_ptr, nbytes, keep = self._resid(H1)
+        rank = Vh.shape[0]
+        Vh, inv_sigma = Vh.contiguous(), inv_sigma.contiguous()
+        U = torch.empty((self.M, rank), dtype=torch.float64, device=self.device)
+        sums = torch.empty(2 * rank, dtype=torch.float64, device=self.device)
+        _lib.check(_lib.lib().dmf_resid_project(self.h, C.byref(d), C.c_void_p(Vh.data_ptr()), C.c_void_p(inv_sigma.data_ptr()), rank,
+                                                C.c_void_p(U.data_ptr()), C.c_void_p(sums.data_ptr()), ws_ptr, nbytes, _stream_ptr()))
+        return U, sums
+
+    def nndsvd_apply(self, U, Vh, sigma, sums):
+        """NNDSVD factors (W rows of this rank, H) from U and the all-reduced sums -> ndarrays."""
+        rank = Vh.shape[0]
+        Vh, sigma, sums = Vh.contiguous(), sigma.contiguous(), sums.contiguous()
+        W = torch.empty((self.M, rank), dtype=torch.float64, device=self.device)
+        H = torch.empty((rank, self.N), dtype=torch.float64, device=self.device)
+        _lib.check(_lib.lib().dmf_nndsvd_apply(C.c_void_p(U.data_ptr()), self.M, C.c_void_p(Vh.data_ptr()), C.c_void_p(sigma.data_ptr()),
+                                               C.c_void_p(sums.data_ptr()), self.N, rank, C.c_void_p(W.data_ptr()),
+                                               C.c_void_p(H.data_ptr()), _stream_ptr()))
+        return W.cpu().numpy(), H.cpu().numpy()
+
+
+class ShardedInit:
+    """The row reductions of the initial iterate on row-sharded data; `backend` does this rank's arithmetic (GpuInitBackend, or a
+    numpy restatement in the tests), every rank of `group` calls the same steps in the same order."""
+
+    def __init__(self, backend, group=None):
+        self.be, self.group = backend, group
+        rows = torch.tensor([backend.M], dtype=torch.int64, device=backend.device)
+        if self._multi():
+            parts = [torch.zeros_like(rows) for _ in range(dist.get_world_size(group))]
+            dist.all_gather(parts, rows, group=group)
+            counts = [int(t.item()) for t in parts]
+        else:
+            counts = [backend.M]
+        rank = dist.get_rank(group) if self._multi() else 0
+        self.M = sum(counts)                          # global row count
+        self.lo = sum(counts[:rank])                  # this rank's rows are lo .. lo + backend.M of the full matrix
+        self.hi = self.lo + backend.M
+
+    def _multi(self):
+        return dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
+
+    def _allreduce(self, t, op=None):
+        if self._multi():
+            dist.all_reduce(t, op=op or dist.ReduceOp.SUM, group=self.group)
+        return t
+
+    def _broadcast(self, t):
+        if self._multi():
+            dist.broadcast(t, src=dist.get_global_rank(self.group, 0) if self.group is not None else 0, group=self.group)
+        return t
+
+    def wls(self, extra=None, y_is_dx=False):
+        """wls_intercept of every sample over all rows (init_func.py:8-14): `extra` holds this rank's rows of the second regressor
+        block.  -> (K + K2) x N ndarray, the same on every rank."""
+        mom = self._allreduce(self.be.wls_moments(extra, y_is_dx))
+        return self.be.wls_solve(mom, self.M, 0 if extra is None else np.shape(extra)[1])
+
+    def nndsvd(self, rank, H1=None):
+        """nndsvd_initialize (init_func.py:40-82, flag 0) of the residual max(X - R_trunc H1, 1e-8), or of X when H1 is None, over
+        all rows -> (this rank's rows of W, H).  The right singular vectors and the singular values come from the eigen-
+        decomposition of the all-reduced N x N Gram matrix (descending, sigma = sqrt(max(lambda, 0))), the left ones from
+        projecting this rank's residual rows on them."""
+        G, neg = self.be.resid_gram(H1)
+        self._allreduce(G)
+        if H1 is None and int(self._allreduce(neg, dist.ReduceOp.MAX).item()):
+            raise ValueError("The input matrix contains negative elements.")
+        if rank > min(self.M, self.be.N):
+            raise IndexError(f"index {min(self.M, self.be.N)} is out of bounds for axis 1 with size {min(self.M, self.be.N)}")
+        lam, V = torch.linalg.eigh(G)
+        order = torch.arange(G.shape[0] - 1, G.shape[0] - 1 - rank, -1, device=G.device)
+        Vh = V[:, order].T.contiguous()
+        sigma = torch.sqrt(torch.clamp(lam[order], min=0.0)).contiguous()
+        self._broadcast(Vh)                           # one decomposition for all ranks
+        self._broadcast(sigma)
+        inv = torch.where(sigma > 0, 1.0 / sigma, torch.zeros_like(sigma))
+        U, sums = self.be.resid_project(H1, Vh, inv)
+        self._allreduce(sums)
+        return self.be.nndsvd_apply(U, Vh, sigma, sums)
+
+
+def _init_of(backend, X_local, d_local, R_local, group):
+    return ShardedInit(backend if backend is not None else GpuInitBackend(X_local, d_local, R_local), group)
+
+
+def wls_all_samples_sharded(X_local, d_local, R_local, extra=None, y_is_dx=False, group=None, backend=None):
+    """init_func.wls_all_samples over row-sharded data: every rank passes ITS rows (and its rows of `extra`) -> (K [+ K2], N)
+    ndarray, the same on every rank.  With y_is_dx it is the reference-based fit (n_u = 0, demethify.py:209-213)."""
+    return _init_of(backend, X_local, d_local, R_local, group).wls(extra, y_is_dx)
+
+
+def _draw_sharded(si, init_option, K, n_u):
+    """deconvolution._draw on row-sharded data: every rank draws the full u from the global stream and keeps its rows."""
+    M, N, lo, hi = si.M, si.be.N, si.lo, si.hi
+    if init_option == "uniform":
+        u = rd.uniform(size=(M, n_u))[lo:hi]
+        alpha = si.wls(extra=u)
+    elif init_option == "uniform_":
+        u = rd.uniform(size=(M, n_u))[lo:hi]
+        alpha = rd.dirichlet(np.ones(K + n_u), N).T
+    elif init_option == "beta":
+        temp = np.ones((M, n_u))
+        u = rd.beta(temp * 0.5, temp * 0.5)[lo:hi]
+        alpha = rd.dirichlet(np.ones(K + n_u), N).T
+    elif init_option == "SVD":
+        H1 = si.wls()                                 # constrained_nndsvd (init_func.py:17-37)
+        W2, H2 = si.nndsvd(n_u, H1)
+        u, alpha = np.clip(W2, 0, 1), np.vstack([H1, H2])
+    elif init_option == "ICA":
+        raise NotImplementedError("--init ICA forms an M x M covariance (init_func.py:120) and is out of scope of the "
+                                  "B200 path (SURVEY.md 2.1 row 4); use uniform_, uniform, beta or SVD")
+    else:
+        raise ValueError(f"unknown init option {init_option!r}")
+    return u, alpha
+
+
+def init_BSSMF_md_sharded(init_option, X_local, d_local, R_local, n_u, seed=None, group=None, backend=None):
+    """deconvolution.init_BSSMF_md over row-sharded data: every rank passes ITS rows of X, d_x and R_trunc (or a resident
+    DeviceProblem of them) -> (u_local, alpha); alpha is the same on every rank and u_local holds this rank's rows of the
+    single-process u."""
+    set_seed(seed)
+    si = _init_of(backend, X_local, d_local, R_local, group)
+    if init_option != "uniform_" and n_u > si.be.N:
+        init_option = "uniform_"
+    u, alpha = _draw_sharded(si, init_option, si.be.K, n_u)
+    if init_option == "SVD":
+        alpha = projection_simplex_sort_2d(alpha)
+    if alpha[-n_u:][0].all() == 0.0:                      # deconvolution.py:74-76
+        alpha[-n_u:][0] = 1e-10
+        alpha[:-n_u] = (1 - 1e-10) * alpha[:-n_u]
+    return u, alpha
+
+
+def init_BSSMF_md_p_sharded(init_option, X_local, d_local, R_local, n_u, purity, seed=None, group=None, backend=None):
+    """deconvolution.init_BSSMF_md_p over row-sharded data -> (u_local, alpha)."""
+    set_seed(seed)
+    si = _init_of(backend, X_local, d_local, R_local, group)
+    nb = si.be.N
+    if init_option != "uniform" and n_u > nb:
+        if not si._multi() or dist.get_rank(group) == 0:
+            print("The number of unknowns is greater than the number of samples, we'll go with a uniform initialisation. ")
+        init_option = "uniform"
+    if init_option != "uniform_" and n_u > nb:
+        init_option = "uniform_"
+    u, alpha = _draw_sharded(si, init_option, si.be.K, n_u)
+    if init_option == "SVD":                               # deconvolution.py:262
+        alpha = np.vstack((purity * projection_simplex_sort_2d(alpha[:-n_u]), projection_simplex_sort_2d(alpha[-n_u:])))
+    return u, alpha
+
+
+def unsupervised_init_sharded(init_option, X_local, d_local, n_u, seed=None, group=None, backend=None):
+    """The initial iterate of deconvolution.unsupervised_deconv (deconvolution.py:107-150) over row-sharded data ->
+    (u_local, alpha)."""
+    set_seed(seed)
+    si = _init_of(backend, X_local, d_local, None, group)
+    M, nb, lo, hi = si.M, si.be.N, si.lo, si.hi
+    if init_option != "uniform_" and n_u > nb:
+        init_option = "uniform_"
+    if init_option == "uniform_":
+        u = rd.uniform(size=(M, n_u))[lo:hi]
+        alpha = rd.dirichlet(np.ones(n_u), nb).T
+    elif init_option == "beta":
+        temp = np.ones((M, n_u))
+        u = rd.beta(temp * 0.5, temp * 0.5)[lo:hi]
+        alpha = rd.dirichlet(np.ones(n_u), nb).T
+    elif init_option == "SVD":
+        u, alpha = si.nndsvd(n_u)
+        u = u.clip(0, 1)
+        alpha = projection_simplex_sort_2d(alpha)
+    elif init_option == "uniform":
+        raise NameError("name 'R_trunc' is not defined")   # what the reference does (deconvolution.py:117, SURVEY Q8)
+    else:
+        raise NotImplementedError(f"init option {init_option!r} is not available on the B200 path")
+    return u, alpha

@@ -239,6 +239,39 @@ typedef struct dmf_wls_desc {
 } dmf_wls_desc_t;
 int dmf_wls_workspace_bytes(dmf_handle_t h, const dmf_wls_desc_t* d, size_t* bytes);
 int dmf_wls_fit(dmf_handle_t h, const dmf_wls_desc_t* d, void* workspace_dev, size_t workspace_bytes, void* stream);
+/* dmf_wls_fit in two halves, for CpG rows sharded over several GPUs.  dmf_wls_moments streams the caller's M rows and writes the
+ * weighted moment matrix  mom[(p Kz + q) N + j] = sum_m D[m,j] z_p z_q,  z = [1, y, R1 row, R2 row],  Kz = K + K2 + 2  (DEVICE
+ * buffer of Kz Kz N doubles; all zero when M = 0).  dmf_wls_solve runs the per-sample NNLS on a moment matrix the caller may have
+ * summed over GPUs: it reads M (the GLOBAL row count: the NNLS tolerance depends on it), N, K, K2 and out from the descriptor and
+ * needs 256 bytes of workspace.  Moments then solve on one GPU give dmf_wls_fit's result bit for bit. */
+int dmf_wls_moments(dmf_handle_t h, const dmf_wls_desc_t* d, double* mom, void* workspace_dev, size_t workspace_bytes, void* stream);
+int dmf_wls_solve(dmf_handle_t h, const dmf_wls_desc_t* d, const double* mom, void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* NNDSVD of the floored residual over row-sharded rows (init_func.py:17-93) ------------------------------------------------ */
+/* r_mj = max(X[m,j] - sum_k R[m,k] H1[k,j], 1e-8) for K > 0 (the partial / purity SVD init), r_mj = X[m,j] for K = 0 (the
+ * reference-free SVD init).  X (M x ldx) and R (M x ldr) are fp64 with even, zero-padded pitches; H1 is K x N row-major;
+ * N <= 512.  The residual is formed on the fly and never written to memory.  M = 0 is allowed (a GPU without rows). */
+typedef struct dmf_resid_desc {
+    int64_t M;
+    int32_t N, K;
+    int64_t ldx, ldr;
+    const double* X;
+    const double* R;
+    const double* H1;
+} dmf_resid_desc_t;
+int dmf_resid_workspace_bytes(dmf_handle_t h, const dmf_resid_desc_t* d, size_t* bytes);
+/* G = sum_m r_m r_m^T over the caller's rows (N x N, DEVICE, fp64 on the tensor cores; bit-reproducible for a given device and
+ * shape).  *has_negative (DEVICE int32) becomes 1 when K = 0 and X has a negative entry, else 0. */
+int dmf_resid_gram(dmf_handle_t h, const dmf_resid_desc_t* d, double* G, int32_t* has_negative, void* workspace_dev,
+                   size_t workspace_bytes, void* stream);
+/* U = r Vh^T diag(inv_sigma) for the caller's rows (M x rank row-major; Vh is rank x N row-major, rank <= 32), and
+ * sums[i] = sum_m max(U[m,i], 0)^2, sums[rank + i] = sum_m max(-U[m,i], 0)^2 over the caller's rows (DEVICE, 2 rank doubles). */
+int dmf_resid_project(dmf_handle_t h, const dmf_resid_desc_t* d, const double* Vh, const double* inv_sigma, int32_t rank, double* U,
+                      double* sums, void* workspace_dev, size_t workspace_bytes, void* stream);
+/* dmf_nndsvd_split's rule on the caller's rows of U with the norms of U taken from `sums` (dmf_resid_project's sums added over
+ * all GPUs): W (M x rank, the caller's rows) and H (rank x N), both row-major. */
+int dmf_nndsvd_apply(const double* U, int64_t M, const double* Vh, const double* S, const double* sums, int32_t N, int32_t rank,
+                     double* W, double* H, void* stream);
 
 /* utilities ------------------------------------------------------------------------------------ */
 /* narrow fp64/fp32/int64 coverage to u16 with range/integrality check; *bad receives the number of

@@ -2,7 +2,8 @@
 """2+ GPU check of CpG-row sharding (run under torchrun on the GPU box):
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/sharded_check.py
 Every rank fits its row range over NCCL; rank 0 gathers u and compares alpha, u and the outer-iteration count with the
-CPU oracle on the full problem."""
+CPU oracle on the full problem.  Then the `demethify` command runs its main fit with --shard rows for every init option (partial,
+purity, reference-free, n_u = 0) and rank 0 compares the CSV files with a one-GPU run of the same seed."""
 import os
 import sys
 
@@ -55,8 +56,61 @@ def main():
             ok &= good
             print(f"sharded_check world={world} peer_xchg={peer} graph={graph} it1={it1}: n_outer={n_outer} oracle={tr['n_outer']} max|d alpha|={da:.2e} max|d u|={du:.2e} "
                   f"alpha replicated={same_alpha} peer={sharded.last_info} -> {'OK' if good else 'FAIL'}", flush=True)
+    ok &= cli_check(rank, world)
     dist.destroy_process_group()
     sys.exit(0 if ok else 1)
+
+
+def cli_check(rank, world):
+    import tempfile
+    import pandas as pd
+    from demethify_b200 import demethify
+    rs = np.random.RandomState(8)
+    M, N, K = 9001, 10, 5
+    Rf = rs.beta(0.5, 0.5, size=(M, K + 2))
+    D = rs.poisson(40, size=(M, N)) + 1
+    X = rs.binomial(D, np.clip(Rf @ rs.dirichlet(np.ones(K + 2), N).T, 0, 1)) / D
+    box = [tempfile.mkdtemp(prefix="dmf_cli_") if rank == 0 else None]
+    dist.broadcast_object_list(box, src=0)
+    d = box[0]
+    if rank == 0:
+        pd.DataFrame(Rf[:, :K], columns=[f"ct{k}" for k in range(K)]).to_csv(f"{d}/ref.csv", index=False)
+        for j in range(N):
+            pd.DataFrame({"percent_modified": X[:, j], "valid_coverage": D[:, j]}).to_csv(f"{d}/s{j}.csv", index=False)
+    dist.barrier()
+    files = [f"{d}/s{j}.csv" for j in range(N)]
+    cases = [("uniform_", ["--nbunknown", "2"]), ("uniform", ["--nbunknown", "2"]), ("beta", ["--nbunknown", "2"]),
+             ("SVD", ["--nbunknown", "2"]), ("SVD", ["--nbunknown", "2", "--purity"] + ["60"] * N), ("SVD", ["--nbunknown", "2", "--noref"]),
+             ("uniform_", ["--nbunknown", "0"])]
+    ok = True
+    for c, (init, extra) in enumerate(cases):
+        ref = [] if "--noref" in extra else ["--ref", f"{d}/ref.csv"]
+        extra = [e for e in extra if e != "--noref"]
+        common = ["--methfreq"] + files + ref + ["--init", init, "--iterations", "300", "20", "--termination", "1e-2", "--seed", "3",
+                                                  "--noprint"] + extra
+        demethify.main(common + ["--outdir", f"{d}/rows{c}", "--shard", "rows"])
+        dist.barrier()
+        if rank == 0:
+            env = os.environ["WORLD_SIZE"]
+            os.environ["WORLD_SIZE"] = "1"                         # the same command on one GPU
+            try:
+                demethify.main(common + ["--outdir", f"{d}/one{c}"])
+            finally:
+                os.environ["WORLD_SIZE"] = env
+            dev = 0.0
+            for name in ("celltypes_proportions.csv", "methylation_profile_estimate.csv"):
+                if os.path.exists(f"{d}/one{c}/{name}"):
+                    a = pd.read_csv(f"{d}/rows{c}/{name}").select_dtypes("number").values
+                    b = pd.read_csv(f"{d}/one{c}/{name}").select_dtypes("number").values
+                    dev = max(dev, np.abs(a - b).max() if a.shape == b.shape else np.inf)
+            good = dev <= 1e-6
+            ok &= good
+            print(f"sharded_check cli world={world} --init {init} {' '.join(extra[:3])}{' (reference-free)' if not ref else ''}: "
+                  f"max|rows - one GPU|={dev:.2e} -> {'OK' if good else 'FAIL'}", flush=True)
+        dist.barrier()
+    box = [ok]
+    dist.broadcast_object_list(box, src=0)
+    return box[0]
 
 
 if __name__ == "__main__":
