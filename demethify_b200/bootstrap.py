@@ -17,7 +17,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .deconvolution import init_BSSMF_md, init_BSSMF_md_p
+from .deconvolution import _init_option, _initial_iterate, _quiet, _zero_guard, init_BSSMF_md, init_BSSMF_md_p
 from .engine import DeviceProblem, FitBatch, device_free_bytes
 from .init_func import wls_all_samples
 
@@ -70,17 +70,8 @@ def resample_indices(seed, M):
 def _shape_only_init(seed, init_option, M, K, N, n_u, with_zero_guard):
     """uniform_ / beta inits (deconvolution.py:54-61, :246-253) from a PRIVATE legacy stream: RandomState(seed) produces
     exactly what the reference's set_seed(seed) + global numpy.random calls produce, and is safe to use from worker threads."""
-    rs = np.random.RandomState(seed)
-    if init_option == "uniform_":
-        u = rs.uniform(size=(M, n_u))
-    else:
-        temp = np.ones((M, n_u))
-        u = rs.beta(temp * 0.5, temp * 0.5)
-    alpha = rs.dirichlet(np.ones(K + n_u), N).T
-    if with_zero_guard and alpha[-n_u:][0].all() == 0.0:      # deconvolution.py:74-76 (init_BSSMF_md only)
-        alpha[-n_u:][0] = 1e-10
-        alpha[:-n_u] = (1 - 1e-10) * alpha[:-n_u]
-    return u, alpha
+    return _initial_iterate("partial" if with_zero_guard else "purity", init_option, M, N, K, n_u, rng=np.random.RandomState(seed),
+                            say=_quiet)
 
 
 def device_draws(chunk, M, n_u, K, N, dev, with_zero_guard):
@@ -110,10 +101,7 @@ def device_draws(chunk, M, n_u, K, N, dev, with_zero_guard):
     for k in range(B):
         rs.set_state(("MT19937", st[k, :624], int(st[k, 624]), 0, 0.0))
         alpha = rs.dirichlet(np.ones(K + n_u), N).T
-        if with_zero_guard and alpha[-n_u:][0].all() == 0.0:      # deconvolution.py:74-76 (init_BSSMF_md only)
-            alpha[-n_u:][0] = 1e-10
-            alpha[:-n_u] = (1 - 1e-10) * alpha[:-n_u]
-        A0[k] = alpha
+        A0[k] = _zero_guard(alpha, n_u) if with_zero_guard else alpha      # init_BSSMF_md only
     return idx_d, u0_d, A0
 
 
@@ -174,13 +162,7 @@ def bootstrap_fits(n_bootstrap, n_u, meth_f, counts, ref, init_option, n_iter1, 
     if n_u > 0:
         # the reference falls back to uniform_ when n_u > N (deconvolution.py:44-45, :234-239), then dispatches on the option;
         # anything it would run that this path does not have is refused BEFORE a resample is drawn (never silently replaced)
-        if init_option != "uniform_" and n_u > N:
-            init_option = "uniform_"
-        if init_option == "ICA":
-            raise NotImplementedError("--init ICA forms an M x M covariance (init_func.py:120) and is out of scope of the B200 path "
-                                      "(SURVEY.md 2.1 row 4); use uniform_, uniform, beta or SVD")
-        if init_option not in ("uniform_", "uniform", "beta", "SVD"):
-            raise ValueError(f"unknown init option {init_option!r}")
+        init_option = _init_option("partial" if purity is None else "purity", init_option, n_u, N, say=_quiet)
     seeds = bootstrap_seeds(seed, n_bootstrap) if seeds is None else list(seeds)
     n_bootstrap = len(seeds)
     restarts = max(1, int(restarts))

@@ -11,7 +11,7 @@ import torch
 
 from . import _lib
 from .engine import DeviceProblem, FitBatch, to_device
-from .init_func import wls_intercept, wls_all_samples, constrained_nndsvd, nndsvd_initialize
+from .init_func import wls_intercept, wls_all_samples, nndsvd_initialize
 
 __all__ = ["set_seed", "cost_f_w", "projection_simplex_sort_2d", "init_BSSMF_md", "init_BSSMF_md_p", "update_u", "update_alpha",
            "frank_wolfe_nmf", "mdwbssmf_deconv", "mdwbssmf_deconv_p", "unsupervised_deconv", "last_fit_info", "best_of_restarts"]
@@ -71,44 +71,93 @@ def projection_simplex_sort_2d(v, z=1):
     return np.maximum(v - theta, 0)
 
 
-def _draw(init_option, meth_frequency, d_x, R_trunc, n_u):
-    M, K = R_trunc.shape
-    nb = meth_frequency.shape[1]
-    if init_option == "uniform":
-        u = rd.uniform(size=(M, n_u))
-        alpha = wls_all_samples(meth_frequency, d_x, R_trunc, extra=u)      # per-sample wls_intercept on [R_trunc | u], :49-52
-    elif init_option == "uniform_":
-        u = rd.uniform(size=(M, n_u))
-        alpha = rd.dirichlet(np.ones(K + n_u), nb).T
-    elif init_option == "beta":
-        temp = np.ones((M, n_u))
-        u = rd.beta(temp * 0.5, temp * 0.5)
-        alpha = rd.dirichlet(np.ones(K + n_u), nb).T
-    elif init_option == "SVD":
-        W, alpha = constrained_nndsvd(meth_frequency, R_trunc, d_x, rank=n_u, flag=0)
-        u = W[:, K:]
+def _quiet(message):
+    pass
+
+
+def _init_option(variant, init_option, n_u, N, say=print):
+    """The option the reference dispatches on for `variant` ("partial", "purity" or "free", see _initial_iterate).  With more
+    unknowns than samples the purity variant first falls back to `uniform` and says so (:232-234), then every variant falls back to
+    `uniform_` (:44-45); an option this path does not run raises what the reference raises, or NotImplementedError."""
+    if variant == "purity" and init_option != "uniform" and n_u > N:
+        say("The number of unknowns is greater than the number of samples, we'll go with a uniform initialisation. ")
+        init_option = "uniform"
+    if init_option != "uniform_" and n_u > N:
+        init_option = "uniform_"
+    if variant == "free":
+        if init_option == "uniform":
+            raise NameError("name 'R_trunc' is not defined")   # what the reference does (deconvolution.py:117, SURVEY Q8)
+        if init_option not in ("uniform_", "beta", "SVD"):
+            raise NotImplementedError(f"init option {init_option!r} is not available on the B200 path")
     elif init_option == "ICA":
         raise NotImplementedError("--init ICA forms an M x M covariance (init_func.py:120) and is out of scope of the "
                                   "B200 path (SURVEY.md 2.1 row 4); use uniform_, uniform, beta or SVD")
-    else:
+    elif init_option not in ("uniform_", "uniform", "beta", "SVD"):
         raise ValueError(f"unknown init option {init_option!r}")
-    return u, alpha
+    return init_option
+
+
+def _zero_guard(alpha, n_u):
+    """:74-76 (init_BSSMF_md only): a zero in the first unknown row of alpha sets that row to 1e-10 and scales the known rows by
+    1 - 1e-10, in place."""
+    if alpha[-n_u:][0].all() == 0.0:
+        alpha[-n_u:][0] = 1e-10
+        alpha[:-n_u] = (1 - 1e-10) * alpha[:-n_u]
+    return alpha
+
+
+def _initial_iterate(variant, init_option, M, N, K, n_u, rows=None, wls=None, nndsvd=None, purity=None, rng=rd, say=print):
+    """The reference's initial iterate of an M x N problem with K known and n_u unknown types -> (rows [lo, hi) = `rows` of u0, all M
+    rows when None; alpha0).  `variant` is "partial" (init_BSSMF_md, :40-78), "purity" (init_BSSMF_md_p, :228-267) or "free"
+    (unsupervised_deconv, :107-150, K = 0).  `rng` is numpy's legacy stream: the numpy.random module after set_seed, or a private
+    RandomState(seed); the draws are issued in the reference's order, so u0 and alpha0 are bit-identical to it.  The data-dependent
+    options call `wls(extra=None)`, the reference-based fit of every sample over all rows with the caller's rows of u as an extra
+    regressor block, and `nndsvd(rank, H1=None)`, the NNDSVD (flag 0) of max(X - R_trunc H1, 1e-8), or of X, -> (the caller's rows of
+    W, H).  `say` prints the purity fallback message."""
+    init_option = _init_option(variant, init_option, n_u, N, say)
+    if init_option == "SVD":
+        if variant == "free":
+            u, alpha = nndsvd(n_u)
+            return u.clip(0, 1), projection_simplex_sort_2d(alpha)
+        H1 = wls()                                         # constrained_nndsvd (init_func.py:17-37)
+        W2, H2 = nndsvd(n_u, H1)
+        u, alpha = np.clip(W2, 0, 1), np.vstack([H1, H2])
+        if variant == "purity":                            # :262
+            return u, np.vstack((purity * projection_simplex_sort_2d(alpha[:-n_u]), projection_simplex_sort_2d(alpha[-n_u:])))
+        alpha = projection_simplex_sort_2d(alpha)
+    else:
+        if init_option == "beta":
+            temp = np.ones((M, n_u))
+            u = rng.beta(temp * 0.5, temp * 0.5)
+        else:
+            u = rng.uniform(size=(M, n_u))
+        if rows is not None:
+            u = u[rows[0]:rows[1]]
+        # `uniform`: per-sample wls_intercept on [R_trunc | u] (:49-52)
+        alpha = wls(extra=u) if init_option == "uniform" else rng.dirichlet(np.ones(K + n_u), N).T
+    return u, (_zero_guard(alpha, n_u) if variant == "partial" else alpha)
+
+
+def _host_steps(meth_frequency, d_x, R_trunc):
+    """`wls` and `nndsvd` of _initial_iterate on one process: wls_all_samples of the caller's data (a resident DeviceProblem too), and
+    nndsvd_initialize of the float64 host residual that constrained_nndsvd forms."""
+    def wls(extra=None):
+        return wls_all_samples(meth_frequency, d_x, R_trunc, extra=extra)
+
+    def nndsvd(rank, H1=None):
+        Y = np.asarray(meth_frequency, dtype=np.float64)
+        if H1 is not None:
+            Y = np.maximum(Y - np.asarray(R_trunc, dtype=np.float64) @ H1, 1e-8)
+        return nndsvd_initialize(Y, rank=rank)
+    return dict(wls=wls, nndsvd=nndsvd)
 
 
 def init_BSSMF_md(init_option, meth_frequency, d_x, R_trunc, n_u, seed=None, rb_alg=wls_intercept):
     """deconvolution.py:40-78."""
     set_seed(seed)
-    nb = meth_frequency.shape[1]
-    if init_option != "uniform_" and n_u > nb:
-        init_option = "uniform_"
-    u, alpha = _draw(init_option, meth_frequency, d_x, R_trunc, n_u)
-    if init_option == "SVD":
-        alpha = projection_simplex_sort_2d(alpha)
-    R = np.c_[R_trunc, u]
-    if alpha[-n_u:][0].all() == 0.0:                      # :74-76
-        alpha[-n_u:][0] = 1e-10
-        alpha[:-n_u] = (1 - 1e-10) * alpha[:-n_u]
-    return u, R, alpha
+    M, K = R_trunc.shape
+    u, alpha = _initial_iterate("partial", init_option, M, meth_frequency.shape[1], K, n_u, **_host_steps(meth_frequency, d_x, R_trunc))
+    return u, np.c_[R_trunc, u], alpha
 
 
 def _problem(meth_frequency, d_x, R_trunc):
@@ -179,17 +228,10 @@ def update_alpha(n_iter2, alpha, a2, l_h_, l_h, alpha_, R, d_x, meth_frequency):
 def init_BSSMF_md_p(init_option, meth_frequency, d_x, R_trunc, n_u, purity, rb_alg=wls_intercept, seed=None):
     """deconvolution.py:228-267."""
     set_seed(seed)
-    nb = meth_frequency.shape[1]
-    if init_option != "uniform" and n_u > nb:
-        print("The number of unknowns is greater than the number of samples, we'll go with a uniform initialisation. ")
-        init_option = "uniform"
-    if init_option != "uniform_" and n_u > nb:
-        init_option = "uniform_"
-    u, alpha = _draw(init_option, meth_frequency, d_x, R_trunc, n_u)
-    if init_option == "SVD":                               # :262
-        alpha = np.vstack((purity * projection_simplex_sort_2d(alpha[:-n_u]), projection_simplex_sort_2d(alpha[-n_u:])))
-    R = np.c_[R_trunc, u]
-    return u, R, alpha
+    M, K = R_trunc.shape
+    u, alpha = _initial_iterate("purity", init_option, M, meth_frequency.shape[1], K, n_u, purity=purity,
+                                **_host_steps(meth_frequency, d_x, R_trunc))
+    return u, np.c_[R_trunc, u], alpha
 
 
 def frank_wolfe_nmf(W1, W2, meth_frequency, H1, H2, purity, n_iter2, d_x):
@@ -237,23 +279,7 @@ def unsupervised_deconv(meth_frequency, n_u, d_x, init_option, n_iter1=100000, n
     """deconvolution.py:107-184 — reference-free variant (no R_trunc)."""
     set_seed(seed)
     M, nb = meth_frequency.shape
-    if init_option != "uniform_" and n_u > nb:
-        init_option = "uniform_"
-    if init_option == "uniform_":
-        u = rd.uniform(size=(M, n_u))
-        alpha = rd.dirichlet(np.ones(n_u), nb).T
-    elif init_option == "beta":
-        temp = np.ones((M, n_u))
-        u = rd.beta(temp * 0.5, temp * 0.5)
-        alpha = rd.dirichlet(np.ones(n_u), nb).T
-    elif init_option == "SVD":
-        u, alpha = nndsvd_initialize(meth_frequency, rank=n_u)
-        u = u.clip(0, 1)
-        alpha = projection_simplex_sort_2d(alpha)
-    elif init_option == "uniform":
-        raise NameError("name 'R_trunc' is not defined")   # what the reference does (deconvolution.py:117, SURVEY Q8)
-    else:
-        raise NotImplementedError(f"init option {init_option!r} is not available on the B200 path")
+    u, alpha = _initial_iterate("free", init_option, M, nb, 0, n_u, **_host_steps(meth_frequency, d_x, None))
     return _solve(_lib.DMF_MODE_UNSUPERVISED, u, alpha, meth_frequency, d_x, None, n_u, n_iter1, n_iter2, tol)
 
 

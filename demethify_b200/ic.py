@@ -9,7 +9,7 @@ import torch.distributed as dist
 import tqdm
 
 from . import _lib
-from .deconvolution import init_BSSMF_md, mdwbssmf_deconv, unsupervised_deconv, cost_f_w, last_fit_info
+from .deconvolution import _initial_iterate, init_BSSMF_md, mdwbssmf_deconv, unsupervised_deconv, cost_f_w, last_fit_info
 from .engine import DeviceProblem, FitBatch
 
 __all__ = ["compute_bic", "compute_aic", "compute_consensus_matrix", "compute_ccc", "run_deconvolution", "bicross_validation",
@@ -149,12 +149,10 @@ def _row_sharded_member(prob_local, lo, hi, M, K, N, n_u, init_option, seed, ite
     """One sweep member with the CpG rows sharded over the ranks of `group` (BASELINE config 5): every rank draws the same
     initial iterate from the same seed, keeps its rows of u and runs the row-sharded solver -> (u_local, alpha, cost).  The
     `uniform` and `SVD` inits all-reduce their row sums (sharded.ShardedInit)."""
-    from .bootstrap import _shape_only_init
     from .sharded import init_BSSMF_md_sharded, mdwbssmf_deconv_sharded
     if init_option in ("uniform_", "beta"):
         # RandomState(seed) == the reference's set_seed(seed) + global stream (int -> init_genrand, list -> init_by_array, Q1)
-        u0, a0 = _shape_only_init(seed, init_option if n_u <= N else "uniform_", M, K, N, n_u, with_zero_guard=True)
-        u0 = u0[lo:hi]
+        u0, a0 = _initial_iterate("partial", init_option, M, N, K, n_u, rows=(lo, hi), rng=np.random.RandomState(seed))
     elif init_option in ("uniform", "SVD"):
         u0, a0 = init_BSSMF_md_sharded(init_option, prob_local, None, None, n_u, seed=seed, group=group)
     else:

@@ -17,12 +17,11 @@ interface whose product implementation (`GpuShardBackend`) drives libdemethify_s
 import ctypes as C
 
 import numpy as np
-import numpy.random as rd
 import torch
 import torch.distributed as dist
 
 from . import _lib
-from .deconvolution import projection_simplex_sort_2d, set_seed
+from .deconvolution import _initial_iterate, _quiet, set_seed
 from .engine import DeviceProblem, FitBatch, _handle, _stream_ptr, to_device
 from .init_func import aligned_workspace, wls_desc
 
@@ -451,63 +450,22 @@ def wls_all_samples_sharded(X_local, d_local, R_local, extra=None, y_is_dx=False
     return _init_of(backend, X_local, d_local, R_local, group).wls(extra, y_is_dx)
 
 
-def _draw_sharded(si, init_option, K, n_u):
-    """deconvolution._draw on row-sharded data: every rank draws the full u from the global stream and keeps its rows."""
-    M, N, lo, hi = si.M, si.be.N, si.lo, si.hi
-    if init_option == "uniform":
-        u = rd.uniform(size=(M, n_u))[lo:hi]
-        alpha = si.wls(extra=u)
-    elif init_option == "uniform_":
-        u = rd.uniform(size=(M, n_u))[lo:hi]
-        alpha = rd.dirichlet(np.ones(K + n_u), N).T
-    elif init_option == "beta":
-        temp = np.ones((M, n_u))
-        u = rd.beta(temp * 0.5, temp * 0.5)[lo:hi]
-        alpha = rd.dirichlet(np.ones(K + n_u), N).T
-    elif init_option == "SVD":
-        H1 = si.wls()                                 # constrained_nndsvd (init_func.py:17-37)
-        W2, H2 = si.nndsvd(n_u, H1)
-        u, alpha = np.clip(W2, 0, 1), np.vstack([H1, H2])
-    elif init_option == "ICA":
-        raise NotImplementedError("--init ICA forms an M x M covariance (init_func.py:120) and is out of scope of the "
-                                  "B200 path (SURVEY.md 2.1 row 4); use uniform_, uniform, beta or SVD")
-    else:
-        raise ValueError(f"unknown init option {init_option!r}")
-    return u, alpha
-
-
 def init_BSSMF_md_sharded(init_option, X_local, d_local, R_local, n_u, seed=None, group=None, backend=None):
     """deconvolution.init_BSSMF_md over row-sharded data: every rank passes ITS rows of X, d_x and R_trunc (or a resident
     DeviceProblem of them) -> (u_local, alpha); alpha is the same on every rank and u_local holds this rank's rows of the
     single-process u."""
     set_seed(seed)
     si = _init_of(backend, X_local, d_local, R_local, group)
-    if init_option != "uniform_" and n_u > si.be.N:
-        init_option = "uniform_"
-    u, alpha = _draw_sharded(si, init_option, si.be.K, n_u)
-    if init_option == "SVD":
-        alpha = projection_simplex_sort_2d(alpha)
-    if alpha[-n_u:][0].all() == 0.0:                      # deconvolution.py:74-76
-        alpha[-n_u:][0] = 1e-10
-        alpha[:-n_u] = (1 - 1e-10) * alpha[:-n_u]
-    return u, alpha
+    return _initial_iterate("partial", init_option, si.M, si.be.N, si.be.K, n_u, rows=(si.lo, si.hi), wls=si.wls, nndsvd=si.nndsvd)
 
 
 def init_BSSMF_md_p_sharded(init_option, X_local, d_local, R_local, n_u, purity, seed=None, group=None, backend=None):
-    """deconvolution.init_BSSMF_md_p over row-sharded data -> (u_local, alpha)."""
+    """deconvolution.init_BSSMF_md_p over row-sharded data -> (u_local, alpha); rank 0 prints the fallback message."""
     set_seed(seed)
     si = _init_of(backend, X_local, d_local, R_local, group)
-    nb = si.be.N
-    if init_option != "uniform" and n_u > nb:
-        if not si._multi() or dist.get_rank(group) == 0:
-            print("The number of unknowns is greater than the number of samples, we'll go with a uniform initialisation. ")
-        init_option = "uniform"
-    if init_option != "uniform_" and n_u > nb:
-        init_option = "uniform_"
-    u, alpha = _draw_sharded(si, init_option, si.be.K, n_u)
-    if init_option == "SVD":                               # deconvolution.py:262
-        alpha = np.vstack((purity * projection_simplex_sort_2d(alpha[:-n_u]), projection_simplex_sort_2d(alpha[-n_u:])))
-    return u, alpha
+    say = print if not si._multi() or dist.get_rank(group) == 0 else _quiet
+    return _initial_iterate("purity", init_option, si.M, si.be.N, si.be.K, n_u, rows=(si.lo, si.hi), wls=si.wls, nndsvd=si.nndsvd,
+                            purity=purity, say=say)
 
 
 def unsupervised_init_sharded(init_option, X_local, d_local, n_u, seed=None, group=None, backend=None):
@@ -515,22 +473,4 @@ def unsupervised_init_sharded(init_option, X_local, d_local, n_u, seed=None, gro
     (u_local, alpha)."""
     set_seed(seed)
     si = _init_of(backend, X_local, d_local, None, group)
-    M, nb, lo, hi = si.M, si.be.N, si.lo, si.hi
-    if init_option != "uniform_" and n_u > nb:
-        init_option = "uniform_"
-    if init_option == "uniform_":
-        u = rd.uniform(size=(M, n_u))[lo:hi]
-        alpha = rd.dirichlet(np.ones(n_u), nb).T
-    elif init_option == "beta":
-        temp = np.ones((M, n_u))
-        u = rd.beta(temp * 0.5, temp * 0.5)[lo:hi]
-        alpha = rd.dirichlet(np.ones(n_u), nb).T
-    elif init_option == "SVD":
-        u, alpha = si.nndsvd(n_u)
-        u = u.clip(0, 1)
-        alpha = projection_simplex_sort_2d(alpha)
-    elif init_option == "uniform":
-        raise NameError("name 'R_trunc' is not defined")   # what the reference does (deconvolution.py:117, SURVEY Q8)
-    else:
-        raise NotImplementedError(f"init option {init_option!r} is not available on the B200 path")
-    return u, alpha
+    return _initial_iterate("free", init_option, si.M, si.be.N, 0, n_u, rows=(si.lo, si.hi), wls=si.wls, nndsvd=si.nndsvd)
