@@ -58,7 +58,8 @@ def build_parser():
     p.add_argument("--shard", choices=["fits", "rows"], default="fits",
                    help="(B200 path, under torchrun) how several GPUs are used: 'fits' runs independent fits per GPU (--ic, --confidence; "
                         "the main fit runs on every GPU), 'rows' shards the CpG rows of every fit over the GPUs (the main fit and --ic AIC / "
-                        "BIC; --confidence and --ic CCC / BCV stay fit-sharded)")
+                        "BIC / CCC / BCV with a reference matrix, a CCC member's restarts and a BCV member's folds as one batch; --confidence stays "
+                        "fit-sharded)")
     return p
 
 

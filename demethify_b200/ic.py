@@ -13,7 +13,7 @@ from .deconvolution import _initial_iterate, init_BSSMF_md, mdwbssmf_deconv, uns
 from .engine import DeviceProblem, FitBatch
 
 __all__ = ["compute_bic", "compute_aic", "compute_consensus_matrix", "compute_ccc", "run_deconvolution", "bicross_validation",
-           "evaluate_best_ic", "merge_sweep", "sweep_member_supported"]
+           "evaluate_best_ic", "merge_sweep", "sweep_member_supported", "consensus_runs_sharded", "bicross_validation_sharded"]
 
 
 def _world(group=None):
@@ -145,21 +145,128 @@ def sweep_member_supported(K, n_u):
     return n_u >= 0 and (K + (K & 1)) + (n_u + (n_u & 1)) <= 32
 
 
+def _sharded_initial_iterate(X_loc, D_loc, R_loc, M, K, N, lo, hi, n_u, init_option, seed, group, init_backend, rng=None):
+    """init_BSSMF_md on the rows [lo, hi) of an M x N problem whose rows are sharded over `group` -> (u_local, alpha).  `uniform_` /
+    `beta` draw from `rng`, by default RandomState(seed) (== the reference's set_seed(seed) + global stream: int -> init_genrand,
+    list -> init_by_array, Q1); `uniform` / `SVD` re-seed the global stream and all-reduce their row sums (sharded.ShardedInit) on
+    `init_backend(X_loc, D_loc, R_loc)`."""
+    from .sharded import GpuInitBackend, init_BSSMF_md_sharded
+    if init_option in ("uniform_", "beta"):
+        return _initial_iterate("partial", init_option, M, N, K, n_u, rows=(lo, hi), rng=np.random.RandomState(seed) if rng is None else rng)
+    if init_option in ("uniform", "SVD"):
+        return init_BSSMF_md_sharded(init_option, None, None, None, n_u, seed=seed, group=group,
+                                     backend=(init_backend or GpuInitBackend)(X_loc, D_loc, R_loc))
+    raise NotImplementedError("row-sharded sweeps: --init uniform_, beta, uniform or SVD")
+
+
+def _gpu_fit_backend(problems, n_u, U0s, A0s):
+    """The sharded fits of one member as one batch: `problems` holds one (X, d_x, R_trunc) of this rank's rows per fit, or one
+    that all fits share; X may be a resident DeviceProblem."""
+    from .sharded import GpuShardBackend
+    probs = [p[0] if isinstance(p[0], DeviceProblem) else DeviceProblem(*p) for p in problems]
+    return GpuShardBackend(probs, None, None, n_u, [np.asarray(u).reshape(-1, n_u) for u in U0s], [np.asarray(a) for a in A0s])
+
+
+def _sum_over_ranks(values, group):
+    """Sum of the float64 `values` over the ranks of `group` (one all-reduce) -> ndarray."""
+    import torch
+    t = torch.tensor(np.asarray(values, dtype=np.float64))
+    if _world(group)[1] > 1:
+        if dist.get_backend(group) == "nccl":
+            t = t.cuda()
+        dist.all_reduce(t, group=group)
+    return t.cpu().numpy()
+
+
 def _row_sharded_member(prob_local, lo, hi, M, K, N, n_u, init_option, seed, iter1, iter2, tol, group):
     """One sweep member with the CpG rows sharded over the ranks of `group` (BASELINE config 5): every rank draws the same
-    initial iterate from the same seed, keeps its rows of u and runs the row-sharded solver -> (u_local, alpha, cost).  The
-    `uniform` and `SVD` inits all-reduce their row sums (sharded.ShardedInit)."""
-    from .sharded import init_BSSMF_md_sharded, mdwbssmf_deconv_sharded
-    if init_option in ("uniform_", "beta"):
-        # RandomState(seed) == the reference's set_seed(seed) + global stream (int -> init_genrand, list -> init_by_array, Q1)
-        u0, a0 = _initial_iterate("partial", init_option, M, N, K, n_u, rows=(lo, hi), rng=np.random.RandomState(seed))
-    elif init_option in ("uniform", "SVD"):
-        u0, a0 = init_BSSMF_md_sharded(init_option, prob_local, None, None, n_u, seed=seed, group=group)
-    else:
-        raise NotImplementedError("row-sharded sweeps: --init uniform_, beta, uniform or SVD")
+    initial iterate from the same seed, keeps its rows of u and runs the row-sharded solver -> (u_local, alpha, cost)."""
+    from .sharded import mdwbssmf_deconv_sharded
+    u0, a0 = _sharded_initial_iterate(prob_local, None, None, M, K, N, lo, hi, n_u, init_option, seed, group, None)
     u_loc, alpha, _n, cost = mdwbssmf_deconv_sharded(u0, a0, prob_local, None, None, n_u, n_iter1=iter1, n_iter2=iter2, tol=tol,
                                                      group=group)
     return u_loc, alpha, cost
+
+
+def consensus_runs_sharded(X_loc, D_loc, R_loc, M, lo, hi, n_u, init_option, seeds, iter1, iter2, tol, group=None, init_backend=None,
+                           fit_backend=None):
+    """The restarts of a CCC member (ic.py:195-200) with the CpG rows [lo, hi) of this rank: one initial iterate per seed by the
+    rules of the row-sharded sweep, then all restarts as ONE row-sharded batch (one all-reduce per step covers every restart) ->
+    (alpha of every restart, u_local and alpha of the last restart).  `init_backend(X, d_x, R)` (sharded.GpuInitBackend) and
+    `fit_backend(problems, n_u, U0s, A0s)` (a GpuShardBackend batch) do this rank's arithmetic; X_loc may be a resident
+    DeviceProblem of the rows (then D_loc and R_loc are None)."""
+    from .sharded import fit_row_sharded
+    K, N = (X_loc.K, X_loc.N) if isinstance(X_loc, DeviceProblem) else (np.shape(R_loc)[1], np.shape(X_loc)[1])
+    inits = [_sharded_initial_iterate(X_loc, D_loc, R_loc, M, K, N, lo, hi, n_u, init_option, s, group, init_backend) for s in seeds]
+    fits = fit_row_sharded((fit_backend or _gpu_fit_backend)([(X_loc, D_loc, R_loc)], n_u, [i[0] for i in inits], [i[1] for i in inits]),
+                           iter1, iter2, tol, group)
+    return [f[1] for f in fits], fits[-1][0], fits[-1][1]
+
+
+def _state_key(state):
+    return (np.asarray(state[1], dtype=np.uint32).tobytes(), int(state[2]), int(state[3]), float(state[4]))
+
+
+def bicross_validation_sharded(X_loc, D_loc, R_loc, M, lo, hi, n_u, init_option, seed, n_folds, iter1, iter2, tol, fraction=0.3, group=None,
+                               init_backend=None, fit_backend=None, cost=None):
+    """bicross_validation (ic.py:58-89) with a reference matrix and the CpG rows [lo, hi) of an M x N problem on this rank ->
+    (total PRESS, u_local and alpha of the best fold, test error of every fold (None where the reference skips it)).
+
+    Every fold draws its mask from numpy's global stream and then re-seeds it in its init, so a fold's mask starts either where the
+    seeding put the stream (the first fold), or after the init's draws (every later fold), or 2 M N words after a skipped fold's
+    mask (a mask with no train or no test entry over all rows, :119-120).  The planner replays those stream positions: each rank
+    draws only its rows of each distinct mask (mt_jump.mask_rows), the train counts are all-reduced for the skip test, and a fold
+    whose start state was seen before repeats that fold.  Only the distinct folds are fitted - at most two when no fold is skipped
+    - as one row-sharded batch of masked problems, each from its own initial iterate.  The test error ||(X - R alpha) o test||^2
+    is summed over the ranks and divided by the global test count; errors add to the total in fold order, the best fold is the
+    first strict minimum, and the global stream is left where the reference leaves it.  `init_backend` and `fit_backend` as in
+    consensus_runs_sharded; `cost(X, R, alpha, W)` is cost_f_w on this rank's rows."""
+    from .deconvolution import set_seed
+    from .mt_jump import mask_rows
+    from .sharded import fit_row_sharded
+    if seed is None and _world(group)[1] > 1:
+        raise ValueError("row-sharded bicross-validation needs a seed: every rank draws its rows of the same fold masks")
+    K, N = np.shape(R_loc)[1], np.shape(X_loc)[1]
+    X_loc, D_loc, R_loc = (np.asarray(a, dtype=np.float64) for a in (X_loc, D_loc, R_loc))
+    set_seed(seed)
+    state, after_init = np.random.get_state(), None
+    masks, distinct, order = {}, [], []          # start state -> (train rows, global train count, state after the mask); fitted folds
+    for _ in range(n_folds):
+        key = _state_key(state)
+        if key not in masks:
+            train, end = mask_rows(state, M, N, lo, hi, fraction)
+            masks[key] = (train, _sum_over_ranks([train.sum()], group)[0], end)
+        train, n_train, end = masks[key]
+        if n_train == 0 or n_train == M * N:         # no train or no test entry: the reference skips the fold without re-seeding
+            order.append(None)
+            state = end
+            continue
+        hit = [i for i, d in enumerate(distinct) if d["key"] == key]
+        if not hit:
+            Xm, Dm = X_loc * train, D_loc * train
+            set_seed(seed)                            # the fold's init (:75) re-seeds the global stream and draws from it
+            u0, a0 = _sharded_initial_iterate(Xm, Dm, R_loc, M, K, N, lo, hi, n_u, init_option, seed, group, init_backend, rng=np.random)
+            after_init = np.random.get_state()
+            distinct.append(dict(key=key, test=~train, n_test=M * N - n_train, prob=(Xm, Dm, R_loc), u0=u0, a0=a0))
+            hit = [len(distinct) - 1]
+        order.append(hit[0])
+        state = after_init
+    np.random.set_state(state)
+    if not distinct:
+        return 0, None, None, order
+    fits = fit_row_sharded((fit_backend or _gpu_fit_backend)([d["prob"] for d in distinct], n_u, [d["u0"] for d in distinct],
+                                                             [d["a0"] for d in distinct]), iter1, iter2, tol, group)
+    cost = cost or cost_f_w
+    sse = _sum_over_ranks([cost(X_loc, np.hstack((R_loc, u.reshape(-1, n_u))), a, d["test"].astype(np.float64))
+                           for d, (u, a, _n, _c) in zip(distinct, fits)], group)
+    errors = [None if i is None else sse[i] / distinct[i]["n_test"] for i in order]
+    total_press, best, min_error = 0, None, float("inf")
+    for i, e in zip(order, errors):
+        if i is not None:
+            total_press += e
+            if e < min_error:
+                min_error, best = e, i
+    return total_press, fits[best][0], fits[best][1], errors
 
 
 def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, tol, n_restarts=5, n_u_values=None, shard="fits",
@@ -173,8 +280,9 @@ def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, t
 
     Under torch.distributed: shard="fits" (default) gives position p of the sweep to rank p mod world (every member re-seeds and
     is independent); shard="rows" runs EVERY member with the CpG rows sharded over the ranks (one all-reduce per outer
-    iteration, sharded.py) - the partitioning for matrices that are large per member (AIC / BIC; every init but ICA, and the
-    reference-based member n_u = 0)."""
+    iteration, sharded.py) - the partitioning for matrices that are large per member (every criterion with a reference matrix;
+    every init but ICA, and the reference-based member n_u = 0).  A CCC member's restarts and a BCV member's distinct folds are
+    then one row-sharded batch (consensus_runs_sharded, bicross_validation_sharded)."""
     n_u_values = range(1, 25 + 1) if n_u_values is None else n_u_values
     meth_f = np.asarray(meth_f)
     n_cpg, n_samples = meth_f.shape
@@ -195,8 +303,8 @@ def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, t
         raise ValueError("n_u = 0 (reference-based fit) is available for AIC / BIC with a reference matrix only")
     rank, world = _world(group)
     rows_mode = shard == "rows" and world > 1
-    if rows_mode and (ic not in ("AIC", "BIC") or ref is None):
-        raise NotImplementedError("row-sharded sweeps: AIC / BIC with a reference matrix")
+    if rows_mode and ref is None:
+        raise NotImplementedError("row-sharded sweeps need a reference matrix")
     if rows_mode:
         from .sharded import row_range
         lo, hi = row_range(n_cpg, rank, world)
@@ -229,7 +337,10 @@ def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, t
                 cost = cost_f_w(meth_f, np.asarray(ref), alpha, counts)
             ic_result = compute_bic(cost, 0, n_cpg, n_ct, n_samples) if ic == "BIC" else compute_aic(cost, 0, n_cpg, n_ct, n_samples)
         elif ic == "CCC":
-            if ref is not None:
+            if rows_mode:
+                alpha_runs, u, alpha = consensus_runs_sharded(prob, None, None, n_cpg, lo, hi, n_u, init_option,
+                                                              [seed + r for r in range(n_restarts)], iter1, iter2, tol, group)
+            elif ref is not None:
                 inits = [init_BSSMF_md(init_option, src, counts, ref, n_u, seed=seed + r) for r in range(n_restarts)]
                 fits = _batched_fits(prob, np.asarray(ref), n_u, [(i[0], i[2]) for i in inits], iter1, iter2, tol)
                 alpha_runs = [f[2] for f in fits]
@@ -240,6 +351,10 @@ def evaluate_best_ic(meth_f, ref, counts, init_option, ic, seed, iter1, iter2, t
                     u, alpha = unsupervised_deconv(src, n_u, counts, init_option, n_iter1=iter1, n_iter2=iter2, tol=tol, seed=seed + r)
                     alpha_runs.append(alpha)
             ic_result = -compute_ccc(alpha_runs)
+        elif ic == "BCV" and rows_mode:
+            ic_result, u, alpha, _errors = bicross_validation_sharded(meth_f[lo:hi], np.asarray(counts)[lo:hi], np.asarray(ref)[lo:hi],
+                                                                      n_cpg, lo, hi, n_u, init_option, seed, n_restarts, iter1, iter2, tol,
+                                                                      group=group)
         elif ic == "BCV":
             ic_result, u, alpha = bicross_validation(meth_f, n_u, counts, iter1, iter2, tol, fraction=0.3, n_folds=n_restarts, seed=seed,
                                                      ref=ref, init_option=init_option, base=prob)

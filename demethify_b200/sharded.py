@@ -25,11 +25,11 @@ from .deconvolution import _initial_iterate, _quiet, set_seed
 from .engine import DeviceProblem, FitBatch, _handle, _stream_ptr, to_device
 from .init_func import aligned_workspace, wls_desc
 
-__all__ = ["row_range", "GpuShardBackend", "RowShardedFit", "mdwbssmf_deconv_sharded", "last_info", "GpuInitBackend", "ShardedInit",
-           "wls_all_samples_sharded", "init_BSSMF_md_sharded", "init_BSSMF_md_p_sharded", "unsupervised_init_sharded"]
+__all__ = ["row_range", "GpuShardBackend", "RowShardedFit", "mdwbssmf_deconv_sharded", "fit_row_sharded", "last_info", "GpuInitBackend",
+           "ShardedInit", "wls_all_samples_sharded", "init_BSSMF_md_sharded", "init_BSSMF_md_p_sharded", "unsupervised_init_sharded"]
 
 _peer_cache = {}    # (group, world, device) -> (symmetric buffer, rendezvous handle, bytes): see enable_peer_exchange
-last_info = {}      # of the most recent mdwbssmf_deconv_sharded call: {"peer_exchange": bool, "peer_error": str | None, "collectives": int}
+last_info = {}      # of the most recent row-sharded fit (fit_row_sharded): {"peer_exchange": bool, "peer_error": str | None, "collectives": int}
 
 
 def row_range(M, rank, world):
@@ -40,11 +40,17 @@ def row_range(M, rank, world):
 
 
 class GpuShardBackend:
-    """This rank's rows on its GPU: a one-fit (or few-fit) FitBatch in sharded Gram-engine mode."""
+    """This rank's rows on its GPU: a FitBatch in sharded Gram-engine mode.  One fit, or several when U0_local and A0 are lists of
+    initial iterates (CCC restarts, BCV folds); X_local is then one problem all fits share, or a list of resident DeviceProblems,
+    one per fit.  Every fit has its own statistics block, all-reduced copy and peer slot, so one all-reduce per step covers all."""
 
     def __init__(self, X_local, D_local, Rk_local, n_u, U0_local, A0, mode=_lib.DMF_MODE_PARTIAL, purity=None, precision=None, engine=None):
-        self.prob = X_local if isinstance(X_local, DeviceProblem) else DeviceProblem(X_local, D_local, Rk_local, precision=precision)
-        self.batch = FitBatch(self.prob, n_u, [U0_local], [A0], mode=mode, purity=purity, engine=engine)
+        if isinstance(X_local, (list, tuple)):
+            self.prob = list(X_local)
+        else:
+            self.prob = X_local if isinstance(X_local, DeviceProblem) else DeviceProblem(X_local, D_local, Rk_local, precision=precision)
+        U0s, A0s = (list(U0_local), list(A0)) if isinstance(U0_local, (list, tuple)) else ([U0_local], [A0])
+        self.batch = FitBatch(self.prob, n_u, U0s, A0s, mode=mode, purity=purity, engine=engine)
         lib, b = _lib.lib(), self.batch
         _lib.check(lib.dmf_batch_set_sharded(b.b, 1, _stream_ptr()))
         # fused engine where the shape allows it: ONE pass and ONE all-reduce per outer iteration (RowShardedFit.outer)
@@ -154,7 +160,8 @@ class GpuShardBackend:
 
 
 class RowShardedFit:
-    """Outer loop of one row-sharded fit; `backend` does this rank's arithmetic, `group` is the torch.distributed group."""
+    """Outer loop of the row-sharded fits of `backend` (one or several: each stops at its own termination test, the loop when every
+    fit has); `backend` does this rank's arithmetic, `group` is the torch.distributed group."""
 
     def __init__(self, backend, group=None):
         self.be, self.group = backend, group
@@ -282,17 +289,26 @@ def mdwbssmf_deconv_sharded(u_local, alpha, X_local, d_local, R_local, n_u, n_it
     ITS rows of u, X, d_x, R_trunc (see `row_range`) and the full alpha; returns (u_local, alpha, n_outer, cost)."""
     mode = _lib.DMF_MODE_PURITY if purity is not None else (_lib.DMF_MODE_PARTIAL if R_local is not None else _lib.DMF_MODE_UNSUPERVISED)
     be = GpuShardBackend(X_local, d_local, R_local, n_u, np.asarray(u_local).reshape(-1, n_u), np.asarray(alpha), mode=mode, purity=purity)
+    (u, a, n_outer, cost), = fit_row_sharded(be, n_iter1, n_iter2, tol, group)
+    return u, a, n_outer, cost
+
+
+def fit_row_sharded(be, n_iter1, n_iter2, tol, group=None):
+    """Run every fit of the shard backend `be` to its own termination over `group`, then close the backend ->
+    [(u_local, alpha, n_outer, cost)] per fit.  A GPU backend all-reduces in-kernel over NVLink peer memory unless DMF_PEER_XCHG=0
+    (NCCL is the fall-back when symmetric memory is unavailable)."""
     import os
-    if os.environ.get("DMF_PEER_XCHG", "1") != "0":          # the in-kernel NVLink all-reduce is the default; NCCL when symmetric memory is unavailable
+    if isinstance(be, GpuShardBackend) and os.environ.get("DMF_PEER_XCHG", "1") != "0":
         be.enable_peer_exchange(group)
     fit = RowShardedFit(be, group)
     try:
-        (u, a, n_outer, cost), = fit.fit(n_iter1, n_iter2, tol)
+        return fit.fit(n_iter1, n_iter2, tol)
     finally:
-        last_info.update(peer_exchange=be.peer is not None, peer_error=getattr(be, "peer_error", None), collectives=fit.collectives)
-        torch.cuda.synchronize()
+        last_info.update(peer_exchange=getattr(be, "peer", None) is not None, peer_error=getattr(be, "peer_error", None),
+                         collectives=fit.collectives)
+        if isinstance(be, GpuShardBackend):
+            torch.cuda.synchronize()
         be.close()
-    return u, a, n_outer, cost
 
 
 # ---------------------------------------------------------------------------------------------------------------------------------

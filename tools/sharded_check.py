@@ -3,7 +3,9 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/sharded_check.py
 Every rank fits its row range over NCCL; rank 0 gathers u and compares alpha, u and the outer-iteration count with the
 CPU oracle on the full problem.  Then the `demethify` command runs its main fit with --shard rows for every init option (partial,
-purity, reference-free, n_u = 0) and rank 0 compares the CSV files with a one-GPU run of the same seed."""
+purity, reference-free, n_u = 0) and rank 0 compares the CSV files with a one-GPU run of the same seed.  Last, CCC and BCV
+sweeps run row-sharded (evaluate_best_ic(shard="rows"), what `--shard rows --ic` runs) and rank 0 compares the criteria, the selected
+n_u, alpha and u with the same sweep on one GPU."""
 import os
 import sys
 
@@ -57,6 +59,7 @@ def main():
             print(f"sharded_check world={world} peer_xchg={peer} graph={graph} it1={it1}: n_outer={n_outer} oracle={tr['n_outer']} max|d alpha|={da:.2e} max|d u|={du:.2e} "
                   f"alpha replicated={same_alpha} peer={sharded.last_info} -> {'OK' if good else 'FAIL'}", flush=True)
     ok &= cli_check(rank, world)
+    ok &= ic_check(rank, world)
     dist.destroy_process_group()
     sys.exit(0 if ok else 1)
 
@@ -107,6 +110,33 @@ def cli_check(rank, world):
             ok &= good
             print(f"sharded_check cli world={world} --init {init} {' '.join(extra[:3])}{' (reference-free)' if not ref else ''}: "
                   f"max|rows - one GPU|={dev:.2e} -> {'OK' if good else 'FAIL'}", flush=True)
+        dist.barrier()
+    box = [ok]
+    dist.broadcast_object_list(box, src=0)
+    return box[0]
+
+
+def ic_check(rank, world):
+    from demethify_b200.ic import evaluate_best_ic
+    rs = np.random.RandomState(9)
+    M, N, K = 30011, 12, 5
+    Rf = rs.beta(0.5, 0.5, size=(M, K + 2))
+    D = rs.poisson(40, size=(M, N)) + 1
+    X = rs.binomial(D, np.clip(Rf @ rs.dirichlet(np.ones(K + 2), N).T, 0, 1)) / D
+    one = dist.new_group([0])
+    ok = True
+    for crit, init, seed in (("CCC", "uniform_", 1), ("CCC", "SVD", 2), ("BCV", "uniform_", [3]), ("BCV", "uniform", 4), ("BCV", "SVD", 5)):
+        u, a, best, values = evaluate_best_ic(X, Rf[:, :K], D, init, crit, seed, 300, 20, 1e-2, n_restarts=3, n_u_values=[1, 2, 3],
+                                              shard="rows")
+        if rank == 0:
+            u1, a1, best1, values1 = evaluate_best_ic(X, Rf[:, :K], D, init, crit, seed, 300, 20, 1e-2, n_restarts=3, n_u_values=[1, 2, 3],
+                                                      shard="fits", group=one)
+            dv = np.abs(np.array(values) - np.array(values1)).max()
+            da, du = np.abs(a - a1).max(), np.abs(u - u1).max()
+            good = best == best1 and dv <= 1e-8 * max(1.0, np.abs(values1).max()) and da <= 1e-8 and du <= 1e-8
+            ok &= good
+            print(f"sharded_check ic world={world} {crit} --init {init} seed={seed}: best n_u {best} (one GPU {best1}) max|d criterion|={dv:.2e} "
+                  f"max|d alpha|={da:.2e} max|d u|={du:.2e} -> {'OK' if good else 'FAIL'}", flush=True)
         dist.barrier()
     box = [ok]
     dist.broadcast_object_list(box, src=0)
