@@ -283,4 +283,97 @@ __device__ __forceinline__ double extrap_beta(double a_prev, double a_next, doub
     return fmin((a_prev - 1.0) / a_next, 0.9999 * sqrt(l_old / l_new));
 }
 
+// ------------------------------------------------------------------------------------------------
+// The reference's outer-loop bookkeeping (deconvolution.py:192-221), written once for every engine.  Each function runs in the
+// one thread that owns the fit state; the outer-iteration counts of the parity tests depend on every operation and its order.
+// The set-up reads its partial record through a pointer and the close returns `done`: in those shapes ptxas allocates the
+// calling kernels exactly as it did for the inline copies these functions replace.
+
+// l_w / l_h (deconvolution.py:192-204, :212, :216): the Frobenius norm, squared, times max(d_x)^2
+__device__ __forceinline__ double lipschitz(double ssq, double dmax2) {
+    const double nrm = sqrt(ssq);
+    return (nrm * nrm) * dmax2;
+}
+// max d_x over the CTA partial records [cost, ssq_rk, ssq_u, dmax] (a max, not a sum: hier_reduce does not carry it)
+__device__ __forceinline__ double part_dmax(const Geom& g, const FitDev& f) {
+    double dm = 0.0;
+    for (int p = 0; p < g.n_parts; ++p) dm = fmax(dm, __ldcg(&f.part[(size_t)p * g.part_stride + 3]));
+    return dm;
+}
+// ||alpha[-n_u:]||_F^2 of the alpha slot A (deconvolution.py:198): tiny, done serially in row-major order
+template <typename T>
+__device__ __forceinline__ double alpha_unk_ssq(const Geom& g, const T* A) {
+    double sa = 0.0;
+    for (int q = 0; q < g.nu; ++q)
+        for (int j = 0; j < g.N; ++j) {
+            const double v = (double)A[(size_t)(g.K + q) * g.N + j];
+            sa = fma(v, v, sa);
+        }
+    return sa;
+}
+
+// set-up (deconvolution.py:192-204) from the record [cost, ||R_trunc||^2, ||u||^2] of the initial iterate, max d_x and its alpha slot A
+template <typename T>
+__device__ __forceinline__ void state_setup(FitState* st, const FitDev& f, const double* rec, double dmax, const Geom& g, const T* A) {
+    const double cf = rec[0];
+    st->dmax = dmax;
+    st->dmax2 = dmax * dmax;
+    st->ssq_rk = rec[1];
+    st->ssq_u = rec[2];
+    st->l_w = lipschitz(alpha_unk_ssq(g, A), st->dmax2);
+    st->l_w_old = st->l_w;
+    st->l_h = lipschitz(rec[1] + rec[2], st->dmax2);
+    st->l_h_old = st->l_h;
+    st->a1 = 1.0;
+    st->a2 = 1.0;
+    st->cf = cf;
+    st->cf_prev = cf;
+    st->n_outer = 0;
+    st->t_u = 0;
+    st->t_a = 0;
+    st->phase = 0;
+    if (f.trace && f.trace_cap > 0) f.trace[0] = cf;
+}
+
+// termination test (deconvolution.py:220), plus a NaN cost
+__device__ __forceinline__ bool outer_stops(double cf, double cf_prev, double tol) { return fabs(cf - cf_prev) < tol || !(cf == cf); }
+
+// close of an outer iteration (deconvolution.py:218-221) with the cost of the new iterate; a stop sets done = 1 (converged) or
+// 3 (NaN cost).  Returns whether the fit is done.
+__device__ __forceinline__ bool state_close_outer(FitState* st, const FitDev& f, double cf, double tol) {
+    const double prev = st->cf;
+    st->cf_prev = prev;
+    st->cf = cf;
+    const int n = st->n_outer + 1;
+    st->n_outer = n;
+    if (f.trace && n < f.trace_cap) f.trace[n] = cf;
+    st->phase = 0;                                  // the cost of the current iterate is known (dmf_fused.cuh)
+    if (outer_stops(cf, prev, tol)) st->done = (cf == cf) ? 1 : 3;
+    return st->done != 0;
+}
+
+// end of the U step (deconvolution.py:84-89): momentum a1 and inner-iteration index; l_w_ = l_w once a step ran
+__device__ __forceinline__ void state_end_u(FitState* st, double a1_next, int t_u_next, double l_w_stepped, bool stepped) {
+    st->a1 = a1_next;
+    st->t_u = t_u_next;
+    if (stepped) st->l_w_old = l_w_stepped;
+}
+// ||u||^2 after the U step and l_h = ||[R_trunc, u]||^2 dmax^2 (deconvolution.py:212, read by the alpha steps only)
+__device__ __forceinline__ void state_u_norm(FitState* st, double ssq_u) {
+    st->ssq_u = ssq_u;
+    st->l_h = lipschitz(st->ssq_rk + ssq_u, st->dmax2);
+}
+
+// end of the alpha step (deconvolution.py:96-101, :216 / :327): l_w from ||alpha[-n_u:]||^2; the projected-gradient step also
+// advances its momentum a2 and inner-iteration index, and l_h_ = l_h once a step ran (Frank-Wolfe has no momentum)
+__device__ __forceinline__ void state_end_alpha(FitState* st, double ssq_alpha_unk, bool projected_gradient, double a2_next,
+                                                int t_a_next, double l_h_stepped, bool stepped) {
+    st->l_w = lipschitz(ssq_alpha_unk, st->dmax2);
+    if (projected_gradient) {
+        st->a2 = a2_next;
+        st->t_a = t_a_next;
+        if (stepped) st->l_h_old = l_h_stepped;
+    }
+}
+
 }  // namespace dmf

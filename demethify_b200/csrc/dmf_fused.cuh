@@ -825,26 +825,13 @@ __global__ void __launch_bounds__((FusedCfg<S, NUB>::THREADS), 1) fused_outer_ke
             f.scal[0] = cf;
             f.scal[4] = su;
         } else {
-            if (st->phase == 1) {              // the incoming iterate closes an outer iteration: deconvolution.py:218-221
-                const double prev = st->cf;
-                st->cf_prev = prev;
-                st->cf = cf;
-                const int no = st->n_outer + 1;
-                st->n_outer = no;
-                if (f.trace && no < f.trace_cap) f.trace[no] = cf;
-                st->phase = 0;
-                if (fabs(cf - prev) < a.tol) { st->done = 1; commit = 0; }
-                if (!(cf == cf)) { st->done = 3; commit = 0; }
-            }
+            // a phase-1 iterate closes an outer iteration; a stop leaves the pass uncommitted
+            if (st->phase == 1 && state_close_outer(st, f, cf, a.tol)) commit = 0;
             if (commit) {
                 const int t0 = st->t_u, n2 = a.n_iter2;
                 st->u_cur = ucur ^ 2;
-                st->a1 = a.mom_a[t0 + n2];
-                st->t_u = t0 + n2;
-                if (n2 > 0) st->l_w_old = st->l_w;               // deconvolution.py:89
-                st->ssq_u = su;
-                const double nr = sqrt(st->ssq_rk + su);
-                st->l_h = (nr * nr) * st->dmax2;                 // deconvolution.py:212
+                state_end_u(st, a.mom_a[t0 + n2], t0 + n2, st->l_w, n2 > 0);
+                state_u_norm(st, su);
                 st->phase = 1;
             }
         }

@@ -43,56 +43,6 @@ __host__ __device__ constexpr int rowgram_min_blocks(int kb, int nub, int c, int
 __host__ __device__ constexpr int panel_min_blocks(int pa, int pb, int c) { return pa * (pb + 1) * c <= 40 ? 2 : 1; }
 
 // ------------------------------------------------------------------------------------------------
-// shared by cost_kernel-style epilogues: CTA partial [cost, ssq_rk, ssq_u, dmax] -> fit state
-__device__ __forceinline__ double scan_dmax(const Geom& g, const FitDev& f) {
-    double dm = 0.0;
-    for (int p = 0; p < g.n_parts; ++p) dm = fmax(dm, __ldcg(&f.part[(size_t)p * g.part_stride + 3]));
-    return dm;
-}
-template <bool INITIAL>
-__device__ __forceinline__ void cost_state_update(const Geom& g, const FitDev& f, FitState* st, const double* rec, const void* Acur_v,
-                                                  bool f32, double tol, double dm) {
-    const double cf = rec[0];
-    if (INITIAL) {
-        st->dmax = dm;
-        st->dmax2 = dm * dm;
-        st->ssq_rk = rec[1];
-        st->ssq_u = rec[2];
-        double sa = 0.0;                       // ||alpha[-n_u:]||_F^2, deconvolution.py:198
-        for (int q = 0; q < g.nu; ++q)
-            for (int j = 0; j < g.N; ++j) {
-                const size_t idx = (size_t)(g.K + q) * g.N + j;
-                const double v = f32 ? (double)reinterpret_cast<const float*>(Acur_v)[idx] : reinterpret_cast<const double*>(Acur_v)[idx];
-                sa = fma(v, v, sa);
-            }
-        const double na = sqrt(sa), nr = sqrt(rec[1] + rec[2]);
-        st->l_w = (na * na) * st->dmax2;
-        st->l_w_old = st->l_w;
-        st->l_h = (nr * nr) * st->dmax2;
-        st->l_h_old = st->l_h;
-        st->a1 = 1.0;
-        st->a2 = 1.0;
-        st->cf = cf;
-        st->cf_prev = cf;
-        st->n_outer = 0;
-        st->t_u = 0;
-        st->t_a = 0;
-        st->phase = 0;
-        if (f.trace && f.trace_cap > 0) f.trace[0] = cf;
-    } else {
-        const double prev = st->cf;
-        st->cf_prev = prev;
-        st->cf = cf;
-        st->phase = 0;                                 // the cost of the current iterate is known (dmf_fused.cuh)
-        const int n = st->n_outer + 1;
-        st->n_outer = n;
-        if (f.trace && n < f.trace_cap) f.trace[n] = cf;
-        if (fabs(cf - prev) < tol) st->done = 1;      // deconvolution.py:220
-        if (!(cf == cf)) st->done = 3;
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
 // rowgram pass.  Thread (row group gr, column thread tc) owns C adjacent columns and RPT rows of the tile; the per-row
 // values [b (NUB) | H upper triangle] are summed over the column threads of a warp with the transposed butterfly and
 // written per warp:  rowgram[row][warp-in-row][NG]  (u_inner_kernel adds the <= 8 per-warp partials in fixed order).
@@ -266,11 +216,13 @@ __global__ void __launch_bounds__(kThreads, rowgram_min_blocks(KB, NUB, C, RPT))
     }
     if (!hier_reduce(g, f, rec, 3, &c.ctl->flag)) return;
     if (threadIdx.x == 0) {
-        const double dm = INITIAL ? scan_dmax(g, f) : 0.0;
+        const double dm = INITIAL ? part_dmax(g, f) : 0.0;
         if (a.flags & kFlagPartial) {
             f.scal[0] = rec[0]; f.scal[1] = rec[1]; f.scal[2] = rec[2]; f.scal[3] = dm;
+        } else if (INITIAL) {
+            state_setup(st, f, rec, dm, g, Acur);
         } else {
-            cost_state_update<INITIAL>(g, f, st, rec, Acur, sizeof(T) == 4, a.tol, dm);
+            state_close_outer(st, f, rec[0], a.tol);
         }
     }
 }
@@ -604,11 +556,13 @@ __global__ void __launch_bounds__(kThreads, rowgram_min_blocks(KB, NUB, 4, RPT))
     }
     if (!hier_reduce(g, f, rec, 3, &c.ctl->flag)) return;
     if (threadIdx.x == 0) {
-        const double dm = INITIAL ? scan_dmax(g, f) : 0.0;
+        const double dm = INITIAL ? part_dmax(g, f) : 0.0;
         if ((a.flags & kFlagPartial) || multmode) {
             f.scal[0] = rec[0]; f.scal[1] = rec[1]; f.scal[2] = rec[2]; f.scal[3] = dm;
+        } else if (INITIAL) {
+            state_setup(st, f, rec, dm, g, Acur);
         } else {
-            cost_state_update<INITIAL>(g, f, st, rec, Acur, sizeof(T) == 4, a.tol, dm);
+            state_close_outer(st, f, rec[0], a.tol);
         }
     }
 }
@@ -690,16 +644,9 @@ __global__ void __launch_bounds__(kThreads) u_inner_kernel(const PassArgs a) {
     if (threadIdx.x == 0) f.part[(size_t)part_id(g) * g.part_stride] = s0;
     if (!hier_reduce(g, f, rec, 1, &flag)) return;
     if (threadIdx.x == 0) {
-        st->a1 = a.mom_a[t0 + n2];
-        st->t_u = t0 + n2;
-        if (n2 > 0) st->l_w_old = l_w;                       // deconvolution.py:89
-        if (a.flags & kFlagPartial) {
-            f.scal[4] = rec[0];                              // this GPU's rows; alpha_inner_kernel forms l_h from the all-reduced sum
-        } else {
-            st->ssq_u = rec[0];
-            const double nr = sqrt(st->ssq_rk + rec[0]);
-            st->l_h = (nr * nr) * st->dmax2;                 // deconvolution.py:212
-        }
+        state_end_u(st, a.mom_a[t0 + n2], t0 + n2, l_w, n2 > 0);
+        if (a.flags & kFlagPartial) f.scal[4] = rec[0];      // this GPU's rows; alpha_inner_kernel forms l_h from the all-reduced sum
+        else state_u_norm(st, rec[0]);
     }
 }
 
@@ -781,12 +728,8 @@ __global__ void __launch_bounds__(kThreads) u_inner_mult_kernel(const PassArgs a
     if (threadIdx.x == 0) f.part[(size_t)part_id(g) * g.part_stride] = s0;
     if (!hier_reduce(g, f, rec, 1, &flag)) return;
     if (threadIdx.x == 0) {
-        st->a1 = a.mom_a[t0 + n2];
-        st->t_u = t0 + n2;
-        if (n2 > 0) st->l_w_old = l_w;
-        st->ssq_u = rec[0];
-        const double nr = sqrt(st->ssq_rk + rec[0]);
-        st->l_h = (nr * nr) * st->dmax2;
+        state_end_u(st, a.mom_a[t0 + n2], t0 + n2, l_w, n2 > 0);
+        state_u_norm(st, rec[0]);
     }
 }
 
@@ -862,10 +805,10 @@ __global__ void __launch_bounds__(kThreads) cost_cross_kernel(const PassArgs a) 
     }
     if (!hier_reduce(g, f, rec, 2, &flag)) return;
     if (threadIdx.x == 0) {
-        double r4[4] = {f.scal[0] + rec[0], f.scal[1], rec[1], f.scal[3]};
-        const char* Acur = f.A + (size_t)acur * g.Kt * g.N * sizeof(T);
-        if (initial) cost_state_update<true>(g, f, st, r4, Acur, sizeof(T) == 4, a.tol, r4[3]);
-        else cost_state_update<false>(g, f, st, r4, Acur, sizeof(T) == 4, a.tol, 0.0);
+        const double r4[4] = {f.scal[0] + rec[0], f.scal[1], rec[1], f.scal[3]};
+        const T* Acur = reinterpret_cast<const T*>(f.A + (size_t)acur * g.Kt * g.N * sizeof(T));
+        if (initial) state_setup(st, f, r4, r4[3], g, Acur);
+        else state_close_outer(st, f, r4[0], a.tol);
     }
 }
 
@@ -1206,18 +1149,15 @@ __global__ void __launch_bounds__(32) alpha_inner_kernel(const PassArgs a) {
     const bool fw = (a.flags & kFlagFW) != 0;
     const int n2 = a.k_inner, Kt = g.Kt;
     const int acur = st->a_cur;
-    double l_h = st->l_h;
     const bool sharded = (a.flags & kFlagPartial) != 0;
-    if (sharded) {                                           // ||u||^2 summed over all GPUs -> l_h, deconvolution.py:212
-        const double nr = sqrt(st->ssq_rk + f.rscal[4]);
-        l_h = (nr * nr) * st->dmax2;
-    }
+    // row-sharded: ||u||^2 summed over all GPUs -> l_h, deconvolution.py:212
+    const double l_h = sharded ? lipschitz(st->ssq_rk + f.rscal[4], st->dmax2) : st->l_h;
     // Row-sharded fused engine: the fused pass published this GPU's cost / ||u||^2 / panel; on the all-reduced copies every CTA
     // takes the same termination decision (deconvolution.py:218-221), the last CTA commits it (dmf_fused.cuh, last-CTA logic)
     const bool fcommit = (a.flags & kFlagFusedCommit) != 0;
     const int phase_in = st->phase;
     const double cf_new = fcommit ? f.rscal[0] : 0.0;
-    const bool fstop = fcommit && phase_in == 1 && ((fabs(cf_new - st->cf) < a.tol) || !(cf_new == cf_new));
+    const bool fstop = fcommit && phase_in == 1 && outer_stops(cf_new, st->cf, a.tol);
     const double lw_pass = st->l_w;                      // the l_w the fused pass stepped with
     const int tu_in = st->t_u, ucur_in = st->u_cur;
     const double lho_in = st->l_h_old;
@@ -1302,35 +1242,18 @@ __global__ void __launch_bounds__(32) alpha_inner_kernel(const PassArgs a) {
         f.tickets[0] = 0u;                               // re-arm for the next launch
         if (fcommit) {
             if (phase_in == 1) {                         // the incoming iterate closes an outer iteration
-                const double prev = st->cf;
-                st->cf_prev = prev;
-                st->cf = cf_new;
-                const int no = st->n_outer + 1;
-                st->n_outer = no;
-                if (f.trace && no < f.trace_cap) f.trace[no] = cf_new;
-                st->phase = 0;
-                if (fstop) { st->done = (cf_new == cf_new) ? 1 : 3; return; }
+                state_close_outer(st, f, cf_new, a.tol);
+                if (fstop) return;                       // the same test as state_close_outer's, taken by every CTA above
             }
             st->u_cur = ucur_in ^ 2;                     // commit the U step of the fused pass
-            st->a1 = a.mom_a[tu_in + n2];
-            st->t_u = tu_in + n2;
-            if (n2 > 0) st->l_w_old = lw_pass;
+            state_end_u(st, a.mom_a[tu_in + n2], tu_in + n2, lw_pass, n2 > 0);
             st->phase = 1;
         }
         if (bad) st->done = 3;
-        if (sharded) {
-            st->ssq_u = f.rscal[4];
-            st->l_h = l_h;
-        }
+        if (sharded) state_u_norm(st, f.rscal[4]);
         double sa = 0.0;
         for (int t = 0; t < g.N; ++t) sa += s_part[t];
-        const double na = sqrt(sa);
-        st->l_w = (na * na) * st->dmax2;                 // deconvolution.py:216 / :327
-        if (!fw) {
-            st->a2 = a.mom_a[t0 + n2];
-            st->t_a = t0 + n2;
-            if (n2 > 0) st->l_h_old = l_h;               // deconvolution.py:101
-        }
+        state_end_alpha(st, sa, !fw, a.mom_a[t0 + n2], t0 + n2, l_h, n2 > 0);
     }
 }
 
@@ -1344,10 +1267,13 @@ static __global__ void finalize_cost_kernel(const PassArgs a) {
     const FitDev f = a.fits[i];
     FitState* st = f.st;
     if (st->done) return;
-    const bool f32 = (a.flags & kFlagF32) != 0;
-    const char* Acur = f.A + (size_t)st->a_cur * a.g.Kt * a.g.N * (f32 ? 4 : 8);
-    if (a.flags & kFlagInitial) cost_state_update<true>(a.g, f, st, f.rscal, Acur, f32, a.tol, f.rscal[3]);
-    else cost_state_update<false>(a.g, f, st, f.rscal, Acur, f32, a.tol, 0.0);
+    if (a.flags & kFlagInitial) {
+        const size_t slot = (size_t)st->a_cur * a.g.Kt * a.g.N;
+        if (a.flags & kFlagF32) state_setup(st, f, f.rscal, f.rscal[3], a.g, reinterpret_cast<const float*>(f.A) + slot);
+        else state_setup(st, f, f.rscal, f.rscal[3], a.g, reinterpret_cast<const double*>(f.A) + slot);
+    } else {
+        state_close_outer(st, f, f.rscal[0], a.tol);
+    }
 }
 
 // ------------------------------------------------------------------------------------------------

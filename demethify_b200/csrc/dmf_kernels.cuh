@@ -323,44 +323,8 @@ __global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) cost_kernel(co
     // dmax needs a max, not a sum: it travels through slot 3 of every record and is re-derived below.
     if (!hier_reduce(g, f, rec, 3, &c.ctl->flag)) return;
     if (threadIdx.x == 0) {
-        const double cf = rec[0];
-        if (INITIAL) {
-            double dm = 0.0;
-            for (int p = 0; p < g.n_parts; ++p) dm = fmax(dm, __ldcg(&f.part[(size_t)p * g.part_stride + 3]));
-            st->dmax = dm;
-            st->dmax2 = dm * dm;
-            st->ssq_rk = rec[1];
-            st->ssq_u = rec[2];
-            // ||alpha[-n_u:]||_F^2 (deconvolution.py:198): tiny, done serially in row-major order
-            double sa = 0.0;
-            for (int q = 0; q < g.nu; ++q)
-                for (int j = 0; j < g.N; ++j) {
-                    const double v = (double)Acur[(size_t)(g.K + q) * g.N + j];
-                    sa = fma(v, v, sa);
-                }
-            const double na = sqrt(sa), nr = sqrt(rec[1] + rec[2]);
-            st->l_w = (na * na) * st->dmax2;
-            st->l_w_old = st->l_w;
-            st->l_h = (nr * nr) * st->dmax2;
-            st->l_h_old = st->l_h;
-            st->a1 = 1.0;
-            st->a2 = 1.0;
-            st->cf = cf;
-            st->cf_prev = cf;
-            st->n_outer = 0;
-            st->t_u = 0;
-            st->t_a = 0;
-            if (f.trace && f.trace_cap > 0) f.trace[0] = cf;
-        } else {
-            const double prev = st->cf;
-            st->cf_prev = prev;
-            st->cf = cf;
-            const int n = st->n_outer + 1;
-            st->n_outer = n;
-            if (f.trace && n < f.trace_cap) f.trace[n] = cf;
-            if (fabs(cf - prev) < a.tol) st->done = 1;      // deconvolution.py:220
-            if (!(cf == cf)) st->done = 3;                    // NaN guard
-        }
+        if (INITIAL) state_setup(st, f, rec, part_dmax(g, f), g, Acur);
+        else state_close_outer(st, f, rec[0], a.tol);
     }
 }
 
@@ -588,13 +552,9 @@ __global__ void __launch_bounds__(kThreads, u_pass_min_blocks(KB, NUB, C)) u_pas
     }
     if (!hier_reduce(g, f, rec, 1, &c.ctl->flag)) return;
     if (threadIdx.x == 0) {
-        st->a1 = a_next;
-        st->t_u += 1;
-        st->l_w_old = l_w;                                   // deconvolution.py:89
+        state_end_u(st, a_next, st->t_u + 1, l_w, true);
+        state_u_norm(st, rec[0]);
         st->u_cur = ucur ^ 1;
-        st->ssq_u = rec[0];
-        const double nr = sqrt(st->ssq_rk + rec[0]);
-        st->l_h = (nr * nr) * st->dmax2;                     // deconvolution.py:212 (read by the alpha steps only)
     }
 }
 
@@ -794,14 +754,8 @@ __global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) alpha_pass_ker
     if (threadIdx.x == 0) {
         double sa = 0.0;
         for (int j = 0; j < g.N; ++j) sa += colred[j];
-        const double na = sqrt(sa);
-        st->l_w = (na * na) * st->dmax2;                 // deconvolution.py:216 / :327 (read by the U steps only)
-        if (!fw) {
-            st->a2 = a_next;
-            st->t_a += 1;
-            st->l_h_old = l_h;                           // deconvolution.py:101
-            st->a_cur = acur ^ 1;
-        }
+        state_end_alpha(st, sa, !fw, a_next, st->t_a + 1, l_h, true);
+        if (!fw) st->a_cur = acur ^ 1;
     }
 }
 
