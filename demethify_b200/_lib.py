@@ -74,6 +74,8 @@ EXPORTS = {
     "dmf_batch_set_sharded": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "dmf_batch_stats_buffers": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "dmf_gram_finalize_cost": (C.c_int, [C.c_void_p, C.c_int32, C.c_double, C.c_void_p]),
+    "dmf_pass_u_commit": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "dmf_pass_alpha_commit": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "dmf_batch_peer_bytes": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_size_t)]),
     "dmf_batch_set_peers": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p]),
     "dmf_gram_exchange": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),

@@ -122,6 +122,7 @@ struct Plan {
     size_t off_usum, per_fit_usum;
     size_t off_rowgram, off_stats, off_gstats, off_red, per_fit_rowgram, per_fit_stats, per_fit_red;
     size_t stats_gbx, stats_scal;      // offsets (in doubles) of gbx and scal inside a per-fit stats block [gram | gbx | scal(8)]
+                                       // (shapes without the Gram form: [alpha gradient | scal(8)] of the row-sharded stream engine)
 };
 
 int make_plan(const dmf_handle_s* h, const dmf_shape_t& s, Plan& p) {
@@ -285,6 +286,11 @@ int make_plan(const dmf_handle_s* h, const dmf_shape_t& s, Plan& p) {
             }
         }
     }
+    // ---- row-sharded stream engine (shapes without the Gram form): per-fit statistics block [alpha gradient (Kt*N) | scal (8)]
+    if (!p.gram_ok) {
+        p.stats_scal = (size_t)Kt * s.N;
+        p.per_fit_stats = align_up((p.stats_scal + 8) * 8, 256);
+    }
     // ---- fused engine (dmf_fused.cuh): FP64, n_u <= 2, K <= 8, N <= 256, four U slots, rows that bulk copies can place one by one
     if (p.gram_ok && s.dtype == DMF_F64 && s.n_u <= 2 && s.K <= 8 && s.N <= 256 && s.u_slots >= 4 && (s.ldd * sW) % 16 == 0) {
         p.kb_f = s.K == 0 ? 0 : (s.K <= 4 ? 4 : (s.K <= 6 ? 6 : 8));
@@ -427,13 +433,16 @@ int set_smem(kern_t k, unsigned bytes) {
 int launch(dmf_batch_s* b, kern_t k, int ntc, unsigned smem, int flags, int k_inner, double tol, cudaStream_t st) {
     if (!k) return fail(DMF_E_SHAPE, "no kernel instantiation for this shape");
     if (b->multmode) return fail(DMF_E_STATE, "fits in multiplicity form run on the Gram-form engine only (dmf_gram_*)");
+    // a row-sharded pass only publishes its sums: the stream engine's commits are what advance the state
+    if (b->sharded && b->engine != DMF_ENGINE_STREAM)
+        return fail(DMF_E_STATE, "this row-sharded batch runs the fused or Gram-form engine (dmf_fused_* / dmf_gram_*), not the stream passes");
     PassArgs a;
     a.g = b->p.g;
     a.g.ntc = ntc;
     a.g.rg = kConsumers / ntc;
     a.fits = b->fits_dev;
     a.k_inner = k_inner;
-    a.flags = flags;
+    a.flags = flags | (b->sharded ? kFlagPartial : 0);
     a.tol = tol;
     a.ca0 = a.cb0 = a.with_x = a.pad = 0;
     a.mom_a = b->mom_dev; a.mom_m = b->mom_dev ? b->mom_dev + b->mom_cap : nullptr;
@@ -596,7 +605,7 @@ int dmf_batch_create(dmf_handle_t h, const dmf_shape_t* shape, const dmf_fit_des
     const dmf_shape_t& s = *shape;
     std::vector<FitDev> host(s.n_fits);
     char* base = static_cast<char*>(ws);
-    if (p.gram_ok && cudaMemsetAsync(base + p.off_stats, 0, 2 * p.per_fit_stats * s.n_fits, (cudaStream_t)stream) != cudaSuccess)
+    if (cudaMemsetAsync(base + p.off_stats, 0, 2 * p.per_fit_stats * s.n_fits, (cudaStream_t)stream) != cudaSuccess)
         return fail(DMF_E_CUDA, "batch set-up: clearing the statistics buffers failed");
     bool gather = false;
     int n_mult = 0;
@@ -630,9 +639,9 @@ int dmf_batch_create(dmf_handle_t h, const dmf_shape_t* shape, const dmf_fit_des
         f.tickets = reinterpret_cast<unsigned*>(base + p.off_tickets + p.per_fit_tickets * i);
         f.st = reinterpret_cast<FitState*>(base + p.off_states) + i;
         f.rowgram = p.gram_ok ? reinterpret_cast<double*>(base + p.off_rowgram + p.per_fit_rowgram * i) : nullptr;
-        f.gram = p.gram_ok ? reinterpret_cast<double*>(base + p.off_stats + p.per_fit_stats * i) : nullptr;
+        f.gram = reinterpret_cast<double*>(base + p.off_stats + p.per_fit_stats * i);
         f.gbx = p.gram_ok ? f.gram + p.stats_gbx : nullptr;
-        f.scal = p.gram_ok ? f.gram + p.stats_scal : nullptr;
+        f.scal = f.gram + p.stats_scal;
         f.rgram = f.gram; f.rgbx = f.gbx; f.rscal = f.scal;
         f.red = p.gram_ok ? reinterpret_cast<double*>(base + p.off_red + p.per_fit_red * i) : nullptr;
         f.mult = d.mult; f.offs = d.offs;
@@ -656,8 +665,8 @@ int dmf_batch_create(dmf_handle_t h, const dmf_shape_t* shape, const dmf_fit_des
     b->peers_dev = nullptr; b->xchg_ticket = nullptr; b->peer_rank = 0; b->peer_world = 0; b->xchg_epoch = 0;
     b->n_active = s.n_fits;
     b->fits_host = host;
-    b->stats_local = p.gram_ok ? reinterpret_cast<double*>(base + p.off_stats) : nullptr;
-    b->stats_global = p.gram_ok ? reinterpret_cast<double*>(base + p.off_gstats) : nullptr;
+    b->stats_local = reinterpret_cast<double*>(base + p.off_stats);
+    b->stats_global = reinterpret_cast<double*>(base + p.off_gstats);
     b->fits_dev = reinterpret_cast<FitDev*>(base + p.off_fits);
     b->states_dev = reinterpret_cast<FitState*>(base + p.off_states);
     b->fused_pending = 0;
@@ -850,35 +859,33 @@ int dmf_gram_alpha_inner(dmf_batch_t b, int32_t n_iter2, void* stream) {
 }
 int dmf_batch_set_sharded(dmf_batch_t b, int32_t on, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "row sharding needs the Gram-form engine (n_u <= 4, or n_u <= 8 with K <= 6)");
     if (b->multmode) return fail(DMF_E_STATE, "row sharding and the multiplicity form are not combined");
     cudaStream_t st = (cudaStream_t)stream;
     const size_t per = b->p.per_fit_stats / 8;
     for (int i = 0; i < b->shape.n_fits; ++i) {
         FitDev& f = b->fits_host[i];
         double* src = on ? b->stats_global + per * i : b->stats_local + per * i;
-        f.rgram = src; f.rgbx = src + b->p.stats_gbx; f.rscal = src + b->p.stats_scal;
+        f.rgram = src; f.rgbx = b->p.gram_ok ? src + b->p.stats_gbx : nullptr; f.rscal = src + b->p.stats_scal;
     }
     int rc = upload_fits(b, nullptr, st);
     if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(st));
     b->sharded = on ? 1 : 0;
-    b->engine = b->p.fused_ok ? DMF_ENGINE_FUSED : DMF_ENGINE_GRAM;
+    b->engine = b->p.fused_ok ? DMF_ENGINE_FUSED : (b->p.gram_ok ? DMF_ENGINE_GRAM : DMF_ENGINE_STREAM);
     return DMF_OK;
 }
 int dmf_batch_stats_buffers(dmf_batch_t b, void** local_dev, void** global_dev, int64_t* doubles_per_fit, int64_t* scal_offset) {
     if (!b || !local_dev || !global_dev || !doubles_per_fit || !scal_offset) return fail(DMF_E_ARG, "NULL argument");
-    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
     *local_dev = b->stats_local; *global_dev = b->stats_global;
     *doubles_per_fit = (int64_t)(b->p.per_fit_stats / 8); *scal_offset = (int64_t)b->p.stats_scal;
     return DMF_OK;
 }
 int dmf_gram_finalize_cost(dmf_batch_t b, int32_t initial, double tol, void* stream) {
     if (!b) return fail(DMF_E_ARG, "NULL batch");
-    if (!b->sharded) return fail(DMF_E_STATE, "dmf_gram_finalize_cost is the second half of dmf_gram_rowgram on row-sharded batches");
+    if (!b->sharded) return fail(DMF_E_STATE, "dmf_gram_finalize_cost is the second half of dmf_gram_rowgram / dmf_pass_init / dmf_pass_cost on row-sharded batches");
     PassArgs a;
     memset(&a, 0, sizeof(a));
-    a.g = b->p.gg;
+    a.g = b->p.g;       // the shape fields the set-up reads (N, K, n_u, Kt) are those of every engine's geometry
     a.fits = b->fits_dev;
     a.k_inner = b->n_active;
     a.flags = (initial ? kFlagInitial : 0) | (b->shape.dtype == DMF_F32 ? kFlagF32 : 0);
@@ -888,10 +895,38 @@ int dmf_gram_finalize_cost(dmf_batch_t b, int32_t initial, double tol, void* str
     b->launches++;
     return DMF_OK;
 }
+int dmf_pass_u_commit(dmf_batch_t b, void* stream) {
+    if (!b) return fail(DMF_E_ARG, "NULL batch");
+    if (!b->sharded || b->engine != DMF_ENGINE_STREAM)
+        return fail(DMF_E_STATE, "dmf_pass_u_commit ends the U step of a row-sharded stream-engine batch (after the scalar all-reduce)");
+    PassArgs a;
+    memset(&a, 0, sizeof(a));
+    a.g = b->p.g;
+    a.fits = b->fits_dev;
+    a.k_inner = b->n_active;
+    u_commit_kernel<<<(b->n_active + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    b->launches++;
+    return DMF_OK;
+}
+int dmf_pass_alpha_commit(dmf_batch_t b, int32_t k_inner, void* stream) {
+    if (!b) return fail(DMF_E_ARG, "NULL batch");
+    if (!b->sharded || b->engine != DMF_ENGINE_STREAM)
+        return fail(DMF_E_STATE, "dmf_pass_alpha_commit follows dmf_pass_alpha / dmf_pass_fw on a row-sharded stream-engine batch (after the all-reduce)");
+    PassArgs a;
+    memset(&a, 0, sizeof(a));
+    a.g = b->p.g;
+    a.fits = b->fits_dev;
+    a.k_inner = k_inner;
+    a.flags = (b->shape.mode == DMF_MODE_PURITY ? kFlagFW : 0) | (b->shape.dtype == DMF_F32 ? kFlagF32 : 0);
+    alpha_commit_kernel<<<b->n_active, kThreads, 0, (cudaStream_t)stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    b->launches++;
+    return DMF_OK;
+}
 
 int dmf_batch_peer_bytes(dmf_batch_t b, int32_t world, size_t* bytes) {
     if (!b || !bytes || world < 1) return fail(DMF_E_ARG, "bad argument");
-    if (!b->p.gram_ok) return fail(DMF_E_SHAPE, "no Gram-engine instantiation for this shape");
     const size_t slot = b->p.per_fit_stats / 8 * b->shape.n_fits;
     *bytes = align_up(2 * (size_t)world * slot * 8, 256) + align_up(2 * (size_t)world * 4, 256);
     return DMF_OK;
@@ -1003,6 +1038,9 @@ int dmf_fused_finish(dmf_batch_t b, double tol, void* stream) {
     return dmf_gram_rowgram(b, 0, tol, stream);          // cost-only use of the rowgram pass: counts the outer iteration, runs the test
 }
 
+static const char* const row_sharded_stream_msg =
+    "row-sharded stream batches run step by step: passes, all-reduce of the statistics blocks, dmf_pass_u_commit / dmf_pass_alpha_commit / "
+    "dmf_gram_finalize_cost";
 // engine actually used for a call with n_iter2 inner iterations
 static int effective_engine(const dmf_batch_s* b, int n_iter2) {
     if (b->engine == DMF_ENGINE_FUSED && (n_iter2 < 1 || n_iter2 > kFusedMaxInner || b->sharded || b->multmode)) return DMF_ENGINE_GRAM;      // (sharded fits are driven step by step by the caller)
@@ -1019,6 +1057,7 @@ int dmf_enqueue_outer(dmf_batch_t b, int32_t n_outer, int32_t n_iter2, double to
         return DMF_OK;
     }
     if (b->fused_pending && (rc = dmf_fused_finish(b, tol, stream))) return rc;
+    if (eng == DMF_ENGINE_STREAM && b->sharded) return fail(DMF_E_STATE, row_sharded_stream_msg);
     if (eng == DMF_ENGINE_GRAM) {
         for (int o = 0; o < n_outer; ++o)
             if ((rc = dmf_gram_outer(b, n_iter2, tol, stream))) return rc;
@@ -1054,6 +1093,7 @@ int dmf_fit_batched(dmf_batch_t b, int32_t n_iter1, int32_t n_iter2, double tol,
     if (n_iter1 < 0 || n_iter2 < 0) return fail(DMF_E_ARG, "negative iteration count");
     cudaStream_t st = (cudaStream_t)stream;
     const int eng = effective_engine(b, n_iter2);
+    if (eng == DMF_ENGINE_STREAM && b->sharded) return fail(DMF_E_STATE, row_sharded_stream_msg);
     b->fused_pending = 0;
     int rc = eng != DMF_ENGINE_STREAM ? dmf_gram_init(b, stream) : dmf_pass_init(b, stream);
     if (rc) return rc;

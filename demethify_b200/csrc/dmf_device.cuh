@@ -45,7 +45,8 @@ struct FitDev {
     unsigned* tickets;   // [n_groups + 1]
     FitState* st;
     double* rowgram;     // Gram engine: [M][warps per row][NG] per-row statistics of the U step
-    double* gram;        // Gram engine: [Kt][Kt][N] per-sample G_j = R^T diag(d_.j) R      (written by gram_panel_kernel: this GPU's rows)
+    double* gram;        // Gram engine: [Kt][Kt][N] per-sample G_j = R^T diag(d_.j) R      (written by gram_panel_kernel: this GPU's rows);
+                         // stream engine, row-sharded: [Kt][N] this GPU's alpha gradient (alpha_pass_kernel)
     double* gbx;         // Gram engine: [Kt][N]     per-sample R^T (d_.j o x_.j)
     double* scal;        // Gram engine: [8] row-sharded runs: this GPU's [cost, ||R_trunc||^2, ||u||^2 (set-up), max d, ||u||^2 (U step)]
     double* rgram;       // what alpha_inner_kernel / finalize_cost_kernel READ: == gram / gbx / scal on one GPU, the all-reduced
@@ -105,9 +106,10 @@ struct PassArgs {
 };
 constexpr int kFlagInitial = 1;   // init_cost_kernel: set-up pass (norms, max d, no termination test)
 constexpr int kFlagFW = 2;        // alpha_pass_kernel: Frank-Wolfe step instead of projected gradient
-constexpr int kFlagPartial = 4;   // Gram engine, CpG rows sharded over GPUs: publish this GPU's sums to FitDev::scal, leave the state to
-                                  // finalize_cost_kernel / alpha_inner_kernel, which run on the all-reduced sums
-constexpr int kFlagF32 = 8;       // finalize_cost_kernel: alpha is stored as float
+constexpr int kFlagPartial = 4;   // CpG rows sharded over GPUs: publish this GPU's sums to FitDev::scal (and gram), leave the state to
+                                  // finalize_cost_kernel / alpha_inner_kernel (Gram engine) or u_commit_kernel / alpha_commit_kernel
+                                  // (stream engine), which run on the all-reduced sums
+constexpr int kFlagF32 = 8;       // finalize_cost_kernel, alpha_commit_kernel: alpha is stored as float
 constexpr int kFlagFusedCommit = 16;   // alpha_inner_kernel after a kFlagPartial fused pass (row-sharded): run the termination test and commit
                                        // the U step on the all-reduced sums (what the fused pass's last CTA does on one GPU)
 

@@ -1276,6 +1276,26 @@ static __global__ void finalize_cost_kernel(const PassArgs a) {
     }
 }
 
+// CpG rows sharded over GPUs, stream engine: the end of a U step on the all-reduced ||u||^2 (FitDev::rscal[4]).  One thread per fit.
+static __global__ void u_commit_kernel(const PassArgs a) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.k_inner) return;
+    const FitDev f = a.fits[i];
+    if (f.st->done) return;
+    state_u_norm(f.st, f.rscal[4]);
+}
+
+// CpG rows sharded over GPUs, stream engine: the step of alpha_pass_kernel on the all-reduced gradient (the first Kt*N doubles of
+// FitDev::rgram).  One CTA per fit.
+static __global__ void __launch_bounds__(kThreads) alpha_commit_kernel(const PassArgs a) {
+    __shared__ double colred[kMaxSamples];
+    const FitDev f = a.fits[blockIdx.x];
+    if (f.st->done) return;
+    const bool fw = (a.flags & kFlagFW) != 0;
+    if (a.flags & kFlagF32) alpha_step<float>(a.g, f, f.rgram, colred, fw, a.k_inner);
+    else alpha_step<double>(a.g, f, f.rgram, colred, fw, a.k_inner);
+}
+
 // ------------------------------------------------------------------------------------------------
 // CpG rows sharded over GPUs: all-reduce of the statistics block over NVLink PEER MEMORY, in one kernel and without NCCL.
 // Every rank owns a symmetric buffer  data[2 parities][world slots][n] + flags[2][world]  that all ranks of the box can address

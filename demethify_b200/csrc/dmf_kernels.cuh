@@ -15,6 +15,9 @@
 // stay in registers across the whole CTA lifetime; cross-CTA sums go through the deterministic two-level
 // reduction of dmf_device.cuh and the LAST CTA applies the step (clip / simplex projection / Frank-Wolfe
 // vertex), updates the fit state and re-arms the tickets.
+// CpG rows sharded over GPUs (kFlagPartial): the last CTA publishes this GPU's reduced record in the fit's `local` statistics
+// block [alpha gradient (Kt*N) | scal (8)] instead; the state is then advanced on the all-reduced block by finalize_cost_kernel,
+// u_commit_kernel and alpha_commit_kernel (dmf_gram.cuh).
 #pragma once
 #include "dmf_device.cuh"
 
@@ -323,8 +326,16 @@ __global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) cost_kernel(co
     // dmax needs a max, not a sum: it travels through slot 3 of every record and is re-derived below.
     if (!hier_reduce(g, f, rec, 3, &c.ctl->flag)) return;
     if (threadIdx.x == 0) {
-        if (INITIAL) state_setup(st, f, rec, part_dmax(g, f), g, Acur);
-        else state_close_outer(st, f, rec[0], a.tol);
+        if (a.flags & kFlagPartial) {
+            // CpG rows sharded over GPUs: publish this GPU's sums; finalize_cost_kernel runs the set-up / test on the reduced ones.
+            // scal[4] starts at ||u||^2 so that u_commit_kernel after an outer iteration without U steps keeps the set-up's l_h.
+            f.scal[0] = rec[0];
+            if (INITIAL) { f.scal[1] = rec[1]; f.scal[2] = rec[2]; f.scal[3] = part_dmax(g, f); f.scal[4] = rec[2]; }
+        } else if (INITIAL) {
+            state_setup(st, f, rec, part_dmax(g, f), g, Acur);
+        } else {
+            state_close_outer(st, f, rec[0], a.tol);
+        }
     }
 }
 
@@ -553,7 +564,8 @@ __global__ void __launch_bounds__(kThreads, u_pass_min_blocks(KB, NUB, C)) u_pas
     if (!hier_reduce(g, f, rec, 1, &c.ctl->flag)) return;
     if (threadIdx.x == 0) {
         state_end_u(st, a_next, st->t_u + 1, l_w, true);
-        state_u_norm(st, rec[0]);
+        if (a.flags & kFlagPartial) f.scal[4] = rec[0];     // this GPU's rows; u_commit_kernel forms l_h from the all-reduced sum
+        else state_u_norm(st, rec[0]);
         st->u_cur = ucur ^ 1;
     }
 }
@@ -581,7 +593,66 @@ __device__ __forceinline__ bool project_simplex(double* v, int p) {
     return true;
 }
 
-// alpha pass: G = R^T (d o (x - R a_eval)); last CTA applies the projected-gradient or Frank-Wolfe step
+// The step of one alpha iteration on the Kt x N gradient G = R^T (d o (x - R a_eval)): projected gradient (deconvolution.py:94-101)
+// or Frank-Wolfe (:285-299), then the state update.  Run by all threads of ONE CTA of the fit: the last CTA of alpha_pass_kernel
+// (gradient in shared memory) or alpha_commit_kernel (row-sharded: the all-reduced gradient).  colred: N doubles of shared memory.
+template <typename T>
+__device__ __forceinline__ void alpha_step(const Geom& g, const FitDev& f, const double* grad, double* colred, bool fw, int k_inner) {
+    FitState* st = f.st;
+    const int acur = st->a_cur;
+    const double a_prev = st->a2, l_h = st->l_h, l_h_old = st->l_h_old;
+    const double a_next = next_momentum(a_prev);
+    const T beta = (T)(fw ? 0.0 : extrap_beta(a_prev, a_next, l_h_old, l_h));
+    T* Acur = reinterpret_cast<T*>(f.A) + (size_t)acur * g.Kt * g.N;
+    T* Aprev = reinterpret_cast<T*>(f.A) + (size_t)(acur ^ 1) * g.Kt * g.N;
+    int bad = 0;
+    for (int j = threadIdx.x; j < g.N; j += blockDim.x) {
+        double v[kMaxKt];
+        double sa = 0.0;
+        if (!fw) {
+            for (int k = 0; k < g.Kt; ++k) {
+                const T ac = Acur[(size_t)k * g.N + j], ap = Aprev[(size_t)k * g.N + j];
+                const T atv = ac + beta * (ac - ap);
+                v[k] = (double)(atv + (T)(grad[(size_t)k * g.N + j]) / (T)l_h);
+            }
+            if (!project_simplex(v, g.Kt)) bad = 1;
+            else
+                for (int k = 0; k < g.Kt; ++k) Aprev[(size_t)k * g.N + j] = (T)v[k];   // becomes the current slot
+            for (int q = 0; q < g.nu; ++q) sa = fma(v[g.K + q], v[g.K + q], sa);
+        } else {
+            // gradient = -G; vertex = FIRST argmin of each block (np.argmin), deconvolution.py:286-299
+            const double pj = f.purity[j];
+            const double gamma = 2.0 / (double)(k_inner + 2);
+            int i1 = 0, i2 = 0;
+            double m1 = 0.0, m2 = 0.0;
+            for (int k = 0; k < g.K; ++k) {
+                const double gk = -grad[(size_t)k * g.N + j];
+                if (k == 0 || gk < m1) { m1 = gk; i1 = k; }
+            }
+            for (int q = 0; q < g.nu; ++q) {
+                const double gq = -grad[(size_t)(g.K + q) * g.N + j];
+                if (q == 0 || gq < m2) { m2 = gq; i2 = q; }
+            }
+            for (int k = 0; k < g.Kt; ++k) {
+                const double s = (k < g.K) ? ((k == i1) ? pj : 0.0) : ((k - g.K == i2) ? (1.0 - pj) : 0.0);
+                const double an = (1.0 - gamma) * (double)Acur[(size_t)k * g.N + j] + gamma * s;
+                Acur[(size_t)k * g.N + j] = (T)an;
+                if (k >= g.K) sa = fma(an, an, sa);
+            }
+        }
+        colred[j] = sa;
+    }
+    if (bad) st->done = 3;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double sa = 0.0;
+        for (int j = 0; j < g.N; ++j) sa += colred[j];
+        state_end_alpha(st, sa, !fw, a_next, st->t_a + 1, l_h, true);
+        if (!fw) st->a_cur = acur ^ 1;
+    }
+}
+
+// alpha pass: G = R^T (d o (x - R a_eval)); last CTA applies the step (alpha_step)
 template <typename T, typename WT, int KTB, int C>
 __global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) alpha_pass_kernel(const PassArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -709,54 +780,12 @@ __global__ void __launch_bounds__(kThreads, pass_min_blocks(KTB)) alpha_pass_ker
         for (int e = c.ctid; e < KN; e += kConsumers) part[e] = scratch[e];
     }
     if (!hier_reduce(g, f, scratch, KN, &c.ctl->flag)) return;
-
-    // ---- last CTA: apply the step on the Kt x N gradient held in scratch
-    double* colred = scratch + KN;        // per-column ||alpha_unk||^2 contributions
-    int bad = 0;
-    for (int j = threadIdx.x; j < g.N; j += blockDim.x) {
-        double v[kMaxKt];
-        double sa = 0.0;
-        if (!fw) {
-            for (int k = 0; k < g.Kt; ++k) {
-                const T ac = Acur[(size_t)k * g.N + j], ap = Aprev[(size_t)k * g.N + j];
-                const T atv = ac + beta * (ac - ap);
-                v[k] = (double)(atv + (T)(scratch[(size_t)k * g.N + j]) / (T)l_h);
-            }
-            if (!project_simplex(v, g.Kt)) bad = 1;
-            else
-                for (int k = 0; k < g.Kt; ++k) Aprev[(size_t)k * g.N + j] = (T)v[k];   // becomes the current slot
-            for (int q = 0; q < g.nu; ++q) sa = fma(v[g.K + q], v[g.K + q], sa);
-        } else {
-            // gradient = -G; vertex = FIRST argmin of each block (np.argmin), deconvolution.py:286-299
-            const double pj = f.purity[j];
-            const double gamma = 2.0 / (double)(a.k_inner + 2);
-            int i1 = 0, i2 = 0;
-            double m1 = 0.0, m2 = 0.0;
-            for (int k = 0; k < g.K; ++k) {
-                const double gk = -scratch[(size_t)k * g.N + j];
-                if (k == 0 || gk < m1) { m1 = gk; i1 = k; }
-            }
-            for (int q = 0; q < g.nu; ++q) {
-                const double gq = -scratch[(size_t)(g.K + q) * g.N + j];
-                if (q == 0 || gq < m2) { m2 = gq; i2 = q; }
-            }
-            for (int k = 0; k < g.Kt; ++k) {
-                const double s = (k < g.K) ? ((k == i1) ? pj : 0.0) : ((k - g.K == i2) ? (1.0 - pj) : 0.0);
-                const double an = (1.0 - gamma) * (double)Acur[(size_t)k * g.N + j] + gamma * s;
-                Acur[(size_t)k * g.N + j] = (T)an;
-                if (k >= g.K) sa = fma(an, an, sa);
-            }
-        }
-        colred[j] = sa;
+    if (a.flags & kFlagPartial) {
+        // CpG rows sharded over GPUs: publish this GPU's gradient; alpha_commit_kernel steps on the all-reduced one
+        for (int e = threadIdx.x; e < KN; e += blockDim.x) f.gram[e] = scratch[e];
+        return;
     }
-    if (bad) st->done = 3;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double sa = 0.0;
-        for (int j = 0; j < g.N; ++j) sa += colred[j];
-        state_end_alpha(st, sa, !fw, a_next, st->t_a + 1, l_h, true);
-        if (!fw) st->a_cur = acur ^ 1;
-    }
+    alpha_step<T>(g, f, scratch, scratch + KN, fw, a.k_inner);
 }
 
 }  // namespace dmf

@@ -59,7 +59,8 @@ def build_parser():
                    help="(B200 path, under torchrun) how several GPUs are used: 'fits' runs independent fits per GPU (--ic, --confidence; "
                         "the main fit runs on every GPU), 'rows' shards the CpG rows of every fit over the GPUs (the main fit and --ic AIC / "
                         "BIC / CCC / BCV with a reference matrix, a CCC member's restarts and a BCV member's folds as one batch; --confidence stays "
-                        "fit-sharded)")
+                        "fit-sharded); every shape a one-GPU fit runs can be row-sharded (more than 8 unknown types, or more than 4 with 7+ known "
+                        "ones, run the stream engine's passes with one all-reduce per step)")
     return p
 
 

@@ -8,7 +8,10 @@ and u plus a replica of alpha and of the fit state.  Per outer iteration (deconv
               then every rank runs the identical n_iter2 inner iterations on the reduced copy (dmf_gram_alpha_inner)
   cost        ONE sum all-reduce of 8 doubles per fit, then the identical termination test on every rank
 
-plus one max all-reduce (max d_x) at set-up.  The initial iterate is computed on the same row shards (`ShardedInit`): the
+plus one max all-reduce (max d_x) at set-up.  Shapes without the Gram form (more unknown types, or wider cohorts with many
+types) run the stream engine's passes instead: n_iter2 U passes then ONE scalar all-reduce (||u||^2, l_h), n_iter2 x (alpha or
+Frank-Wolfe pass, ONE all-reduce of the Kt x N gradient, the identical step on every rank), and the cost as above: n_iter2 + 2
+collectives per outer iteration.  The initial iterate is computed on the same row shards (`ShardedInit`): the
 `uniform` init and the reference-based fit all-reduce the WLS moment matrix, the SVD inits the N x N Gram matrix of the residual
 and the NNDSVD column norms.  Every rank therefore holds the same alpha and makes the same termination
 decision; u stays distributed.  `RowShardedFit` is the orchestration; the arithmetic sits behind a small backend
@@ -40,7 +43,7 @@ def row_range(M, rank, world):
 
 
 class GpuShardBackend:
-    """This rank's rows on its GPU: a FitBatch in sharded Gram-engine mode.  One fit, or several when U0_local and A0 are lists of
+    """This rank's rows on its GPU: a FitBatch in sharded mode on the fused, Gram-form or stream engine (by shape).  One fit, or several when U0_local and A0 are lists of
     initial iterates (CCC restarts, BCV folds); X_local is then one problem all fits share, or a list of resident DeviceProblems,
     one per fit.  Every fit has its own statistics block, all-reduced copy and peer slot, so one all-reduce per step covers all."""
 
@@ -55,6 +58,7 @@ class GpuShardBackend:
         _lib.check(lib.dmf_batch_set_sharded(b.b, 1, _stream_ptr()))
         # fused engine where the shape allows it: ONE pass and ONE all-reduce per outer iteration (RowShardedFit.outer)
         self.fused = b.engine == "fused"
+        self.stream = b.engine == "stream"         # shapes without the Gram form: one pass per reference step
         loc, glo, per, so = C.c_void_p(), C.c_void_p(), C.c_int64(), C.c_int64()
         _lib.check(lib.dmf_batch_stats_buffers(b.b, C.byref(loc), C.byref(glo), C.byref(per), C.byref(so)))
         base = b.ws.data_ptr()
@@ -115,7 +119,7 @@ class GpuShardBackend:
         """Make the following steps allocation- and sync-free (CUDA-graph capture)."""
         _lib.check(_lib.lib().dmf_batch_reserve_momentum(self.batch.b, int(n_inner_total), _stream_ptr()))
 
-    # ---- statistics blocks: (n_fits, doubles_per_fit) tensors [G | bx | scal(8)]
+    # ---- statistics blocks: (n_fits, doubles_per_fit) tensors, [G | bx | scal(8)] (Gram form, fused) or [alpha gradient | scal(8)] (stream)
     def stats_local(self):
         return self.local
 
@@ -140,6 +144,28 @@ class GpuShardBackend:
 
     def fused_alpha_commit(self, n_iter2, tol):
         _lib.check(_lib.lib().dmf_fused_alpha_commit(self.batch.b, int(n_iter2), float(tol), _stream_ptr()))
+
+    # ---- stream engine: [alpha gradient | scal(8)] blocks
+    def cost(self, initial, tol):
+        if initial:
+            self.batch.pass_init()
+        else:
+            self.batch.pass_cost(tol)
+
+    def pass_u(self):
+        self.batch.pass_u()
+
+    def u_commit(self):
+        _lib.check(_lib.lib().dmf_pass_u_commit(self.batch.b, _stream_ptr()))
+
+    def pass_alpha(self, k):
+        if self.batch.mode == _lib.DMF_MODE_PURITY:
+            self.batch.pass_fw(k)
+        else:
+            self.batch.pass_alpha()
+
+    def alpha_commit(self, k):
+        _lib.check(_lib.lib().dmf_pass_alpha_commit(self.batch.b, int(k), _stream_ptr()))
 
     def finalize_cost(self, initial, tol):
         _lib.check(_lib.lib().dmf_gram_finalize_cost(self.batch.b, int(bool(initial)), float(tol), _stream_ptr()))
@@ -191,10 +217,14 @@ class RowShardedFit:
     def init(self):
         """deconvolution.py:192-204: cost, ||R||^2, max d_x over ALL rows; then this rank's known x known statistics."""
         be = self.be
-        be.rowgram(True, 0.0)
+        stream = getattr(be, "stream", False)
+        if stream:
+            be.cost(True, 0.0)
+        else:
+            be.rowgram(True, 0.0)
         self._reduce_scal(with_max=True)
         be.finalize_cost(True, 0.0)
-        if be.has_known:
+        if be.has_known and not stream:
             be.panels(True)
 
     def _reduce_blocks(self):
@@ -219,6 +249,20 @@ class RowShardedFit:
             self._reduce_blocks()
             be.fused_alpha_commit(n_iter2, tol)
             self.pending = True
+            return
+        if getattr(be, "stream", False):
+            # stream engine: every pass publishes this rank's sums, the state advances on the all-reduced ones
+            for _ in range(n_iter2):
+                be.pass_u()                           # row-local; publishes ||u||^2 of this rank's rows
+            self._reduce_scal(with_max=False)
+            be.u_commit()                             # l_h from ||u||^2 over all rows
+            for k in range(n_iter2):
+                be.pass_alpha(k)                      # this rank's Kt x N gradient (Frank-Wolfe iteration k for purity fits)
+                self._reduce_blocks()
+                be.alpha_commit(k)                    # the identical step on every rank
+            be.cost(False, tol)
+            self._reduce_scal(with_max=False)
+            be.finalize_cost(False, tol)
             return
         if n_iter2 > 0:
             be.u_inner(n_iter2)                       # row-local
@@ -286,8 +330,10 @@ class RowShardedFit:
 def mdwbssmf_deconv_sharded(u_local, alpha, X_local, d_local, R_local, n_u, n_iter1=100000, n_iter2=50, tol=1e-3, purity=None,
                             group=None):
     """mdwbssmf_deconv / mdwbssmf_deconv_p (deconvolution.py:190-223, :305-337) on a row-sharded problem: every rank passes
-    ITS rows of u, X, d_x, R_trunc (see `row_range`) and the full alpha; returns (u_local, alpha, n_outer, cost)."""
-    mode = _lib.DMF_MODE_PURITY if purity is not None else (_lib.DMF_MODE_PARTIAL if R_local is not None else _lib.DMF_MODE_UNSUPERVISED)
+    ITS rows of u, X, d_x, R_trunc (see `row_range`), or a resident DeviceProblem of them as X_local, and the full alpha; returns
+    (u_local, alpha, n_outer, cost)."""
+    has_ref = R_local is not None or (isinstance(X_local, DeviceProblem) and X_local.K > 0)
+    mode = _lib.DMF_MODE_PURITY if purity is not None else (_lib.DMF_MODE_PARTIAL if has_ref else _lib.DMF_MODE_UNSUPERVISED)
     be = GpuShardBackend(X_local, d_local, R_local, n_u, np.asarray(u_local).reshape(-1, n_u), np.asarray(alpha), mode=mode, purity=purity)
     (u, a, n_outer, cost), = fit_row_sharded(be, n_iter1, n_iter2, tol, group)
     return u, a, n_outer, cost

@@ -165,14 +165,24 @@ int dmf_gram_panels(dmf_batch_t b, int32_t known_block, void* stream);
  * (deconvolution.py:285-299) for purity batches, per sample on (G_j, bx_j) */
 int dmf_gram_alpha_inner(dmf_batch_t b, int32_t n_iter2, void* stream);
 /* CpG rows sharded over several GPUs (one process per GPU, each batch holds its own row range of X, d_x, R_trunc, u and a
- * replica of alpha).  With sharding on, dmf_gram_rowgram / dmf_gram_u_inner / dmf_gram_panels publish THIS GPU's sums in the
- * `local` statistics block of every fit, [G (Kt*Kt*N) | bx (Kt*N) | scal (8): cost, ||R_trunc||^2, ||u||^2 at set-up, max d_x,
- * ||u||^2 after the U step], and leave the fit state alone.  The caller copies local -> global, all-reduces `global` over the
- * GPUs (sum; max for scal[3]) and then runs dmf_gram_finalize_cost (after rowgram) / dmf_gram_alpha_inner (after panels), which
- * read `global`.  Every rank ends up with the identical state and alpha.  Fits are doubles_per_fit apart in both blocks. */
+ * replica of alpha).  Every shape a batch can run can be sharded; the engine is chosen by shape: fused where it applies, then
+ * the Gram form, then the stream engine.  With sharding on, the steps publish THIS GPU's sums in the `local` statistics block
+ * of every fit and leave the fit state alone; the caller copies local -> global, all-reduces `global` over the GPUs (sum; max
+ * for scal[3]) and then runs the step that reads `global`.  scal (8) = [cost, ||R_trunc||^2, ||u||^2 at set-up, max d_x,
+ * ||u||^2 after the U step, unused].  Every rank ends up with the identical state and alpha.  Fits are doubles_per_fit apart
+ * in both blocks.
+ *   Gram form: blocks [G (Kt*Kt*N) | bx (Kt*N) | scal].  dmf_gram_rowgram -> scalars -> dmf_gram_finalize_cost;
+ *     dmf_gram_u_inner + dmf_gram_panels -> blocks -> dmf_gram_alpha_inner.
+ *   Stream engine (shapes without the Gram form): blocks [alpha gradient (Kt*N) | scal].  dmf_pass_init / dmf_pass_cost ->
+ *     scalars -> dmf_gram_finalize_cost; n_iter2 x dmf_pass_u -> scalars -> dmf_pass_u_commit (l_h from the reduced ||u||^2);
+ *     n_iter2 x (dmf_pass_alpha or dmf_pass_fw(k) -> blocks -> dmf_pass_alpha_commit(k)), the projected-gradient or Frank-Wolfe
+ *     step on the reduced gradient.  dmf_enqueue_outer / dmf_fit_batched refuse such batches; the dmf_pass_* calls and the two commits
+ * refuse sharded batches on the fused or Gram-form engine. */
 int dmf_batch_set_sharded(dmf_batch_t b, int32_t on, void* stream);
 int dmf_batch_stats_buffers(dmf_batch_t b, void** local_dev, void** global_dev, int64_t* doubles_per_fit, int64_t* scal_offset);
 int dmf_gram_finalize_cost(dmf_batch_t b, int32_t initial, double tol, void* stream);
+int dmf_pass_u_commit(dmf_batch_t b, void* stream);
+int dmf_pass_alpha_commit(dmf_batch_t b, int32_t k_inner, void* stream);
 /* Row-sharded runs, all-reduce over NVLink PEER MEMORY instead of NCCL: every rank provides a zero-initialised symmetric buffer of
  * dmf_batch_peer_bytes() bytes that all ranks of the box have mapped (peer_bases[r] = rank r's buffer as addressable from THIS
  * process, e.g. torch symmetric memory's buffer_ptrs).  dmf_gram_exchange is then ONE kernel per rank that pushes this rank's sums

@@ -64,12 +64,12 @@ def main():
     sys.exit(0 if ok else 1)
 
 
-def cli_check(rank, world):
+def cli_check(rank, world, cases=None, K=5):
     import tempfile
     import pandas as pd
     from demethify_b200 import demethify
     rs = np.random.RandomState(8)
-    M, N, K = 9001, 10, 5
+    M, N = 9001, 10
     Rf = rs.beta(0.5, 0.5, size=(M, K + 2))
     D = rs.poisson(40, size=(M, N)) + 1
     X = rs.binomial(D, np.clip(Rf @ rs.dirichlet(np.ones(K + 2), N).T, 0, 1)) / D
@@ -82,9 +82,9 @@ def cli_check(rank, world):
             pd.DataFrame({"percent_modified": X[:, j], "valid_coverage": D[:, j]}).to_csv(f"{d}/s{j}.csv", index=False)
     dist.barrier()
     files = [f"{d}/s{j}.csv" for j in range(N)]
-    cases = [("uniform_", ["--nbunknown", "2"]), ("uniform", ["--nbunknown", "2"]), ("beta", ["--nbunknown", "2"]),
-             ("SVD", ["--nbunknown", "2"]), ("SVD", ["--nbunknown", "2", "--purity"] + ["60"] * N), ("SVD", ["--nbunknown", "2", "--noref"]),
-             ("uniform_", ["--nbunknown", "0"])]
+    cases = cases or [("uniform_", ["--nbunknown", "2"]), ("uniform", ["--nbunknown", "2"]), ("beta", ["--nbunknown", "2"]),
+                      ("SVD", ["--nbunknown", "2"]), ("SVD", ["--nbunknown", "2", "--purity"] + ["60"] * N),
+                      ("SVD", ["--nbunknown", "2", "--noref"]), ("uniform_", ["--nbunknown", "0"])]
     ok = True
     for c, (init, extra) in enumerate(cases):
         ref = [] if "--noref" in extra else ["--ref", f"{d}/ref.csv"]
@@ -116,26 +116,28 @@ def cli_check(rank, world):
     return box[0]
 
 
-def ic_check(rank, world):
+def ic_check(rank, world, runs=None, n_u_values=(1, 2, 3), K=5):
     from demethify_b200.ic import evaluate_best_ic
     rs = np.random.RandomState(9)
-    M, N, K = 30011, 12, 5
+    M, N = 30011, 12
+    n_u_values = list(n_u_values)
     Rf = rs.beta(0.5, 0.5, size=(M, K + 2))
     D = rs.poisson(40, size=(M, N)) + 1
     X = rs.binomial(D, np.clip(Rf @ rs.dirichlet(np.ones(K + 2), N).T, 0, 1)) / D
     one = dist.new_group([0])
     ok = True
-    for crit, init, seed in (("CCC", "uniform_", 1), ("CCC", "SVD", 2), ("BCV", "uniform_", [3]), ("BCV", "uniform", 4), ("BCV", "SVD", 5)):
-        u, a, best, values = evaluate_best_ic(X, Rf[:, :K], D, init, crit, seed, 300, 20, 1e-2, n_restarts=3, n_u_values=[1, 2, 3],
+    runs = runs or (("CCC", "uniform_", 1), ("CCC", "SVD", 2), ("BCV", "uniform_", [3]), ("BCV", "uniform", 4), ("BCV", "SVD", 5))
+    for crit, init, seed in runs:
+        u, a, best, values = evaluate_best_ic(X, Rf[:, :K], D, init, crit, seed, 300, 20, 1e-2, n_restarts=3, n_u_values=n_u_values,
                                               shard="rows")
         if rank == 0:
-            u1, a1, best1, values1 = evaluate_best_ic(X, Rf[:, :K], D, init, crit, seed, 300, 20, 1e-2, n_restarts=3, n_u_values=[1, 2, 3],
+            u1, a1, best1, values1 = evaluate_best_ic(X, Rf[:, :K], D, init, crit, seed, 300, 20, 1e-2, n_restarts=3, n_u_values=n_u_values,
                                                       shard="fits", group=one)
             dv = np.abs(np.array(values) - np.array(values1)).max()
             da, du = np.abs(a - a1).max(), np.abs(u - u1).max()
             good = best == best1 and dv <= 1e-8 * max(1.0, np.abs(values1).max()) and da <= 1e-8 and du <= 1e-8
             ok &= good
-            print(f"sharded_check ic world={world} {crit} --init {init} seed={seed}: best n_u {best} (one GPU {best1}) max|d criterion|={dv:.2e} "
+            print(f"sharded_check ic world={world} {crit} --init {init} seed={seed} n_u {n_u_values}: best n_u {best} (one GPU {best1}) max|d criterion|={dv:.2e} "
                   f"max|d alpha|={da:.2e} max|d u|={du:.2e} -> {'OK' if good else 'FAIL'}", flush=True)
         dist.barrier()
     box = [ok]
