@@ -508,10 +508,10 @@ __global__ void pack_u16_kernel(const S* src, long long n, uint16_t* dst, int* b
         const S v = src[i];
         const double d = (double)v;
         const bool ok = d >= 0.0 && d <= 65535.0 && d == floor(d);
-        if (!ok) local_bad = 1;
+        local_bad += ok ? 0 : 1;        // a thread visits several entries once count > the grid: count entries, not threads
         dst[i] = ok ? (uint16_t)d : (uint16_t)0;
     }
-    if (local_bad) atomicAdd(bad, 1);
+    if (local_bad) atomicAdd(bad, local_bad);
 }
 
 __global__ void gather_rows_kernel(const char* src, const int32_t* rows, long long n_rows, long long row_bytes, char* dst) {

@@ -2,7 +2,16 @@
 // library's instantiation objects.  It makes no CUDA call: it reads one shape per stdin line
 //   M N K n_u dtype wtype mode n_fits max_ctas_per_fit u_slots ldx ldd ldr ldu u_slot form      (form: 0 plain, 1 multiplicity, 2 gather)
 // and prints one JSON object per line: the geometry of every engine the planner makes available, the kernels it would launch that
-// resolve to nothing, and the workspace regions.
+// resolve to nothing, the dispatch entries a fit on each engine launches ("launch") and the workspace regions.
+//   plan_probe universe   prints every dispatch entry: a (lookup function, storage tag, arguments) triple over the domain of the
+//                         kernel tables (dmf_inst_body.cuh) that resolves to a kernel, one name per line
+//   plan_probe scan       prints the dispatch entries that some shape of the planner's whole domain launches on some engine
+//                         (N 1..512, K + n_u <= 32, every storage tag, mode and form, three pitch styles), one name per line,
+//                         then one line "combo <storage tag> <engine> <mode>" per combination some shape offers
+#include <map>
+#include <set>
+#include <tuple>
+
 #include "dmf_api.cu"
 
 namespace {
@@ -23,10 +32,183 @@ void print_engine(const char* name, const Geom& g, unsigned smem, unsigned ring,
     printf("}");
 }
 
+// ---- dispatch entries.  The name holds every argument the lookup function reads, e.g. rowgram<f32_f32>[kb=16,nub=2,initial=1]
+enum Fn { F_COST, F_ALPHA, F_U, F_ROWGRAM, F_PANEL, F_UINNER, F_AINNER, F_FUSED, F_WLS };
+const char* const kTag[4] = {"f64_f64", "f64_u16", "f32_f32", "f32_u16"};   // the order of by_types
+wls_kern_t (*const g_wls[4])() = {pick_wls_f64_f64, pick_wls_f64_u16, pick_wls_f32_f32, pick_wls_f32_u16};
+
+std::vector<std::string> g_names;                               // entry id -> name
+std::map<std::tuple<int, int, const void*>, int> g_entry;       // (function, tag, kernel) -> entry id
+
+std::string entry_name(int fn, int tag, int a, int b, int c) {
+    char buf[128];
+    const char* t = kTag[tag];
+    switch (fn) {
+        case F_COST: snprintf(buf, sizeof buf, "cost<%s>[ktb=%d,c=%d,initial=%d]", t, a, c, b); break;
+        case F_ALPHA: snprintf(buf, sizeof buf, "alpha<%s>[ktb=%d,c=%d]", t, a, c); break;
+        case F_U: snprintf(buf, sizeof buf, "u<%s>[kb=%d,nub=%d]", t, a, b); break;
+        case F_ROWGRAM: snprintf(buf, sizeof buf, "rowgram<%s>[kb=%d,nub=%d,initial=%d]", t, a, b, c); break;
+        case F_PANEL: snprintf(buf, sizeof buf, "%s<%s>[pb=%d,c=%d]", c == 0 ? "panel" : (c == 1 ? "panel_mult" : "panel_mult_u1"), t, a, b); break;
+        case F_UINNER: {
+            const char* k[4] = {"u_inner", "u_inner_mult", "cost_cross", "usum"};
+            snprintf(buf, sizeof buf, "%s<%s>[nub=%d]", k[b], t, a);
+            break;
+        }
+        case F_AINNER: snprintf(buf, sizeof buf, "alpha_inner<%s>[ktb=%d]", t, a); break;
+        case F_FUSED: snprintf(buf, sizeof buf, "fused<%s>[kb=%d,nub=%d,s=%d]", t, a, b, c); break;
+        default: snprintf(buf, sizeof buf, "wls<%s>", t);
+    }
+    return buf;
+}
+
+void add_entry(int fn, int tag, int a, int b, int c, const void* k) {
+    if (!k) return;
+    const std::string name = entry_name(fn, tag, a, b, c);
+    const auto key = std::make_tuple(fn, tag, k);
+    const auto it = g_entry.find(key);
+    if (it != g_entry.end()) {
+        if (g_names[it->second] != name) {           // one kernel under two names: the name misses an argument the lookup reads
+            fprintf(stderr, "plan_probe: %s and %s resolve to the same kernel\n", g_names[it->second].c_str(), name.c_str());
+            exit(2);
+        }
+        return;
+    }
+    for (const std::string& n : g_names)
+        if (n == name) {                               // one name, two kernels: the name ignores an argument the lookup reads
+            fprintf(stderr, "plan_probe: %s resolves to two kernels\n", name.c_str());
+            exit(2);
+        }
+    g_entry[key] = (int)g_names.size();
+    g_names.push_back(name);
+}
+
+// every argument combination of the tables' domain (arguments beyond it select nothing or a duplicate)
+void build_universe() {
+    for (int t = 0; t < 4; ++t) {
+        for (int a = 0; a <= 32; ++a) {
+            for (int c = 0; c <= 4; ++c) {
+                for (int b = 0; b <= 1; ++b) add_entry(F_COST, t, a, b, c, (const void*)g_cost[t](a, b, c));
+                add_entry(F_ALPHA, t, a, 0, c, (const void*)g_alpha[t](a, 0, c));
+                for (int m = 0; m <= 2; ++m) add_entry(F_PANEL, t, a, c, m, (const void*)g_panel[t](a, c, m));
+            }
+            for (int b = 0; b <= 32; ++b) {
+                add_entry(F_U, t, a, b, 0, (const void*)g_u[t](a, b, 0));
+                for (int c = 0; c <= 1; ++c) add_entry(F_ROWGRAM, t, a, b, c, (const void*)g_rowgram[t](a, b, c));
+                for (int c = 0; c <= 4; ++c) add_entry(F_FUSED, t, a, b, c, (const void*)g_fused[t](a, b, c));
+            }
+            for (int w = 0; w <= 3; ++w) add_entry(F_UINNER, t, a, w, 0, (const void*)g_uinner[t](a, w, 0));
+            add_entry(F_AINNER, t, a, 0, 0, (const void*)g_ainner[t](a, 0, 0));
+        }
+        add_entry(F_WLS, t, 0, 0, 0, (const void*)g_wls[t]());
+    }
+}
+
+int tag_of(const dmf_shape_t& s) { return (s.dtype == DMF_F64 ? 0 : 2) + (s.wtype == DMF_W_U16 ? 1 : 0); }
+int entry_of(int fn, const dmf_shape_t& s, const void* k) {
+    const auto it = g_entry.find(std::make_tuple(fn, tag_of(s), k));
+    return it == g_entry.end() ? -1 : it->second;
+}
+
+// The dispatch entries a dmf_fit_batched call launches on each engine the batch offers (-1: a launch that resolves to nothing).
+// Stream: dmf_pass_init, dmf_pass_u, dmf_pass_alpha / dmf_pass_fw, dmf_pass_cost.  Gram: dmf_gram_init (rowgram, known-block
+// panels) and dmf_gram_outer (u_inner, panels, alpha_inner, rowgram), with the multiplicity form's cost_cross and usum.  Fused:
+// dmf_gram_init, dmf_fused_outer (fused pass, alpha_inner) and dmf_fused_finish (rowgram).
+struct Launches { std::vector<int> e[3]; bool on[3]; };
+Launches launches_of(dmf_batch_s* b) {
+    const dmf_shape_t& s = b->shape;
+    const Plan& q = b->p;
+    Launches L{};
+    L.on[0] = !b->multmode;
+    if (L.on[0])
+        L.e[0] = {entry_of(F_COST, s, (const void*)k_cost(b, 1)), entry_of(F_COST, s, (const void*)k_cost(b, 0)),
+                  entry_of(F_U, s, (const void*)k_u(b)), entry_of(F_ALPHA, s, (const void*)k_alpha(b))};
+    L.on[1] = q.gram_ok;
+    if (L.on[1]) {
+        std::vector<int>& g = L.e[1];
+        g = {entry_of(F_ROWGRAM, s, (const void*)k_rowgram(b, 1)), entry_of(F_ROWGRAM, s, (const void*)k_rowgram(b, 0)),
+             entry_of(F_UINNER, s, (const void*)k_uinner(b)), entry_of(F_AINNER, s, (const void*)k_ainner(b))};
+        if (s.K) g.push_back(entry_of(F_PANEL, s, (const void*)k_panel(b)));
+        g.push_back(entry_of(F_PANEL, s, (const void*)(b->multmode && s.n_u == 1 ? k_panel_u1(b) : k_panel(b))));
+        if (b->multmode) {
+            g.push_back(entry_of(F_UINNER, s, (const void*)k_costcross(b)));
+            g.push_back(entry_of(F_UINNER, s, (const void*)k_usum(b)));
+        }
+    }
+    L.on[2] = q.fused_ok;
+    if (L.on[2]) {
+        std::vector<int>& f = L.e[2];
+        f = {entry_of(F_ROWGRAM, s, (const void*)k_rowgram(b, 1)), entry_of(F_ROWGRAM, s, (const void*)k_rowgram(b, 0)),
+             entry_of(F_FUSED, s, (const void*)by_types_f(s, q.kb_f, q.nub_f, q.s_f)), entry_of(F_AINNER, s, (const void*)k_ainner(b))};
+        if (s.K) f.push_back(entry_of(F_PANEL, s, (const void*)k_panel(b)));
+    }
+    return L;
+}
+
+// the batch-specific part of dmf_batch_create: gather form, multiplicity form, its one-unknown panel, the fused engine's exclusions
+void batch_of(dmf_batch_s& b, const dmf_shape_t& s, const Plan& p, int form) {
+    b.shape = s;
+    b.p = p;
+    b.multmode = form == 1;
+    b.p.p1_ok = b.multmode && p.p1_ok;
+    b.p.fused_ok = p.fused_ok && form == 0;
+    if (b.multmode) std::copy(p.tx_mult, p.tx_mult + kMaxSrc, b.p.gg.tile_tx);
+}
+
+// the planner's whole domain: every shape it accepts, with DeviceProblem's pitches, the smallest even pitches and 16-byte pitches
+int scan(const dmf_handle_s& h) {
+    const char* const engine_names[3] = {"stream", "gram", "fused"};
+    const char* const mode_names[3] = {"partial", "purity", "unsup"};      // DMF_MODE_*
+    std::set<int> reached;
+    std::set<std::string> combos;
+    for (int tag = 0; tag < 4; ++tag)
+        for (int K = 0; K < kMaxKt; ++K)
+            for (int n_u = 1; K + n_u <= kMaxKt; ++n_u)
+                for (int mode = 0; mode < 3; ++mode)
+                    for (int N = 1; N <= 512; ++N)
+                        for (int style = 0; style < 3; ++style)
+                            for (int form = 0; form < 2; ++form) {
+                                dmf_shape_t s{};
+                                s.M = 100000; s.N = N; s.K = K; s.n_u = n_u;
+                                s.dtype = tag < 2 ? DMF_F64 : DMF_F32; s.wtype = tag & 1 ? DMF_W_U16 : DMF_W_FLOAT;
+                                s.mode = mode; s.n_fits = 1; s.u_slots = form == 1 ? 2 : 4;
+                                const int es = s.dtype == DMF_F64 ? 8 : 4, ew = s.wtype == DMF_W_U16 ? 2 : es;
+                                const auto even = [](long long v) { return v + (v & 1); };
+                                const auto al16 = [](long long v, int e) { return (v * e + 15) / 16 * 16 / e; };
+                                const bool wide = N * es >= 512;
+                                const auto dev = [&](int e) { return wide ? ((N * e + 127) / 128 * 128 + 16) / e : (long long)(N + 7) / 8 * 8; };
+                                if (style == 0) { s.ldx = dev(es); s.ldd = s.wtype == DMF_W_U16 ? dev(2) : s.ldx; }
+                                else if (style == 1) { s.ldx = s.ldd = even(N); }
+                                else { s.ldx = al16(even(N), es); s.ldd = al16(even(N), ew); }
+                                s.ldr = even(K); s.ldu = even(n_u);
+                                s.u_slot = al16(s.M * s.ldu, es);
+                                Plan p;
+                                if (make_plan(&h, s, p)) continue;
+                                if (form == 1 && !p.mult_ok) continue;
+                                dmf_batch_s b{};
+                                batch_of(b, s, p, form);
+                                const Launches L = launches_of(&b);
+                                for (int e = 0; e < 3; ++e)
+                                    if (L.on[e]) {
+                                        reached.insert(L.e[e].begin(), L.e[e].end());
+                                        combos.insert(std::string("combo ") + kTag[tag] + " " + engine_names[e] + " " + mode_names[mode]);
+                                    }
+                            }
+    for (int id : reached)
+        if (id >= 0) printf("%s\n", g_names[id].c_str());
+    for (const std::string& c : combos) printf("%s\n", c.c_str());
+    return 0;
+}
+
 }  // namespace
 
-int main() {
+int main(int argc, char** argv) {
     const dmf_handle_s h{0, 148, 232448};
+    build_universe();
+    if (argc > 1 && !strcmp(argv[1], "universe")) {
+        for (const std::string& n : g_names) printf("%s\n", n.c_str());
+        return 0;
+    }
+    if (argc > 1 && !strcmp(argv[1], "scan")) return scan(h);
     dmf_shape_t s;
     int form;
     long long M, ldx, ldd, ldr, ldu, u_slot;
@@ -44,14 +226,8 @@ int main() {
             printf(", \"mult_ok\": 0}\n");
             continue;
         }
-        // the batch-specific part of dmf_batch_create: multiplicity form, its one-unknown panel, the fused engine's exclusions
         dmf_batch_s b{};
-        b.shape = s;
-        b.p = p;
-        b.multmode = form == 1;
-        b.p.p1_ok = b.multmode && p.p1_ok;
-        b.p.fused_ok = p.fused_ok && form == 0;
-        if (b.multmode) std::copy(p.tx_mult, p.tx_mult + kMaxSrc, b.p.gg.tile_tx);
+        batch_of(b, s, p, form);
         const Plan& q = b.p;
         printf(", \"mult_ok\": %d, \"cap\": %d, \"buckets\": {\"ktb\": %d, \"kb\": %d, \"nub\": %d, \"kb_g\": %d, \"nub_g\": %d, \"s_f\": %d}",
                p.mult_ok, h.max_smem_optin, p.ktb, p.kb, p.nub, p.kb_g, p.nub_g, p.s_f);
@@ -86,6 +262,18 @@ int main() {
                    q.fc.threads, f.offStats);
             print_list("offs", off, kMaxSrc);
             printf("}");
+        }
+        printf("}");
+
+        const char* const engine_names[3] = {"stream", "gram", "fused"};
+        const Launches L = launches_of(&b);
+        printf(", \"launch\": {");
+        for (int e = 0, first = 1; e < 3; ++e) {
+            if (!L.on[e]) continue;
+            printf("%s\"%s\": [", first ? "" : ", ", engine_names[e]);
+            first = 0;
+            for (size_t i = 0; i < L.e[e].size(); ++i) printf("%s\"%s\"", i ? ", " : "", L.e[e][i] < 0 ? "null" : g_names[L.e[e][i]].c_str());
+            printf("]");
         }
         printf("}");
 
