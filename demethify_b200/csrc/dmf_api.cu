@@ -1277,8 +1277,9 @@ int wls_status(const void* status_dev, cudaStream_t st) {
     int status = 0;
     CUDA_TRY(cudaMemcpyAsync(&status, status_dev, sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    if (status & 1) return fail(DMF_E_STATE, "wls: a sample produced non-finite proportions (all of its weights zero, or non-finite inputs)");
+    if (status & 1) return fail(DMF_E_STATE, "wls: a sample produced non-finite proportions (non-finite inputs)");
     if (status & 2) return fail(DMF_E_STATE, "wls: the regressors of a sample are collinear (non-positive pivot in the normal equations)");
+    if (status & 4) return fail(DMF_E_STATE, "wls: the active-set NNLS of a sample reached its limit of 3 K inner iterations with a non-positive coefficient");
     return DMF_OK;
 }
 

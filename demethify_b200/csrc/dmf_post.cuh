@@ -80,6 +80,8 @@ static __global__ void __launch_bounds__(256) nndsvd_split_kernel(const double* 
 // a + (b - a) g for g < 0.5, b - (b - a)(1 - g) otherwise (numpy's _lerp).  One thread per entry p; stack is B x P row-major, so
 // the threads of a warp read consecutive addresses for every b.  The thread keeps the KS smallest and the KL largest values seen
 // so far in two sorted arrays (insertion): KS = floor((B-1) q_lo/100) + 2, KL = B - floor((B-1) q_hi/100), both <= KMAX.
+// A NaN among the B values makes both outputs NaN, as np.percentile does (it sorts NaN last and then returns np.nan); the
+// comparisons of the insertion would otherwise skip it, or keep it and block every later insertion.
 template <int KMAX>
 __global__ void __launch_bounds__(128) percentile_kernel(const double* __restrict__ stack, int B, long long P, double q_lo, double q_hi,
                                                          double* __restrict__ out_lo, double* __restrict__ out_hi) {
@@ -91,8 +93,10 @@ __global__ void __launch_bounds__(128) percentile_kernel(const double* __restric
     const int KS = min(klo + 2, B), KL = min(B - khi, B);
     double sm[KMAX], lg[KMAX];         // sm ascending (the KS smallest), lg descending (the KL largest)
     int ns = 0, nl = 0;
+    bool nan = false;
     for (int b = 0; b < B; ++b) {
         const double v = stack[(long long)b * P + p];
+        if (v != v) { nan = true; continue; }
         if (ns < KS || v < sm[ns - 1]) {
             int k = ns < KS ? ns++ : ns - 1;
             while (k > 0 && sm[k - 1] > v) { sm[k] = sm[k - 1]; --k; }
@@ -103,6 +107,10 @@ __global__ void __launch_bounds__(128) percentile_kernel(const double* __restric
             while (k > 0 && lg[k - 1] < v) { lg[k] = lg[k - 1]; --k; }
             lg[k] = v;
         }
+    }
+    if (nan) {
+        out_lo[p] = out_hi[p] = __longlong_as_double(0x7ff8000000000000ll);     // np.nan
+        return;
     }
     auto lerp = [](double a, double b, double g) { const double d = b - a; return g >= 0.5 ? b - d * (1.0 - g) : a + d * g; };
     {
@@ -117,7 +125,7 @@ __global__ void __launch_bounds__(128) percentile_kernel(const double* __restric
 }
 
 // ------------------------------------------------------------------------------------------------
-// ic.py:24-37: labels[r][j] = argmax_k alpha_r[k][j] (first maximum, np.argmax), consensus[i][j] = mean_r (labels[r][i] == labels[r][j])
+// ic.py:24-37: labels[r][j] = argmax_k alpha_r[k][j] (first maximum, np.argmax: a NaN counts as the maximum, the first one wins), consensus[i][j] = mean_r (labels[r][i] == labels[r][j])
 static __global__ void labels_kernel(const double* __restrict__ alpha, int n_runs, int Kt, int N, int* __restrict__ labels) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_runs * N) return;
@@ -127,7 +135,7 @@ static __global__ void labels_kernel(const double* __restrict__ alpha, int n_run
     double bv = a[0];
     for (int k = 1; k < Kt; ++k) {
         const double v = a[(size_t)k * N];
-        if (v > bv) { bv = v; best = k; }
+        if (v > bv || (v != v && bv == bv)) { bv = v; best = k; }
     }
     labels[e] = best;
 }

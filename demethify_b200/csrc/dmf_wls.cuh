@@ -149,7 +149,7 @@ static __global__ void wls_nnls_kernel(const double* __restrict__ mom, int K, in
     for (int p = 0; p < K; ++p) nb += fabs(b[p]);
     const double tolx = 10.0 * (double)(M > K ? M : K) * 2.220446049250313e-16;     // threshold on the coefficients: unscaled
     const double tol = tolx * nb;                                                     // threshold on the dual w = A^T (b - A x): scaled by |A^T b|_1
-    bool singular = false;
+    bool singular = false, capped = false;
     // solve G_PP s_P = b_P by Cholesky on the passive set
     auto solve = [&]() {
         int idx[kMaxKt], n = 0;
@@ -191,11 +191,12 @@ static __global__ void wls_nnls_kernel(const double* __restrict__ mom, int K, in
         if (best < 0) break;
         pas[best] = true;
         solve();
-        while (it < max_it) {
+        while (true) {
             double smin = 1e300;
             for (int p = 0; p < K; ++p)
                 if (pas[p] && s[p] < smin) smin = s[p];
             if (smin > 0.0) break;
+            if (it >= max_it) { capped = true; break; }     // x = s below would keep a non-positive coefficient
             ++it;
             double step = 1e300;
             for (int p = 0; p < K; ++p)
@@ -214,8 +215,10 @@ static __global__ void wls_nnls_kernel(const double* __restrict__ mom, int K, in
     for (int p = 0; p < K; ++p) sum += x[p];
     const double den = sum > 1e-10 ? sum : 1e-10;
     for (int p = 0; p < K; ++p) out[(size_t)p * ldo + j] = x[p] / den;
-    if (!(sum == sum)) atomicOr(status, 1);           // NaN proportions (e.g. a sample whose weights are all zero)
+    if (!(sum == sum)) atomicOr(status, 1);           // NaN proportions (non-finite inputs).  A sample whose weights are all zero
+                                                      // (masked out) has NaN normal equations, admits no variable and gets 0
     if (singular) atomicOr(status, 2);
+    if (capped) atomicOr(status, 4);
 }
 #endif  // DMF_INST_BODY
 
